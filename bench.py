@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 self-play search engine (driver contract in the task).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload encode|selfplay] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload encode|selfplay] [--impl reference] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`):
   selfplay  configs[3]/[4]: batched self-play, G concurrent games x 800 sims/move, ResNet-24 bf16;
@@ -115,6 +115,37 @@ def barrier(world: int):
     torch.cuda.synchronize()
 
 
+DUMP_ROWS = 512          # --dump-outputs keeps at most this many rows of an array ...
+DUMP_BYTES = 64 << 20    # ... and at most this many bytes in all
+
+
+def dump_outputs(directory: str, arrays) -> None:
+    """--dump-outputs: every array (torch or numpy) as DIR/<name>.npy.  Floating arrays keep float32 / float64, integer ones
+    become float64 (exact).  An array of more than DUMP_ROWS rows is cut to a sample of rows drawn from a fixed seed, the same
+    rows for every array of that length, so that two builds run with the same arguments can be compared output for output.
+    The rows are picked where the array lives (on the device for a CUDA tensor) before anything is copied to the host."""
+    import numpy as np
+    out = {}
+    for name, a in arrays.items():
+        if not hasattr(a, "detach"):
+            a = np.asarray(a)
+        if a.ndim and a.shape[0] > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_ROWS, replace=False))
+            if hasattr(a, "detach"):
+                import torch
+                rows = torch.from_numpy(rows).to(a.device)
+            a = a[rows]
+        if hasattr(a, "detach"):
+            a = a.detach().cpu().numpy()
+        out[name] = np.ascontiguousarray(a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes, more than {DUMP_BYTES}")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # ---- workload: encode (configs[1]) -------------------------------------------------------------
 ENC_BYTES_PER_POS = 72 + 19 * 64 * 4 + 4672   # packed position read + float32 planes + uint8 mask written
 
@@ -165,6 +196,8 @@ def bench_encode(args, rank, world, local):
     clocks = sampler.stop()
     total_ms = max_over_ranks(t0.elapsed_time(t1), world)
     kern_ms = sum(a.elapsed_time(b) for a, b in evs) / len(evs)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"planes": planes, "legal_mask": mask})
 
     # end to end through the public Python API with HOST buffers: raw records in pinned memory ->
     # H2D -> pack + encode kernels -> D2H of planes and mask into pinned host buffers
@@ -279,7 +312,18 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     ap.add_argument("--no-extras", action="store_true", help="headline record only: skip the as_shipped / encode / forward_sweep sub-records")
     ap.add_argument("--precision", default=os.environ.get("M0_BENCH_PRECISION", "fp16"), choices=["fp16", "bf16", "fp32"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed as DIR/<name>.npy (rank 0; the same seeded sample "
+                         f"of at most {DUMP_ROWS} rows of every array).  Equal arguments give equal inputs and, on one build, equal files.  "
+                         "Self-play games reach the last step through moves the build itself searched and sampled, so the planes that step "
+                         "evaluated are written too: between two builds, compare the rows whose planes agree")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup is not None and args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native engine: it needs --impl native")
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints "NCCL version ..." on the first
     # collective), so file descriptor 1 points at stderr while the run lasts and the line goes to the saved descriptor.
     sys.stdout.flush()
@@ -316,13 +360,15 @@ def main():
         args.games = args.total_games // world
     if args.workload == "selfplay":
         import bench_selfplay
-        out = bench_selfplay.run(args, rank, world, local, ClockSampler, load_peaks, barrier, max_over_ranks)
+        dump = (lambda arrays: dump_outputs(args.dump_outputs, arrays)) if args.dump_outputs and rank == 0 else None
+        out = bench_selfplay.run(args, rank, world, local, ClockSampler, load_peaks, barrier, max_over_ranks, dump=dump)
         if world == 1 and not args.no_extras:
             # BASELINE configs[1] beside the headline: the encode + legal-mask microbenchmark with its own roofline / e2e / cpu_baseline
             import torch
             torch.cuda.empty_cache()
             enc_args = argparse.Namespace(**vars(args))
             enc_args.steps, enc_args.warmup, enc_args.cpu_seconds = 10, 3, min(args.cpu_seconds, 5.0)
+            enc_args.dump_outputs = None
             out["encode"] = bench_encode(enc_args, rank, world, local)
     else:
         out = bench_encode(args, rank, world, local)

@@ -45,7 +45,8 @@ def load_traffic():
         return None
 
 
-def run(args, rank, world, local, ClockSampler, load_peaks, barrier, max_over_ranks):
+def run(args, rank, world, local, ClockSampler, load_peaks, barrier, max_over_ranks, dump=None):
+    """`dump`: None, or a callable that receives, by name, the arrays the last timed step produced (bench.py --dump-outputs)."""
     import numpy as np
     import torch
     from matrix0_b200 import _native
@@ -84,6 +85,13 @@ def run(args, rank, world, local, ClockSampler, load_peaks, barrier, max_over_ra
     while Cycle.i % per_move:
         step()
     torch.cuda.synchronize()
+    last = {}
+    forward = sp._forward
+
+    def keep_last(planes):     # the last timed step's evaluator call, for `dump`: its input planes and its outputs
+        last["planes"] = planes.clone()
+        last["policy_logits"], last["value"] = forward(planes)
+        return last["policy_logits"], last["value"]
     c0 = sp.counters()
     l0 = int(lib.m0_launch_count())
     r0 = sp.graph_replays
@@ -93,7 +101,9 @@ def run(args, rank, world, local, ClockSampler, load_peaks, barrier, max_over_ra
     t0 = torch.cuda.Event(enable_timing=True)
     t1 = torch.cuda.Event(enable_timing=True)
     t0.record(stream)
-    for _ in range(args.steps):
+    for i in range(args.steps):
+        if dump is not None and i == args.steps - 1:
+            sp._forward = keep_last
         step()
     t1.record(stream)
     barrier(world)
@@ -104,6 +114,16 @@ def run(args, rank, world, local, ClockSampler, load_peaks, barrier, max_over_ra
     launches = int(lib.m0_launch_count()) - l0 + (sp.graph_replays - r0) * sp.graph_kernels
     d = {k: c1[k] - c0[k] for k in c1}
     nn_rows = args.steps * G
+    if dump is not None:
+        # what a caller of the search receives after that step: the root statistics of every game (m0_search_result) and the
+        # move each game played last, beside the evaluator's input planes, policy logits and values of the step.  The games reach
+        # that step through moves this build searched and sampled, so two builds' outputs compare row by row where the planes agree.
+        sp._forward = forward
+        eng = sp.engine
+        eng.result(with_pi=True)
+        dump(dict(last, root_moves=eng.res_moves, root_move_count=eng.res_count, root_visits=eng.res_visits, root_child_q=eng.res_q,
+                  root_child_prior=eng.res_prior, root_pi=eng.res_pi, root_q=eng.res_root_q, root_n=eng.res_root_n,
+                  moves_played=sp.moves_played))
 
     def allsum(x):
         if world == 1:

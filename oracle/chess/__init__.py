@@ -2,7 +2,7 @@
 
 Matrix0 depends on the third-party PyPI package ``python-chess`` (import name ``chess``;
 ``requirements.txt:4`` pins ``python-chess[syzygy]>=1.9.0``, no lock file).  It is not vendored in
-``/root/reference`` and not installed in this image, so its *published* algorithm (python-chess
+the reference tree and not a dependency of this repository, so its *published* algorithm (python-chess
 1.9 - 1.11, ``chess/__init__.py``: bitboard board, ``generate_legal_moves`` ordering,
 ``_transposition_key``, game-end predicates) is restated here from its documented behaviour.
 The module is deliberately shaped as a drop-in ``chess`` module: with ``oracle/`` on ``sys.path``

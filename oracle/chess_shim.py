@@ -2,7 +2,7 @@
 
 If the real python-chess is installed it wins (then the oracle restatements are checked against
 the genuine third-party implementation); otherwise ``oracle/chess`` is registered under the name
-``chess`` so that both the oracle modules and -- on a box with /root/reference -- the unmodified
+``chess`` so that both the oracle modules and -- where the reference tree is present -- the unmodified
 reference modules import it.
 """
 import importlib.util

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- CPU restatement of ``azchess/encoding.py`` (numpy + oracle/chess).
 
-Every function cites the reference lines it follows.  Pinned (tests/test_oracle_pinning.py, run
-where /root/reference exists) against the unmodified reference module executed on the same shim,
+Every function cites the reference lines it follows.  Pinned (tests/test_oracle_chess.py, run
+where the reference tree is present) against the unmodified reference module executed on the same shim,
 and against the reference's own known-answer tests (tests/test_encoding.py, test_board_tensor.py)
 restated in tests/test_oracle_encoding.py.  Only tests/, smoke() and bench.py's CPU legs import it.
 """

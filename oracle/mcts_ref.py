@@ -9,7 +9,7 @@ softmax / float32 renormalisation of priors.
 Deterministic harness (SURVEY 7-0c): ``jitter_value=0.5`` plays the role of ``random.random()``
 patched to 0.5; Dirichlet / entropy noise / playout randomisation off; memory cleanups (wall-clock
 and RSS driven, Q6) are not modelled.  Pinned against the UNMODIFIED reference executed on the same
-shim in tests/test_oracle_pinning.py (build container) and through tests/golden/mcts_golden.json.
+shim in tests/test_oracle_mcts.py (where the reference tree is present) and through tests/golden/mcts_golden.json.
 Only tests/, smoke() and bench.py's CPU legs import this module.
 """
 from __future__ import annotations

@@ -3,7 +3,7 @@
 Plain PyTorch CPU ops on a reference-format ``state_dict`` (``azchess/model/resnet.py``), each step
 citing the reference lines it follows.  ``infer_amp_tower`` is forced off: this is the fp32 oracle
 (SURVEY Q11).  Pinned against the UNMODIFIED reference module (loaded with a stub ``chess``) in
-tests/test_oracle_nn.py where /root/reference exists, and through tests/golden/nn_golden.npz.
+tests/test_oracle_nn.py where the reference tree is present, and through tests/golden/nn_golden.npz.
 ``make_state_dict`` produces deterministic weights from the parameter names so that goldens need
 to store outputs only.  Only tests/, smoke() and bench.py's CPU legs import this module.
 """

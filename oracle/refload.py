@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- load the *unmodified* reference modules on top of the oracle shim.
 
-Only usable where ``/root/reference`` exists (the build container, never the GPU box).  Used by
+Only usable where an unmodified checkout of the reference project is present: at ``oracle/_ref`` (ignored by git) or at the
+directory named by ``MATRIX0_REFERENCE_ROOT``.  Used by
 ``tests/golden/make_golden.py`` to generate the committed golden vectors and by the ``not gpu``
 pinning tests that compare ``oracle/*_ref.py`` restatements with the real reference code.
 
@@ -19,8 +20,9 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("MATRIX0_REFERENCE_ROOT", "/root/reference")
 _ORACLE_DIR = os.path.dirname(os.path.abspath(__file__))
+REFERENCE_ROOT = os.environ.get("MATRIX0_REFERENCE_ROOT", os.path.join(_ORACLE_DIR, "_ref"))
+MISSING = "needs the unmodified reference tree (oracle/_ref or MATRIX0_REFERENCE_ROOT)"
 
 
 def reference_available() -> bool:

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- CPU restatement of the per-game loop of ``azchess/selfplay/internal.py:326-600`` and of
 ``azchess/draw.py`` around a search whose results are handed in (visit counts, pi, value), with the ``np.random`` draw of
 ``sample_move_from_counts`` supplied by the caller.  ``should_adjudicate_draw`` and ``sample_move_from_counts`` are pinned against
-the UNMODIFIED reference functions in tests/test_oracle_selfplay.py (build container).  Only tests/ import this module.
+the UNMODIFIED reference functions in tests/test_oracle_selfplay.py (stored answers, and live where the reference tree is present).  Only tests/ import this module.
 """
 from __future__ import annotations
 

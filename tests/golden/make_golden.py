@@ -1,7 +1,7 @@
 """Generate the committed golden vectors by running the UNMODIFIED reference modules
-(/root/reference/azchess/encoding.py, mcts.py) on top of the oracle chess shim.
+(azchess/encoding.py, mcts.py of the reference tree) on top of the oracle chess shim.
 
-Run in the build container only (needs /root/reference):  python tests/golden/make_golden.py
+Needs the unmodified reference tree (oracle/_ref or MATRIX0_REFERENCE_ROOT):  python tests/golden/make_golden.py
 Outputs (small, committed):
   tests/golden/encoding_golden.npz   positions + reference planes / move lists / policy indices
   tests/golden/tactical_kat.json     FEN + legal-move count + a legal move, sampled from the

@@ -1,4 +1,4 @@
-"""Golden arrays of SURVEY 8a row E6 from the UNMODIFIED reference (azchess/encoding.py:310-386), build container only:
+"""Golden arrays of SURVEY 8a row E6 from the UNMODIFIED reference (azchess/encoding.py:310-386), needs the reference tree:
     python tests/golden/make_permutation_golden.py  ->  tests/golden/permutations_golden.json"""
 import json
 import os

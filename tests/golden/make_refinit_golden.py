@@ -1,6 +1,6 @@
 """Golden vectors for the reduced-precision gate on the REFERENCE'S OWN random initialisation.
 
-Run in the build container only (needs /root/reference):  python tests/golden/make_refinit_golden.py
+Needs the unmodified reference tree (oracle/_ref or MATRIX0_REFERENCE_ROOT):  python tests/golden/make_refinit_golden.py
   tests/golden/refinit_digest.json   SHA-256 of every parameter tensor of the UNMODIFIED reference
                                      ``PolicyValueNet.from_config(config.yaml model + R24 overrides)`` built under
                                      ``torch.manual_seed(0)`` (pins matrix0_b200.model.reference_init)

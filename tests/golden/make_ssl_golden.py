@@ -1,6 +1,6 @@
 """Generate tests/golden/ssl_golden.npz by running the UNMODIFIED reference `azchess/ssl_algorithms.py`
 (`create_enhanced_ssl_targets`, called per played ply with a batch of ONE position by selfplay_worker, internal.py:460-466)
-on top of the oracle chess shim.  Build container only (needs /root/reference):  python tests/golden/make_ssl_golden.py
+on top of the oracle chess shim.  Needs the reference tree (oracle/_ref or MATRIX0_REFERENCE_ROOT):  python tests/golden/make_ssl_golden.py
 """
 import os
 import sys

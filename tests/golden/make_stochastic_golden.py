@@ -2,7 +2,7 @@
 (per-child per-simulation ``random.random()``, mcts.py:893-897), entropy noise (``np.random.normal(0, 0.1)``, :170-186), child
 pruning (:806-826) and the direct-model path (:697-703), fed SEEDED streams of random draws.
 
-Run in the build container only (needs /root/reference):  python tests/golden/make_stochastic_golden.py
+Needs the unmodified reference tree (oracle/_ref or MATRIX0_REFERENCE_ROOT):  python tests/golden/make_stochastic_golden.py
 Output: tests/golden/mcts_stochastic_golden.json
         python tests/golden/make_stochastic_golden.py vl   ->  tests/golden/mcts_vl_golden.json: the same with the reference's
         in-flight marking switched ON inside every mini-batch (the engine's throughput mode).  The reference ships that code in

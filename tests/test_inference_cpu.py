@@ -1,7 +1,7 @@
 """Host logic of the shared-memory evaluation seam (matrix0_b200/inference.py <-> azchess/selfplay/inference.py):
 mailbox layout, client time-outs / errors, the server sweep with a test evaluator, interoperability with the UNMODIFIED
-reference client and server where /root/reference is mounted, and the loud failure of the product entry point on a box
-without CUDA.  No compute of the product path runs here."""
+reference client and server where the reference tree is present (oracle/_ref or MATRIX0_REFERENCE_ROOT), and the loud failure
+of the product entry point on a box without CUDA.  No compute of the product path runs here."""
 import os
 import sys
 import threading
@@ -55,10 +55,14 @@ class ServerThread:
         assert not self.t.is_alive()
 
 
+# the reference's mailbox keys in its order (inference.py:18-35), as test_reference_client_against_our_server compares them live
+REFERENCE_KEYS = ("request_tensor", "response_policy_tensor", "response_value_tensor", "request_event", "response_event", "batch_size_tensor")
+
+
 def test_mailbox_layout():
     """inference.py:18-35 -- keys, shapes, dtypes, shared memory."""
     res = m0inf.setup_shared_memory_for_worker(3, PLANES, POLICY, 96)
-    assert tuple(res.keys()) == m0inf.RESOURCE_KEYS
+    assert tuple(res.keys()) == m0inf.RESOURCE_KEYS == REFERENCE_KEYS
     assert res["request_tensor"].shape == (96, PLANES, 8, 8) and res["request_tensor"].dtype == torch.float32
     assert res["response_policy_tensor"].shape == (96, POLICY) and res["response_policy_tensor"].dtype == torch.float32
     assert res["response_value_tensor"].shape == (96, 1) and res["response_value_tensor"].dtype == torch.float32
@@ -173,7 +177,7 @@ def test_product_server_fails_loudly_without_cuda():
     assert not ready.is_set()
 
 
-# ---- interoperability with the unmodified reference module (build container only) --------------------------------
+# ---- interoperability with the unmodified reference module (where the reference tree is present) --------------------
 def _reference_inference():
     resnet = refload.load_reference("model.resnet")
     sys.modules["azchess.model"].PolicyValueNet = resnet.PolicyValueNet       # what azchess/model/__init__.py exports
@@ -182,7 +186,7 @@ def _reference_inference():
     return importlib.import_module("azchess.selfplay.inference"), resnet
 
 
-needs_reference = pytest.mark.skipif(not refload.reference_available(), reason="reference tree not mounted")
+needs_reference = pytest.mark.skipif(not refload.reference_available(), reason=refload.MISSING)
 
 
 @needs_reference

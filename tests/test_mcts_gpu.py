@@ -117,14 +117,13 @@ def test_root_children_follow_python_chess_order_on_edge_positions():
     eng.close()
 
 
-def test_configs0_single_game_through_the_dropin_search_object(tmp_path):
+def test_configs0_single_game_through_the_dropin_search_object():
     """BASELINE configs[0] on the GPU: ONE game from the start position, 800 simulations per move, ResNet-24 random init, searched by
     `MCTS(cfg, model, device="cuda").run(board)` move after move -- the call `selfplay_worker` / `arena.py` / `cli_play.py` of the reference
     make (one board per call, host dictionaries back).  The latency case: ten evaluator calls of <= 96 rows per move and nothing to batch
-    across games.  The numbers go to gpurun_out/single_game.json (copied to profiles/); the assertion is only a floor well above the
+    across games.  The numbers are printed as one JSON line (shown with `pytest -s`); the assertion is only a floor well above the
     reference's CPU rate on the same configuration (65 ... 450 sims/s, `bench.py --impl reference`)."""
     import json
-    import os
     import time
     import torch
     from bench_selfplay import reference_cfg
@@ -155,7 +154,4 @@ def test_configs0_single_game_through_the_dropin_search_object(tmp_path):
                      "sims_per_s": sims / total, "positions_per_s": len(per_move) / total}
         mcts.shutdown()
         assert sims / total > 2000.0, out[name]
-    root = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "gpurun_out")
-    os.makedirs(root, exist_ok=True)
-    with open(os.path.join(root, "single_game.json"), "w") as f:
-        json.dump(out, f, indent=1)
+    print(json.dumps(out))

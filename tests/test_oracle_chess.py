@@ -1,5 +1,5 @@
 """Pin the oracle python-chess restatement: public perft constants, the reference's tactical KAT
-(legal-move counts), its encoding known-answer tests, and -- when /root/reference is present --
+(legal-move counts), its encoding known-answer tests, and -- when the reference tree is present --
 the full fixture sweep (10k/40k/5k FENs, 140 PGN games)."""
 import glob
 import json
@@ -119,8 +119,8 @@ def test_ref_kat_fools_mate_fen():  # tests/test_error_handling.py:146
     assert b.is_checkmate() and b.is_game_over() and b.result() == "0-1"
 
 
-# ---- full sweep against the reference's data fixtures (build container only) ---------------------
-needs_ref = pytest.mark.skipif(not refload.reference_available(), reason="/root/reference not present")
+# ---- full sweep against the reference's data fixtures (where the reference tree is present) ------
+needs_ref = pytest.mark.skipif(not refload.reference_available(), reason=refload.MISSING)
 
 
 @needs_ref
@@ -168,7 +168,7 @@ def test_reference_fixture_sweep():
 
 @needs_ref
 def test_restatement_matches_unmodified_reference():
-    """oracle/encoding_ref == /root/reference/azchess/encoding.py executed on the same boards."""
+    """oracle/encoding_ref == the reference tree's azchess/encoding.py executed on the same boards."""
     from conftest import random_playout_boards
     enc = refload.load_reference("encoding")
     for b in random_playout_boards(12, 120, seed=11):

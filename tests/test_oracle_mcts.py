@@ -1,5 +1,5 @@
 """The oracle search restatement (oracle/mcts_ref.py) reproduces the committed golden vectors that
-the UNMODIFIED reference MCTS produced (tests/golden/make_golden.py), and -- where /root/reference
+the UNMODIFIED reference MCTS produced (tests/golden/make_golden.py), and -- where the reference tree
 exists -- is compared live with the reference on further seeds."""
 import logging
 
@@ -21,7 +21,7 @@ def test_oracle_reproduces_reference_goldens():
     assert run_all(make_ref, prior_rtol=0.0) >= 80
 
 
-@pytest.mark.skipif(not refload.reference_available(), reason="/root/reference not present")
+@pytest.mark.skipif(not refload.reference_available(), reason=refload.MISSING)
 def test_oracle_matches_unmodified_reference_live():
     logging.disable(logging.CRITICAL)
     try:

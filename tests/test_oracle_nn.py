@@ -1,5 +1,5 @@
 """The functional fp32 NN restatement (oracle/nn_ref.py) reproduces the committed outputs of the
-UNMODIFIED reference PolicyValueNet (tests/golden/nn_golden.npz) and, where /root/reference exists,
+UNMODIFIED reference PolicyValueNet (tests/golden/nn_golden.npz) and, where the reference tree is present,
 is compared live with the reference module."""
 import json
 import os
@@ -32,7 +32,7 @@ def test_restatement_reproduces_reference_outputs(golden_dir, name):
         assert np.abs(s.numpy() - g[f"{name}_ssl_{t}"]).max() < 2e-5
 
 
-@pytest.mark.skipif(not refload.reference_available(), reason="/root/reference not present")
+@pytest.mark.skipif(not refload.reference_available(), reason=refload.MISSING)
 def test_restatement_matches_reference_module_live(golden_dir):
     resnet = refload.load_reference("model.resnet")
     g, cfg, sd = load_case(golden_dir, "small")
@@ -68,7 +68,7 @@ def test_reference_init_matches_committed_digests(golden_dir):
         assert hashlib.sha256(sd[k].contiguous().numpy().tobytes()).hexdigest() == d["sha256"][k], k
 
 
-@pytest.mark.skipif(not refload.reference_available(), reason="/root/reference not present")
+@pytest.mark.skipif(not refload.reference_available(), reason=refload.MISSING)
 def test_reference_init_matches_reference_module_live(golden_dir):
     from matrix0_b200.model import reference_init
     resnet = refload.load_reference("model.resnet")

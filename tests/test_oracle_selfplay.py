@@ -1,75 +1,56 @@
 """oracle/selfplay_ref.py (restatements of azchess/draw.py and of sample_move_from_counts, azchess/selfplay/internal.py:690-735)
-against the UNMODIFIED reference code, where /root/reference exists."""
-import ast
-import os
-import random
-
+against the reference's stored answers (tests/golden/selfplay_golden.json) and, where the unmodified reference tree is present,
+against the reference code itself."""
 import numpy as np
 import pytest
 
 import chess
+import selfplay_cases as C
 from oracle import refload, selfplay_ref as R
 
-pytestmark = pytest.mark.skipif(not refload.reference_available(), reason="/root/reference not present")
+needs_ref = pytest.mark.skipif(not refload.reference_available(), reason=refload.MISSING)
 
 
-def _reference_function(rel_path, name):
-    """Compile ONE top-level function of a reference file unmodified (selfplay/internal.py cannot be imported as a module here: its
-    imports pull in the data manager / orchestrator stack)."""
-    src = open(os.path.join(refload.REFERENCE_ROOT, rel_path)).read()
-    tree = ast.parse(src)
-    fn = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == name)
-    from typing import Dict
-    ns = {"np": np, "chess": chess, "Dict": Dict}
-    exec(compile(ast.Module(body=[fn], type_ignores=[]), rel_path, "exec"), ns)
-    return ns[name]
+def test_should_adjudicate_draw_matches_reference_goldens():
+    g = C.load()["draw"]
+    assert g["cfgs"] == C.DRAW_CFGS
+    games = [[chess.Move.from_uci(u) for u in game] for game in g["games"]]
+    got = "".join("1" if R.should_adjudicate_draw(b, moves, cfg) else "0" for b, moves, cfg in C.draw_cases(games))
+    assert got == g["decisions"]
+    assert len(got) > 5000 and 200 < got.count("1") < len(got) - 200
 
 
+def test_sample_move_from_counts_matches_reference_goldens():
+    g = C.load()["sample"]
+    moves = list(chess.Board(g["fen"]).legal_moves)
+    assert len(g["trials"]) == 400
+    for t in g["trials"]:
+        got = R.sample_move_from_counts(moves[:t["moves"]], t["counts"], t["temperature"], C.uniform(t["seed"]))
+        assert got == t["choice"], t
+
+
+@needs_ref
 def test_should_adjudicate_draw_matches_reference():
     ref = refload.load_reference("draw").should_adjudicate_draw
-    rng = random.Random(5)
-    cfgs = [{}, {"enabled": True}, {"enabled": True, "min_plies": 6, "window": 6, "min_unique": 5, "halfmove_cap": 5, "material_draw_threshold": 76},
-            {"enabled": True, "min_plies": 0, "window": 4, "min_unique": 3, "halfmove_cap": 0, "material_draw_threshold": 0},
-            {"enabled": True, "min_plies": 10, "window": 0, "min_unique": 3, "halfmove_cap": 8, "material_draw_threshold": 60, "stalemate_draw": False}]
     n = hits = 0
-    for game in range(40):
-        b = chess.Board()
-        moves = []
-        for ply in range(rng.randint(5, 120)):
-            if b.is_game_over():
-                break
-            legal = list(b.legal_moves)
-            # shuffling knights makes repetitions and low-uniqueness windows likely
-            back = [m for m in legal if moves and m.from_square == moves[-2].to_square and m.to_square == moves[-2].from_square] if len(moves) >= 2 else []
-            m = back[0] if back and rng.random() < 0.5 else rng.choice(legal)
-            b.push(m)
-            moves.append(m)
-            for cfg in cfgs:
-                want = ref(b, moves, cfg)
-                assert R.should_adjudicate_draw(b, moves, cfg) == want, (b.fen(), cfg)
-                n += 1
-                hits += bool(want)
+    for b, moves, cfg in C.draw_cases(C.draw_games()):
+        want = ref(b, moves, cfg)
+        assert R.should_adjudicate_draw(b, moves, cfg) == want, (b.fen(), cfg)
+        n += 1
+        hits += bool(want)
     assert n > 5000 and 200 < hits < n - 200
 
 
+@needs_ref
 def test_sample_move_from_counts_matches_reference():
-    ref = _reference_function("azchess/selfplay/internal.py", "sample_move_from_counts")
-    rng = random.Random(9)
-    b = chess.Board("r3k2r/p1ppqpb1/bn2pnp1/3PN3/1p2P3/2N2Q1p/PPPBBPPP/R3K2R w KQkq - 0 1")
-    moves = list(b.legal_moves)
+    ref = C.reference_function("azchess/selfplay/internal.py", "sample_move_from_counts")
+    b = chess.Board(C.SAMPLE_FEN)
     n = 0
-    for trial in range(400):
-        k = rng.randint(1, len(moves))
-        counts = {m: (rng.randint(0, 300) if rng.random() < 0.8 else 0) for m in moves[:k]}
-        if not any(counts.values()):
-            counts[moves[0]] = 1
-        T = rng.choice([1.2, 1.0, 0.75, 0.3, 0.1, 0.0005])
-        seed = 1000 + trial
-        np.random.seed(seed)
-        u = np.random.random_sample()
+    for counts, T, seed in C.sample_trials():
+        u = C.uniform(seed)
         np.random.seed(seed)
         want = ref(b, counts, T)
         got = R.sample_move_from_counts(list(counts.keys()), list(counts.values()), T, u)
-        assert list(counts.keys())[got] == want, (trial, T)
+        assert list(counts.keys())[got] == want, (seed, T)
         n += 1
     assert n == 400

@@ -1,5 +1,5 @@
 """oracle/ssl_ref.py (numpy restatement of azchess/ssl_algorithms.py) against the golden vectors generated from the unmodified
-reference module (tests/golden/make_ssl_golden.py), and -- where /root/reference exists -- against the module itself."""
+reference module (tests/golden/make_ssl_golden.py), and -- where the reference tree is present -- against the module itself."""
 import os
 
 import numpy as np
@@ -25,7 +25,7 @@ def test_ssl_oracle_matches_reference_goldens(golden):
 def test_ssl_oracle_matches_live_reference():
     from oracle import refload
     if not refload.reference_available():
-        pytest.skip("reference tree not mounted")
+        pytest.skip(refload.MISSING)
     import torch
     enc, ssl = refload.load_reference("encoding", "ssl_algorithms")
     from conftest import random_playout_boards
