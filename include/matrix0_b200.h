@@ -158,6 +158,14 @@ int m0_search_multi_encode(m0_engine* e, int g0, int g1, int row0, int mode, flo
  * their samples, so an evaluator batch of row_cap rows can be launched before the host has read the row numbering */
 int m0_search_expand_backup_multi(m0_engine* e, int g0, int g1, const float* d_logits, int logits_stride, const float* d_values, int row0,
                                   int per_sample, int row_cap, void* stream);
+/* ---- reuse of the root's evaluation across moves: a store of `slots` (1..64) entries per game keeps the network output of every
+ * evaluated child of the root; the next m0_search_begin expands a root whose packed position (all 9 words) equals a stored one from
+ * that entry.  The other roots needing an evaluation are ALSO written in compact rows to d_miss_planes float32[G][19][8][8], their
+ * count to d_miss_count int32[1], and m0_search_expand_backup reads their outputs from the evaluator rows 0..count-1 of d_logits /
+ * d_values.  Both buffers are the caller's and must stay alive.  Entries belong to the network that produced them: clear the store
+ * when the evaluator changes.  Counter 12 counts the roots expanded from the store. */
+int m0_search_reuse_enable(m0_engine* e, int slots, float* d_miss_planes, int32_t* d_miss_count);
+int m0_search_reuse_clear(m0_engine* e, void* stream);
 int m0_engine_counters(m0_engine* e, unsigned long long* h_out16); /* host buffer; synchronises */
 int m0_engine_status(m0_engine* e, int32_t* d_status_out, int32_t* d_node_count_out, void* stream);
 

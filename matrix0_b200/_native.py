@@ -55,6 +55,8 @@ SIGNATURES = {
     "m0_search_select_multi": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "m0_search_multi_encode": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
     "m0_search_expand_backup_multi": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "m0_search_reuse_enable": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
+    "m0_search_reuse_clear": (c_int, [c_void_p, c_void_p]),
     "m0_engine_counters": (c_int, [c_void_p, c_void_p]),
     "m0_engine_status": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "m0_search_select_var": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),

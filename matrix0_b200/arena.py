@@ -20,6 +20,8 @@ from .selfplay import SelfPlayEngine
 
 @_native.on_own_device
 class _TwoEvaluatorGames(SelfPlayEngine):
+    reuse_root_evals = False      # the root's children were evaluated by the other player's network
+
     def __init__(self, model_a, model_b, *args, **kw):
         super().__init__(model_a, *args, **kw)
         import torch

@@ -18,7 +18,8 @@ enum { ST_NODE_OVERFLOW = 1, ST_TT_OVERFLOW = 2, ST_DEPTH_CAP = 4, ST_HIST_OVERF
 // counters
 enum { CTR_SIMS = 0, CTR_TERMINAL_SIMS, CTR_NN_EVALS, CTR_EXPANSIONS, CTR_TT_HOPS, CTR_CHILDREN_SCANNED,
        CTR_PATH_NODES, CTR_CHILDREN_CREATED, CTR_GAMES_FINISHED, CTR_POSITIONS_PLAYED, CTR_NOISY_EXPANSIONS, CTR_LEAF_SAMPLES,
-       CTR_COUNT = 16 };
+       CTR_ROOT_REUSED, CTR_COUNT = 16 };
+static constexpr int REUSE_MAX_SLOTS = 64;   // stored root children per game (the root's warp compares 32 at a time)
 
 struct SearchParams {
   double fpu_reduction;     // mcts.py:868-869
@@ -105,6 +106,17 @@ struct EngineView {
   int* ml_row_base;       // [G + 1] exclusive prefix of ml_n_leaves: compact network rows
   u16* node_inflight;     // [G][max_nodes] in-flight selections of an edge child within the current mini-batch (virtual loss)
   double* full_scratch;   // [G][4672] entropy noise over the FULL policy vector (legal_softmax = false, mcts.py:164-186); else NULL
+  // network outputs of the root's children, kept for the next move (m0_search_reuse_enable; rc_slots = 0: not enabled).  The next
+  // root is the child that was played, and a row's output is a function of its packed position alone, so a stored entry whose
+  // position equals the new root is exactly what a second evaluation would return.
+  int rc_slots;           // entries per game (<= REUSE_MAX_SLOTS)
+  int* rc_fill;           // [G] entries recorded since the last search_begin
+  u64* rc_pos;            // [G][rc_slots][9]
+  float* rc_logits;       // [G][rc_slots][4672]
+  float* rc_value;        // [G][rc_slots] value as the network returned it (before clipping)
+  int* rc_src;            // [G] where the root expansion reads its row: entry s -> -1 - s, compact miss row r -> r
+  float* rc_miss_planes;  // [G][19][8][8] caller's buffer: planes of the roots found in no entry, in compact rows
+  int* rc_miss_count;     // [1] caller's counter: rows written to rc_miss_planes by the last search_begin
 };
 
 static constexpr u32 MOVE_NONE = 0xFFFFu;

@@ -195,8 +195,11 @@ static inline int tree_blocks(const m0_engine* e) { return (e->v.G + TREE_WARPS 
 
 // MCTS.run prologue (mcts.py:336-371): d_info int32[G] (bit0 terminal root, bit1 needs evaluation),
 // d_value float64[G] terminal value; d_planes float32[G][19][8][8] receives the roots to evaluate.
+// With the store of m0_search_reuse_enable, a root found among the stored entries is expanded from that entry and the other roots
+// are also written, in compact rows, to the miss buffer (the miss counter gives the row count).
 int m0_search_begin(m0_engine* e, float* d_planes, int32_t* d_info, double* d_value, void* stream) {
   if (!e || !d_info || !d_value) { m0_set_error("m0_search_begin: invalid argument"); return M0_ERR_ARG; }
+  if (e->v.rc_slots) M0_CUDA_TRY(cudaMemsetAsync(e->v.rc_miss_count, 0, sizeof(int), (cudaStream_t)stream));
   search_begin_kernel<<<tree_blocks(e), TREE_WARPS * 32, 0, (cudaStream_t)stream>>>(e->v, d_planes, d_info, d_value);
   return m0_check_launch("m0_search_begin");
 }
@@ -340,6 +343,38 @@ int m0_search_expand_backup_multi(m0_engine* e, int g0, int g1, const float* d_l
   search_expand_backup_multi_kernel<<<(g1 - g0 + TREE_WARPS - 1) / TREE_WARPS, TREE_WARPS * 32, 0, (cudaStream_t)stream>>>(
       e->v, g0, g1, d_logits, logits_stride, d_values, row0, per_sample, per_sample ? 0 : row_cap);
   return m0_check_launch("m0_search_expand_backup_multi");
+}
+
+// ---- reuse of the root's evaluation across moves ------------------------------------------------------------------------------------
+// Allocates a store of `slots` (1..64) entries per game: the expansion kernels keep the network output of every evaluated child of the
+// root, and the next m0_search_begin expands a root whose packed position equals a stored one from that entry instead of asking for an
+// evaluation.  Roots without an entry go to d_miss_planes float32[G][19][8][8] in compact rows, counted in d_miss_count int32[1]; the
+// expansion then reads the evaluator's row r for the root written to row r.  The two caller buffers must stay alive.  The entries are
+// the outputs of the network that produced them: m0_search_reuse_clear must be called when the evaluator changes.
+int m0_search_reuse_enable(m0_engine* e, int slots, float* d_miss_planes, int32_t* d_miss_count) {
+  if (!e || slots <= 0 || slots > REUSE_MAX_SLOTS || !d_miss_planes || !d_miss_count) { m0_set_error("m0_search_reuse_enable: invalid argument"); return M0_ERR_ARG; }
+  if (e->v.rc_slots && e->v.rc_slots != slots) { m0_set_error("m0_search_reuse_enable: already enabled with %d slots", e->v.rc_slots); return M0_ERR_STATE; }
+  EngineView& v = e->v;
+  if (!v.rc_slots) {
+    m0::DeviceGuard device_guard(e->device);
+    M0_CUDA_TRY(device_guard.err);
+    const size_t G = v.G, S = G * (size_t)slots;
+    TRY(dev_alloc(e, &v.rc_fill, G));
+    TRY(dev_alloc(e, &v.rc_pos, S * POSITION_WORDS, false));
+    TRY(dev_alloc(e, &v.rc_logits, S * POLICY_SIZE, false));
+    TRY(dev_alloc(e, &v.rc_value, S, false));
+    TRY(dev_alloc(e, &v.rc_src, G, false));
+    v.rc_slots = slots;
+  }
+  v.rc_miss_planes = d_miss_planes;
+  v.rc_miss_count = d_miss_count;
+  return M0_OK;
+}
+
+// Forgets every stored entry (the evaluator's weights changed, or a caller wants every root evaluated again).
+int m0_search_reuse_clear(m0_engine* e, void* stream) {
+  if (!e || !e->v.rc_slots) { m0_set_error("m0_search_reuse_clear: invalid argument (store not enabled)"); return M0_ERR_ARG; }
+  return m0_check_cuda(cudaMemsetAsync(e->v.rc_fill, 0, sizeof(int) * e->v.G, (cudaStream_t)stream), "m0_search_reuse_clear");
 }
 
 // Engine counters (uint64[16], see engine.cuh CTR_*) and sticky per-game status bits (int32[G])

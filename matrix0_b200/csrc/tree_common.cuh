@@ -355,4 +355,30 @@ __device__ __forceinline__ void warp_expand(const EngineView& E, const SearchPar
   __syncwarp();
 }
 
+// Keeps the network output of a child of the root (a leaf at path length 2) for the next move's root (EngineView::rc_*): the
+// logits row, the value as the network returned it and the packed position.  A full store records nothing more; the next root is
+// then evaluated again, which gives the same result.
+__device__ __forceinline__ void warp_record_root_child(const EngineView& E, int g, const u64* pos_words, const float* __restrict__ lg,
+                                                       float value, int lane) {
+  const int n = E.rc_fill[g];
+  if (n >= E.rc_slots) return;
+  const size_t e = (size_t)g * E.rc_slots + n;
+  float* dst = E.rc_logits + e * POLICY_SIZE;
+  if ((reinterpret_cast<uintptr_t>(lg) & 15) == 0) {
+    const float4* s4 = reinterpret_cast<const float4*>(lg);
+    float4* d4 = reinterpret_cast<float4*>(dst);
+#pragma unroll 4
+    for (int i = lane; i < POLICY_SIZE / 4; i += 32) d4[i] = __ldg(s4 + i);
+  } else {
+    for (int i = lane; i < POLICY_SIZE; i += 32) dst[i] = lg[i];
+  }
+  if (lane < POSITION_WORDS) E.rc_pos[e * POSITION_WORDS + lane] = pos_words[lane];
+  __syncwarp();
+  if (lane == 0) {
+    E.rc_value[e] = value;
+    E.rc_fill[g] = n + 1;
+  }
+  __syncwarp();
+}
+
 }  // namespace m0

@@ -103,6 +103,7 @@ search_begin_kernel(EngineView E, float* __restrict__ planes, int* __restrict__ 
       E.pend_flags[g] = 0;
       E.pend_count[g] = 0;
       E.root_node[g] = -1;
+      if (E.rc_slots) E.rc_fill[g] = 0;
     }
     return;
   }
@@ -155,7 +156,35 @@ search_begin_kernel(EngineView E, float* __restrict__ planes, int* __restrict__ 
       store_position(E.leaf_pos + (size_t)g * POSITION_WORDS, pos);
     }
     if (planes) warp_write_planes(pos, planes + (size_t)g * (19 * 64), lane);
+    if (E.rc_slots) {
+      // the root among the children evaluated during the previous move (all 9 words: pieces, side to move, castling, clocks)?
+      // hit: the expansion reads that entry; miss: the root's planes go to the next compact row of the caller's miss buffer
+      const u64* rw = E.root_pos + (size_t)g * POSITION_WORDS;
+      const int fill = E.rc_fill[g];
+      int src = 0;
+      bool hit = false;
+      for (int e0 = 0; e0 < fill && !hit; e0 += 32) {   // one entry per lane
+        const u64* ew = E.rc_pos + ((size_t)g * E.rc_slots + e0 + lane) * POSITION_WORDS;
+        bool eq = e0 + lane < fill;
+        for (int w = 0; w < POSITION_WORDS && eq; ++w) eq = ew[w] == rw[w];
+        const unsigned hits = __ballot_sync(FULL, eq);
+        if (hits) {
+          hit = true;
+          src = -1 - (e0 + __ffs(hits) - 1);
+        }
+      }
+      if (hit) {
+        if (lane == 0) atomicAdd(&E.counters[CTR_ROOT_REUSED], 1ull);
+      } else {
+        int row = 0;
+        if (lane == 0) row = atomicAdd(E.rc_miss_count, 1);
+        src = __shfl_sync(FULL, row, 0);
+        warp_write_planes(pos, E.rc_miss_planes + (size_t)src * (19 * 64), lane);
+      }
+      if (lane == 0) E.rc_src[g] = src;
+    }
   }
+  if (E.rc_slots && lane == 0) E.rc_fill[g] = 0;   // this move records its own root children
 }
 
 // ---- selection: azchess/mcts.py:742-769 (_collect_leaf_position) + :851-925 (_select) ----------------------
@@ -321,8 +350,26 @@ search_expand_backup_kernel(EngineView E, const float* __restrict__ logits, int 
   const int node = E.pend_node[g];
   const int times = E.pend_count[g];
   const Position pos = load_position(E.leaf_pos + (size_t)g * POSITION_WORDS);
+  // the game's network row: row g, or for a root evaluation with the store enabled, the entry or compact row search_begin chose.
+  // Row g is read only in the branch that uses it: the root evaluation's buffers hold just the compact rows (or none at all).
+  const float* lg;
+  float vf;
+  if ((flags & PEND_ROOT) && E.rc_slots) {
+    const int src = E.rc_src[g];
+    if (src < 0) {
+      const size_t e = (size_t)g * E.rc_slots + (-1 - src);
+      lg = E.rc_logits + e * POLICY_SIZE;
+      vf = E.rc_value[e];
+    } else {
+      lg = logits + (size_t)src * logits_stride;
+      vf = values[src];
+    }
+  } else {
+    lg = logits + (size_t)g * logits_stride;
+    vf = values[g];
+    if (E.rc_slots && E.path_len[g] == 2) warp_record_root_child(E, g, E.leaf_pos + (size_t)g * POSITION_WORDS, lg, vf, lane);
+  }
   // value: float(np.clip(value, -1, 1)) (mcts.py:668) ; _infer clips the same way (:1180)
-  float vf = values[g];
   vf = fminf(fmaxf(vf, -1.0f), 1.0f);
   double v = (double)vf;
   if ((flags & PEND_ROOT) && P.value_from_white && !pos_turn(pos)) v = -v;  // mcts.py:1184-1186
@@ -330,7 +377,7 @@ search_expand_backup_kernel(EngineView E, const float* __restrict__ logits, int 
   const int k = E.leaf_n[g];
   if ((flags & PEND_EXPAND) && E.node_first[nb + node] < 0 && k > 0)
     warp_expand(E, P, g, node, pos, E.leaf_moves + (size_t)g * MAX_MOVES, E.leaf_idx + (size_t)g * MAX_MOVES, k,
-                logits + (size_t)g * logits_stride, (flags & PEND_REGISTER) != 0, (flags & PEND_ROOT) != 0, s_x[wib], lane);
+                lg, (flags & PEND_REGISTER) != 0, (flags & PEND_ROOT) != 0, s_x[wib], lane);
   if ((flags & PEND_SET_Q) && lane == 0) E.node_q[nb + node] = v;  // root.q = v (mcts.py:412-413)
   __syncwarp();
   if (times > 0) warp_backup(E, g, E.path_len[g], py_clip_unit(v), times, lane);

@@ -302,6 +302,9 @@ search_expand_backup_multi_kernel(EngineView E, int g0, int g1, const float* __r
       __syncwarp();
       const long long lrow = base + (per_sample ? leaf_first[r] : r);
       if (k > 0) warp_expand(E, P, g, node, pos, s_moves[wib], s_idx[wib], k, logits + (size_t)lrow * logits_stride, true, false, s_x[wib], lane);
+      if (E.rc_slots && smp_len[s] == 2)
+        warp_record_root_child(E, g, E.ml_leaf_pos + ((size_t)g * E.ml_cap + r) * POSITION_WORDS, logits + (size_t)lrow * logits_stride,
+                               values[lrow], lane);
     }
     // Consecutive samples with the same leaf row and the same path (the common case: a mini-batch mostly repeats one path) back the same
     // value up the same nodes: `run` sequential backups collapse into one pass that performs the same `run` additions per node in the same

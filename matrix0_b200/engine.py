@@ -15,7 +15,7 @@ from . import _native
 from .boards import MAX_MOVES, PLANES, POLICY_SIZE, POSITION_WORDS, board_to_raw, move_to_code
 
 COUNTER_NAMES = ["sims", "terminal_sims", "nn_evals", "expansions", "tt_hops", "children_scanned", "path_nodes",
-                 "children_created", "games_finished", "positions_played", "noisy_expansions", "leaf_samples"]
+                 "children_created", "games_finished", "positions_played", "noisy_expansions", "leaf_samples", "root_evals_reused"]
 ST_NODE_OVERFLOW, ST_TT_OVERFLOW, ST_DEPTH_CAP, ST_HIST_OVERFLOW, ST_STREAM_EXHAUSTED = 1, 2, 4, 8, 16
 
 
@@ -193,6 +193,20 @@ class SearchEngine:
         self.ml_cap = int(samples_per_batch)
         self.row_base = torch.zeros((self.G + 1,), dtype=torch.int32, device=self.device)
         self.n_samples = torch.zeros((self.G,), dtype=torch.int32, device=self.device)
+
+    # ---- reuse of the root's evaluation across moves -------------------------------------------------------------------------
+    def enable_reuse(self, slots: int) -> None:
+        """Keep the network outputs of the root's children (``slots`` per game) for the next ``begin``.  Afterwards ``begin`` also
+        writes the roots found in no entry to ``miss_planes`` in compact rows (``miss_count`` rows), and ``expand_backup`` of the root
+        evaluation takes the evaluator's outputs for those rows."""
+        import torch
+        self.miss_planes = torch.zeros((self.G, PLANES, 8, 8), dtype=torch.float32, device=self.device)
+        self.miss_count = torch.zeros((1,), dtype=torch.int32, device=self.device)
+        _native.check(self._lib.m0_search_reuse_enable(self._h, int(slots), self.miss_planes.data_ptr(), self.miss_count.data_ptr()),
+                      "m0_search_reuse_enable")
+
+    def clear_reuse(self) -> None:
+        _native.check(self._lib.m0_search_reuse_clear(self._h, self._stream()), "m0_search_reuse_clear")
 
     def set_streams(self, jitter=None, normal=None) -> None:
         """jitter / normal: float64 [G, n] device tensors holding the values ``random.random()`` / ``np.random.normal(0, 0.1)``

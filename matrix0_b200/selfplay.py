@@ -2,7 +2,7 @@
 
 ``SelfPlayEngine`` keeps G games on one GPU and advances all of them in lock step:
 
-    per move :  trees_clear -> search_begin -> NN(root) -> expand           (MCTS.run prologue)
+    per move :  trees_clear -> search_begin -> NN(roots not kept) -> expand (MCTS.run prologue)
                 [select -> NN(leaves) -> expand+backup]  x ceil(sims / inference_batch_size)
                 selfplay_advance (sample move, resign, push, finish / restart games)
 
@@ -85,6 +85,11 @@ def resolve_mcts_config(cfg_dict: Dict[str, Any]) -> MCTSConfig:
 
 @_native.on_own_device
 class SelfPlayEngine:
+    # The root of a move is the child played at the previous move, and that child was evaluated during the previous search (a child
+    # with visits reached its position at least once; only a terminal child has no row, and then the game ends).  The engine keeps
+    # the network outputs of the root's children and expands the next root from them instead of evaluating it again.
+    reuse_root_evals = True
+
     def __init__(self, model, cfg_dict: Dict[str, Any], games: int = 4096, device: Optional[int] = None, deterministic: bool = False,
                  seed: int = 1234, precision: Optional[str] = None, max_nodes: Optional[int] = None, cuda_graph: bool = True,
                  search_mode: str = "collapsed", forward_rows: Optional[int] = None):
@@ -135,6 +140,15 @@ class SelfPlayEngine:
                 # evaluator batch sizes: full chunks of forward_rows rows, the tail chunk in the smallest size that holds it
                 self.forward_sizes = sorted({self.forward_rows} | {s for s in (256, 512, 1024, 2048) if bs <= s < self.forward_rows})
                 self.ml_planes = torch.zeros((self.forward_rows, 19, 8, 8), dtype=torch.float32, device=self.device)
+            if self.reuse_root_evals:
+                # collapsed: one evaluated leaf per game and mini-batch, so at most batches_per_move() root children per move; the
+                # multi-leaf modes evaluate ~12 rows per game and move at all depths together (a full store only makes a later miss)
+                self.engine.enable_reuse(32 if search_mode == "as_shipped" else min(32, self.batches_per_move()))
+                # evaluator batch sizes of the roots that are not kept (new games, a child the store had no room for)
+                self.root_sizes = sorted({self.G} | {s for s in (256, 512, 1024, 2048) if s < self.G})
+                self._no_rows = (torch.zeros((1, 4672), dtype=torch.float32, device=self.device),
+                                 torch.zeros((1,), dtype=torch.float32, device=self.device))
+                self._reuse_epoch = model.ws_epoch
             s = SelfPlayConfigStruct()
             s.temperature_start = float(self.sp.get("temperature_start", 1.0))
             s.temperature_end = float(self.sp.get("temperature_end", 0.1))
@@ -237,8 +251,21 @@ class SelfPlayEngine:
         import torch
         eng = self.engine
         _native.check(self._lib.m0_trees_clear(eng._h, _native.current_stream()), "m0_trees_clear")
-        eng.begin()
-        logits, values = self._forward(eng.planes)
+        if not self.reuse_root_evals:
+            eng.begin()
+            logits, values = self._forward(eng.planes)
+        else:
+            if self.model.ws_epoch != self._reuse_epoch:       # new weights (or only new workspaces): the kept outputs may be stale
+                eng.clear_reuse()
+                self._reuse_epoch = self.model.ws_epoch
+            eng.begin()
+            n = int(eng.miss_count.item())
+            if n:
+                size = next(s for s in self.root_sizes if s >= n)
+                logits, values = self._forward(eng.miss_planes[:size])
+                self.nn_rows += n - size
+            else:
+                logits, values = self._no_rows                      # every root is expanded from a kept output
         eng.expand_backup(logits, values)
         if not self.deterministic and float(self.mcfg.dirichlet_frac) > 0:
             _native.check(self._lib.m0_selfplay_plies(eng._h, self.plies.data_ptr(), _native.current_stream()), "m0_selfplay_plies")
@@ -281,10 +308,11 @@ class SelfPlayEngine:
     def warm_up_forward(self) -> None:
         """Capture the evaluator graphs of every batch size this engine uses (one-off cost of ~1 s per size, otherwise paid inside the
         first move that needs the size)."""
-        if self.search_mode != "as_shipped":
-            return
-        for size in sorted(self.forward_sizes, reverse=True):
-            self._forward(self.ml_planes[:size])
+        calls = [(self.ml_planes, s) for s in self.forward_sizes] if self.search_mode == "as_shipped" else []
+        if self.reuse_root_evals:
+            calls += [(self.engine.miss_planes, s) for s in self.root_sizes]
+        for buf, size in sorted(calls, key=lambda c: -c[1]):
+            self._forward(buf[:size])
         self.nn_evals = self.nn_rows = 0
 
     def _search_step_as_shipped(self) -> None:
