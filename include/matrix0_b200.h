@@ -250,7 +250,9 @@ int m0_net_forward(m0_net* net, const float* d_planes, int B, float* d_logits, f
 /* The dominant kernel on its own (tests, roofline micro-benchmark): tcgen05/TMA implicit GEMM over bf16 operands.
  * taps = 9: 3x3 "same" convolution of NHWC activations d_act_bf16[boards][8][8][cin] with d_w_bf16[n][9*cin]
  * (k = (ky*3+kx)*cin + ci, nn.Conv2d of resnet.py:32-34); taps = 1: d_act_bf16[boards*64][cin] x d_w_bf16[n][cin]^T.
- * d_out_f32[boards*64][n].  boards even, cin % 64 == 0, n % 16 == 0, n <= 320. */
+ * d_out_f32[boards*64][n].  boards even, cin % 32 == 0, n % 16 == 0, n <= 320.  With cin % 64 == 32 the last 64-deep k-block
+ * of each tap is half empty: the activations are zero-filled past cin, and 3x3 weights are copied with each tap padded to whole
+ * k-blocks (stream-ordered allocation, freed after the launch). */
 int m0_tc_conv(const uint16_t* d_act_bf16, const uint16_t* d_w_bf16, int boards, int cin, int n, int taps, float* d_out_f32, void* stream);
 /* Per-launch-site CUDA-event timing of the tensor-core forward (measurement aid, no reference counterpart): after
  * m0_profile_enable(1) every kernel launch of m0_net_forward (precision 1, 2) is bracketed by events on its stream;

@@ -287,22 +287,27 @@ __global__ void layernorm_residual_f32_kernel(const float* __restrict__ proj, co
 
 // Tensor-core path: x_new = LN(proj + x) (resnet.py:182-188) and, fused, a_out = half(act(GroupNorm_16ch(x_new))) = the bn1 +
 // activation of the next residual block (resnet.py:46-47).  One block (8 warps) per board; warp w owns tokens 8w..8w+7, lane l
-// owns channels 2l + 64j (j < C/64): proj and x are read once, the sums live in registers for both normalisations.
+// owns channels 2l + 64j (j < NJ = ceil(C / 64)): proj and x are read once, the sums live in registers for both normalisations.
+// C % 64 == 32: the last j holds channels for lanes 0..15 only (two GroupNorm groups); the other lanes' values there are zero and
+// take no part in the LayerNorm statistics or the stores.
 // HALF_IN: proj is the 16-bit output of the projection GEMM (the reference's proj convolution runs under autocast, resnet.py:676-677);
 // gn_g == nullptr with a_out != nullptr: a_out = half(x_new) without the GroupNorm (the operand of the head GEMMs after the last block)
-template <int NJ, bool HALF_IN>
+template <int C, bool HALF_IN>
 __global__ void __launch_bounds__(256, 2)
 ln_res_gn_kernel(const float* __restrict__ proj, float* __restrict__ x, const float* __restrict__ ln_g, const float* __restrict__ ln_b,
                  const float* __restrict__ gn_g, const float* __restrict__ gn_b, __nv_bfloat16* __restrict__ a_out, int act, int fp16) {
-  constexpr int C = 64 * NJ;
+  constexpr int NJ = (C + 63) / 64;
   __shared__ float s_part[8][NJ][4][2];
   const int b = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const size_t base = ((size_t)b * 64 + warp * 8) * C + 2 * lane;
+  // channels 2 lane + 64 j exist (always, unless C % 64 == 32 and j is the last k-block)
+  auto has = [lane](int j) { return C % 64 == 0 || j < NJ - 1 || lane < 16; };
   float v[8][2 * NJ];
 #pragma unroll
   for (int t = 0; t < 8; ++t)
 #pragma unroll
     for (int j = 0; j < NJ; ++j) {
+      if (!has(j)) { v[t][2 * j] = v[t][2 * j + 1] = 0.f; continue; }
       float2 p2;
       if (HALF_IN) {
         const uint32_t h = __ldg(reinterpret_cast<const uint32_t*>(reinterpret_cast<const uint16_t*>(proj) + base + (size_t)t * C + 64 * j));
@@ -318,6 +323,7 @@ ln_res_gn_kernel(const float* __restrict__ proj, float* __restrict__ x, const fl
   float lg[2 * NJ], lb[2 * NJ];
 #pragma unroll
   for (int j = 0; j < NJ; ++j) {
+    if (!has(j)) { lg[2 * j] = lg[2 * j + 1] = lb[2 * j] = lb[2 * j + 1] = 0.f; continue; }
     const float2 g2 = *reinterpret_cast<const float2*>(ln_g + 2 * lane + 64 * j), b2 = *reinterpret_cast<const float2*>(ln_b + 2 * lane + 64 * j);
     lg[2 * j] = g2.x; lg[2 * j + 1] = g2.y; lb[2 * j] = b2.x; lb[2 * j + 1] = b2.y;
   }
@@ -340,6 +346,7 @@ ln_res_gn_kernel(const float* __restrict__ proj, float* __restrict__ x, const fl
     float d2 = 0.f;
 #pragma unroll
     for (int k = 0; k < 2 * NJ; ++k) {
+      if (!has(k >> 1)) continue;
       const float d = v[t][k] - mean[t];
       d2 = fmaf(d, d, d2);
     }
@@ -355,7 +362,8 @@ ln_res_gn_kernel(const float* __restrict__ proj, float* __restrict__ x, const fl
 #pragma unroll
     for (int k = 0; k < 2 * NJ; ++k) v[t][k] = (v[t][k] - mean[t]) * rstd[t] * lg[k] + lb[k];
 #pragma unroll
-    for (int j = 0; j < NJ; ++j) *reinterpret_cast<float2*>(x + base + (size_t)t * C + 64 * j) = make_float2(v[t][2 * j], v[t][2 * j + 1]);
+    for (int j = 0; j < NJ; ++j)
+      if (has(j)) *reinterpret_cast<float2*>(x + base + (size_t)t * C + 64 * j) = make_float2(v[t][2 * j], v[t][2 * j + 1]);
   }
   if (!a_out) return;
   if (!gn_g) {   // plain 16-bit copy of the new residual stream
@@ -363,6 +371,7 @@ ln_res_gn_kernel(const float* __restrict__ proj, float* __restrict__ x, const fl
     for (int t = 0; t < 8; ++t)
 #pragma unroll
       for (int j = 0; j < NJ; ++j) {
+        if (!has(j)) continue;
         uint32_t pk;
         if (fp16) { __half2 h = __floats2half2_rn(v[t][2 * j], v[t][2 * j + 1]); pk = *reinterpret_cast<uint32_t*>(&h); }
         else { __nv_bfloat162 h = __floats2bfloat162_rn(v[t][2 * j], v[t][2 * j + 1]); pk = *reinterpret_cast<uint32_t*>(&h); }
@@ -409,6 +418,7 @@ ln_res_gn_kernel(const float* __restrict__ proj, float* __restrict__ x, const fl
   if (gn_g) {
 #pragma unroll
     for (int j = 0; j < NJ; ++j) {
+      if (!has(j)) continue;
       const float2 g2 = *reinterpret_cast<const float2*>(gn_g + 2 * lane + 64 * j), b2 = *reinterpret_cast<const float2*>(gn_b + 2 * lane + 64 * j);
       const float g0 = g2.x * gr[j], g1 = g2.y * gr[j];
       const float b0 = b2.x - gm[j] * g0, b1 = b2.y - gm[j] * g1;
@@ -486,16 +496,20 @@ int nn_ln_res_gn(const void* proj, int proj_half, float* x, const float* ln_g, c
                  __nv_bfloat16* a_out, int B, int C, int act, cudaStream_t s) {
   const int fp16 = g_half_fp16;
   const float* p = reinterpret_cast<const float*>(proj);
-#define M0_LN_CASE(NJ)                                                                                                    \
-  if (proj_half) ln_res_gn_kernel<NJ, true><<<B, 256, 0, s>>>(p, x, ln_g, ln_b, gn_g, gn_b, a_out, act, fp16);            \
-  else ln_res_gn_kernel<NJ, false><<<B, 256, 0, s>>>(p, x, ln_g, ln_b, gn_g, gn_b, a_out, act, fp16);                     \
+#define M0_LN_CASE(C)                                                                                                     \
+  if (proj_half) ln_res_gn_kernel<C, true><<<B, 256, 0, s>>>(p, x, ln_g, ln_b, gn_g, gn_b, a_out, act, fp16);             \
+  else ln_res_gn_kernel<C, false><<<B, 256, 0, s>>>(p, x, ln_g, ln_b, gn_g, gn_b, a_out, act, fp16);                      \
   break;
   switch (C) {
-    case 64: M0_LN_CASE(1)
-    case 128: M0_LN_CASE(2)
-    case 192: M0_LN_CASE(3)
-    case 256: M0_LN_CASE(4)
-    case 320: M0_LN_CASE(5)
+    case 64: M0_LN_CASE(64)
+    case 96: M0_LN_CASE(96)
+    case 128: M0_LN_CASE(128)
+    case 160: M0_LN_CASE(160)
+    case 192: M0_LN_CASE(192)
+    case 224: M0_LN_CASE(224)
+    case 256: M0_LN_CASE(256)
+    case 288: M0_LN_CASE(288)
+    case 320: M0_LN_CASE(320)
     default: m0_set_error("ln_res_gn: unsupported channel count %d", C); return M0_ERR_ARG;
   }
 #undef M0_LN_CASE

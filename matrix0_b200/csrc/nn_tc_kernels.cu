@@ -42,13 +42,6 @@ __global__ void transpose_f32_kernel(const float* __restrict__ in, float* __rest
   int r = i / cols, c = i % cols;
   out[c * rows + r] = in[i];
 }
-// stem weights [C][9][P] -> [C][9][64] (zero padded input channels)
-__global__ void pad_stem_kernel(const float* __restrict__ w, float* __restrict__ out, int C, int P) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= C * 9 * 64) return;
-  int ci = i & 63, tap = (i >> 6) % 9, co = i / (9 * 64);
-  out[i] = ci < P ? w[(co * 9 + tap) * P + ci] : 0.0f;
-}
 // SE squeeze folded through conv2 (tc_conv_pair.cuh, ConvPairParams::prims).  With P = the 12 x C half-board sums of conv2's INPUT
 // (k = (half*6 + j)*C + ci), the board mean of conv2's output channel c is (1/64) sum_k Wcomb[c][k] P[k], where zero padding turns
 // each tap (dy, dx) into "all squares minus an edge rank minus an edge file plus their corner":
@@ -84,12 +77,13 @@ __global__ void se_fold_kernel(const float* __restrict__ conv_w, const float* __
   }
   out[i] = acc * (1.0f / 64.0f);
 }
-// in [rows][cols] -> out [rows][cols_pad] with zero padding columns
-__global__ void pad_cols_kernel(const float* __restrict__ in, float* __restrict__ out, int rows, int cols, int cols_pad) {
+// in [rows][cols] -> out [rows][cols_pad] with zero padding columns (T = float, or uint16_t for 16-bit values: zero bits are +0)
+template <typename T>
+__global__ void pad_cols_kernel(const T* __restrict__ in, T* __restrict__ out, int rows, int cols, int cols_pad) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= rows * cols_pad) return;
   const int r = i / cols_pad, c = i - r * cols_pad;
-  out[i] = c < cols ? in[r * cols + c] : 0.0f;
+  out[i] = c < cols ? in[r * cols + c] : T(0);
 }
 }  // namespace m0
 
@@ -204,7 +198,7 @@ struct TcState {
   // heads on tensor cores
   bool heads_tc = false;
   TcWeight pol_conv, pol_fc1, pol_fc2, val_conv1, val_conv2, val_fc1, val_fc2, val_gate;
-  bool val_tail_tc = false;      // value_fc2 and value_gate on tensor cores as well (C % 64 == 0)
+  bool val_tail_tc = false;      // value_fc2 and value_gate on tensor cores as well (M0_TC_VALUE_TAIL=0: fp32 SIMT GEMMs)
   int pol_rank_pad = 0;
   __nv_bfloat16 *ph_h = nullptr, *pf_h = nullptr, *vh_h = nullptr;   // [cap][4096], [cap][rank_pad], [cap][64][128]
   __nv_bfloat16 *vf1_h = nullptr, *vf2_h = nullptr;                  // [cap][2C], [cap][C]: operands of value_fc2 / value_gate
@@ -294,6 +288,11 @@ struct TcProfiler {
 
 int n_part_for(int n) { return n <= 256 ? n : n / 2; }
 
+// 64-deep k-blocks per tap of cin input channels.  A tail block (cin % 64 == 32) reads channels past cin, which the activation maps
+// zero-fill (their channel extent is cin); 3x3 weights are stored with each tap padded to whole k-blocks (make_weight), 1x1 weights
+// [n][cin] are zero-filled by their map as well.
+int kblocks_for(int cin) { return (cin + 63) / 64; }
+
 int env_int(const char* name, int dflt) {
   const char* e = getenv(name);
   return e ? atoi(e) : dflt;
@@ -330,7 +329,7 @@ int launch_conv_pair(TcState* st, const CUtensorMap& a_map, const TcWeight& w, i
   memset(&p, 0, sizeof(p));
   p.boards = boards;
   p.N = w.n_launch;
-  p.kb_per_tap = cin / 64;
+  p.kb_per_tap = kblocks_for(cin);
   p.conv = conv;
   p.n_slices = n_slices;
   if (n_slices > 1 && (gn_gamma || pool_part || fuse)) { m0_set_error("pair kernel: fused epilogues need a single slice"); return M0_ERR_ARG; }
@@ -346,7 +345,7 @@ int launch_conv_pair(TcState* st, const CUtensorMap& a_map, const TcWeight& w, i
   static int cap = -1;
   if (cap < 0) cap = env_int("M0_TC_STAGES", 0);   // pipeline-depth experiments
   const int stage_bytes = conv ? tc::CP_A_SLOT + 3 * (w.n_launch / 4) * 128 : (w.n_launch / 4) * 128;
-  const int a_res = conv ? 0 : 2 * (cin / 64) * tc::A_TILE_BYTES;   // plain mode keeps two resident A tiles (K <= 320)
+  const int a_res = conv ? 0 : 2 * kblocks_for(cin) * tc::A_TILE_BYTES;   // plain mode keeps two resident A tiles (K <= 320)
   const int fz = !fuse ? 0 : fuse->resid_x ? 2 : fuse->prims ? 1 : 0;   // tc_conv_pair.cuh FUSE variants
   const int epi_bytes = fz == 2 ? tc::CP_EPI_BYTES_FUSE : tc::CP_EPI_BYTES;
   int stages = (st->max_smem - 2048 - epi_bytes - a_res) / stage_bytes;
@@ -388,8 +387,12 @@ int launch_conv_pair(TcState* st, const CUtensorMap& a_map, const TcWeight& w, i
   return m0_check_launch("conv_pair_kernel");
 }
 
-// n_launch: output channels per kernel launch (N <= 320 -> <= 512 TMEM columns); wider layers are split by rows
-int make_weight(TcState* st, TcWeight* out, const float* w_f32, int n, int k, int n_launch, cudaStream_t s) {
+// n_launch: output channels per kernel launch (N <= 320 -> <= 512 TMEM columns); wider layers are split by rows.
+// taps = 9: w_f32 is [n][9][k / 9]; each tap is stored in whole 64-channel k-blocks, zero columns after its k / 9 channels, so that the
+// tail k-block of a tap never reads the next tap's weights.
+int make_weight(TcState* st, TcWeight* out, const float* w_f32, int n, int k, int n_launch, cudaStream_t s, int taps = 1) {
+  const int cin = k / taps, cin_pad = taps > 1 ? kblocks_for(cin) * 64 : cin;
+  k = taps * cin_pad;
   out->n = n;
   out->k = k;
   out->n_part = n_part_for(n_launch);
@@ -398,7 +401,17 @@ int make_weight(TcState* st, TcWeight* out, const float* w_f32, int n, int k, in
   M0_CUDA_TRY(cudaMalloc(&p, (size_t)n * k * 2));
   st->allocs.push_back(p);
   out->w = (__nv_bfloat16*)p;
-  TRY(nn_f32_to_bf16(w_f32, out->w, (size_t)n * k, s));
+  if (cin_pad != cin) {
+    float* padded = nullptr;
+    M0_CUDA_TRY(cudaMallocAsync((void**)&padded, (size_t)n * k * 4, s));
+    pad_cols_kernel<float><<<(n * k + 255) / 256, 256, 0, s>>>(w_f32, padded, n * taps, cin, cin_pad);
+    int rc = m0_check_launch("pad_taps");
+    if (rc == M0_OK) rc = nn_f32_to_bf16(padded, out->w, (size_t)n * k, s);
+    cudaFreeAsync(padded, s);
+    TRY(rc);
+  } else {
+    TRY(nn_f32_to_bf16(w_f32, out->w, (size_t)n * k, s));
+  }
   out->n_launch = n_launch;
   out->pair = pair_ok(n_launch) && n % n_launch == 0;
   if (out->pair) TRY(make_map_2d(&out->map_pair, out->w, (uint64_t)n, (uint64_t)k, (uint32_t)(n_launch / 4)));
@@ -423,7 +436,7 @@ int launch_gemm(TcState* st, const CUtensorMap& a_map, const TcWeight& w, int M,
   p.n_slices = n_slices;
   p.k_splits = k_splits;
   p.split_stride = split_stride;
-  if (k_splits > 1 && (out_bf16 || bias || act != ACT_NONE || gn_gamma || pool_part || (taps * (cin / 64)) % k_splits != 0 || !out_f32)) {
+  if (k_splits > 1 && (out_bf16 || bias || act != ACT_NONE || gn_gamma || pool_part || (taps * kblocks_for(cin)) % k_splits != 0 || !out_f32)) {
     m0_set_error("tensor-core GEMM: split-K needs a plain fp32 output and a K range divisible into whole k-blocks");
     return M0_ERR_ARG;
   }
@@ -431,7 +444,7 @@ int launch_gemm(TcState* st, const CUtensorMap& a_map, const TcWeight& w, int M,
   if (w.n_part > N || N % w.n_part != 0) { m0_set_error("tensor-core GEMM: launch width %d does not match the weight map box %d", N, w.n_part); return M0_ERR_ARG; }
   p.n_part = w.n_part;
   p.taps = taps;
-  p.kb_per_tap = cin / 64;
+  p.kb_per_tap = kblocks_for(cin);
   p.conv = conv;
   p.w_row0 = w_row0;
   // two accumulators when they fit into the 512 columns of tensor memory (M0_TC_ACC2=0: single accumulator, for A-B comparison)
@@ -612,8 +625,10 @@ int tc_net_prepare(::m0_net* n, cudaStream_t s) {
   const int fmt = nn_half_format();
   if (all->st[fmt]) return M0_OK;
   const m0_net_config& c = n->cfg;
-  if (c.channels % 64 != 0) { m0_set_error("bf16 tensor-core path needs channels %% 64 == 0 (got %d)", c.channels); return M0_ERR_ARG; }
-  if (c.channels > 320) { m0_set_error("bf16 tensor-core path supports up to 320 channels (got %d)", c.channels); return M0_ERR_ARG; }
+  if (c.channels % 32 != 0 || c.channels < 64 || c.channels > 320) {
+    m0_set_error("16-bit tensor-core path needs channels %% 32 == 0 and 64 <= channels <= 320 (got %d)", c.channels);
+    return M0_ERR_ARG;
+  }
   TcState* st = new (std::nothrow) TcState();
   if (!st) { m0_set_error("out of host memory"); return M0_ERR_ARG; }
   cudaDeviceGetAttribute(&st->sm_count, cudaDevAttrMultiProcessorCount, n->device);
@@ -621,14 +636,8 @@ int tc_net_prepare(::m0_net* n, cudaStream_t s) {
   const int C = c.channels;
   int rc = M0_OK;
   do {
-    {  // stem on tensor cores: input channels zero-padded to 64
-      float* padded = nullptr;
-      if ((rc = m0_check_cuda(cudaMalloc((void**)&padded, (size_t)C * 9 * 64 * 4), "cudaMalloc stem")) != M0_OK) break;
-      st->allocs.push_back(padded);
-      pad_stem_kernel<<<(C * 9 * 64 + 255) / 256, 256, 0, s>>>(n->w.stem_w, padded, C, c.planes);
-      if ((rc = m0_check_launch("pad_stem")) != M0_OK) break;
-      if ((rc = make_weight(st, &st->stem, padded, C, 9 * 64, C, s)) != M0_OK) break;
-    }
+    // stem on tensor cores: input channels zero-padded to 64
+    if ((rc = make_weight(st, &st->stem, n->w.stem_w, C, 9 * c.planes, C, s, 9)) != M0_OK) break;
     if (c.se) {
       st->se_w1t.resize(c.blocks, nullptr);
       st->se_w2t.resize(c.blocks, nullptr);
@@ -663,8 +672,11 @@ int tc_net_prepare(::m0_net* n, cudaStream_t s) {
       if ((rc = make_weight(st, &st->pol_fc2, w2p, ps_pad, rp, 320, s)) != M0_OK) break;
       if ((rc = make_weight(st, &st->val_conv1, n->w.val_conv1_w, 128, C, 128, s)) != M0_OK) break;
       if ((rc = make_weight(st, &st->val_conv2, n->w.val_conv2_w, 128, 128, 128, s)) != M0_OK) break;
-      if ((rc = make_weight(st, &st->val_fc1, n->w.val_fc1_w, 2 * C, 8192, C, s)) != M0_OK) break;
-      if (C % 64 == 0 && env_int("M0_TC_VALUE_TAIL", 1)) {
+      // C > 256 runs as two MMAs of C / 2 columns side by side in tensor memory; 288 is cut into 144-column launches instead, which
+      // keeps every accumulator at a 32-column boundary
+      const int fc1_launch = n_part_for(C) % 32 == 0 ? C : slice_width_for(C, C);
+      if ((rc = make_weight(st, &st->val_fc1, n->w.val_fc1_w, 2 * C, 8192, fc1_launch, s)) != M0_OK) break;
+      if (env_int("M0_TC_VALUE_TAIL", 1)) {
         if ((rc = make_weight(st, &st->val_fc2, n->w.val_fc2_w, C, 2 * C, slice_width_for(C, C), s)) != M0_OK) break;
         if ((rc = make_weight(st, &st->val_gate, n->w.val_gate_w, C, C, slice_width_for(C, C), s)) != M0_OK) break;
         st->val_tail_tc = true;
@@ -673,27 +685,30 @@ int tc_net_prepare(::m0_net* n, cudaStream_t s) {
     }
     if (c.chess_features) {
       if (c.piece_square_tables && (rc = make_weight(st, &st->pst, n->w.pst_w, C, C, env_int("M0_TC_SLICE_PROJ", 1) ? slice_width_for(C, C) : C, s)) != M0_OK) break;
-      if ((rc = make_weight(st, &st->inter, n->w.inter_w, C, 9 * C, C, s)) != M0_OK) break;
+      if ((rc = make_weight(st, &st->inter, n->w.inter_w, C, 9 * C, C, s, 9)) != M0_OK) break;
     }
     // fused SE + residual epilogue of conv2 (M0_TC_FUSE_SE=0 keeps the separate SE / residual kernels)
     st->hid_pad = (c.se_hidden + 63) / 64 * 64;
-    st->se_fused = env_int("M0_TC_FUSE_SE", 1) != 0 && pair_ok(C) && (!c.se || (c.se_hidden % 16 == 0 && c.se_hidden <= 256));
+    st->se_fused = env_int("M0_TC_FUSE_SE", 1) != 0 && pair_ok(C) && (!c.se || c.se_hidden <= 256);
     st->blocks.resize(c.blocks);
     for (int i = 0; i < c.blocks && rc == M0_OK; ++i) {
       const m0_block_weights& b = n->w.blocks[i];
-      if ((rc = make_weight(st, &st->blocks[i].conv1, b.conv1_w, C, 9 * C, C, s)) != M0_OK) break;
-      if ((rc = make_weight(st, &st->blocks[i].conv2, b.conv2_w, C, 9 * C, C, s)) != M0_OK) break;
+      if ((rc = make_weight(st, &st->blocks[i].conv1, b.conv1_w, C, 9 * C, C, s, 9)) != M0_OK) break;
+      if ((rc = make_weight(st, &st->blocks[i].conv2, b.conv2_w, C, 9 * C, C, s, 9)) != M0_OK) break;
       if (st->se_fused && c.se) {
-        const int hid = c.se_hidden, K = 12 * C, hp = st->hid_pad;
+        // the first SE GEMM runs hid16 = hid rounded up to 16 output columns (the MMA width granule); the extra rows of the folded
+        // weight are zero and their columns are not stored
+        const int hid = c.se_hidden, hid16 = (hid + 15) / 16 * 16, K = 12 * C, hp = st->hid_pad;
         float *fold = nullptr, *w2p = nullptr;
-        if ((rc = m0_check_cuda(cudaMalloc((void**)&fold, (size_t)hid * K * 4), "cudaMalloc se_fold")) != M0_OK) break;
+        if ((rc = m0_check_cuda(cudaMalloc((void**)&fold, (size_t)hid16 * K * 4), "cudaMalloc se_fold")) != M0_OK) break;
         st->allocs.push_back(fold);
+        if ((rc = m0_check_cuda(cudaMemsetAsync(fold, 0, (size_t)hid16 * K * 4, s), "memset se_fold")) != M0_OK) break;
         if ((rc = m0_check_cuda(cudaMalloc((void**)&w2p, (size_t)C * hp * 4), "cudaMalloc se_w2")) != M0_OK) break;
         st->allocs.push_back(w2p);
         se_fold_kernel<<<(hid * K + 255) / 256, 256, 0, s>>>(b.conv2_w, b.se_w1, fold, C, hid);
-        pad_cols_kernel<<<(C * hp + 255) / 256, 256, 0, s>>>(b.se_w2, w2p, C, hid, hp);
+        pad_cols_kernel<float><<<(C * hp + 255) / 256, 256, 0, s>>>(b.se_w2, w2p, C, hid, hp);
         if ((rc = m0_check_launch("se_fold")) != M0_OK) break;
-        if ((rc = make_weight(st, &st->blocks[i].se_fold, fold, hid, K, hid, s)) != M0_OK) break;
+        if ((rc = make_weight(st, &st->blocks[i].se_fold, fold, hid16, K, hid16, s)) != M0_OK) break;
         if ((rc = make_weight(st, &st->blocks[i].se_w2, w2p, C, hp, C, s)) != M0_OK) break;
       }
       if (b.has_attention) {
@@ -806,10 +821,11 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
         if (se_nosplit < 0) se_nosplit = env_int("M0_SE_NOSPLIT", 0);
         if (se_nosplit) {
           // one launch: bias + activation in the GEMM epilogue, hidden layer written in the operand format (no split-K, no reduction kernel)
-          PROF("se_fc1", launch_gemm(st, st->prims_mat, tb.se_fold, B, 0, 1, 12 * C, 0, c.se_hidden, nullptr, st->se_hid_h, st->hid_pad, 0, b.se_b1, act, 1.0f, s));
+          PROF("se_fc1", launch_gemm(st, st->prims_mat, tb.se_fold, B, 0, 1, 12 * C, 0, tb.se_fold.n, nullptr, st->se_hid_h, st->hid_pad, 0, b.se_b1, act, 1.0f, s,
+                                     nullptr, nullptr, nullptr, c.se_hidden));
         } else {
-          PROF("se_fc1", launch_gemm(st, st->prims_mat, tb.se_fold, B, 0, 1, 12 * C, 0, c.se_hidden, st->se_part, nullptr, st->hid_pad, 0, none, ACT_NONE, 1.0f, s,
-                                     nullptr, nullptr, nullptr, -1, 1, st->se_splits, (long long)st->se_rows * st->hid_pad));
+          PROF("se_fc1", launch_gemm(st, st->prims_mat, tb.se_fold, B, 0, 1, 12 * C, 0, tb.se_fold.n, st->se_part, nullptr, st->hid_pad, 0, none, ACT_NONE, 1.0f, s,
+                                     nullptr, nullptr, nullptr, c.se_hidden, 1, st->se_splits, (long long)st->se_rows * st->hid_pad));
           static int se_tail = -1;
           if (se_tail < 0) se_tail = env_int("M0_SE_TAIL", 1);
           if (se_tail) {
@@ -860,7 +876,7 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
       // the projection leaves the GEMM in the 16-bit operand format, as under the reference's autocast (M0_TC_PROJ_F32=1: fp32 hand-off)
       static int proj_f32 = -1;
       if (proj_f32 < 0) proj_f32 = env_int("M0_TC_PROJ_F32", 0);
-      const bool fused_ln = C % 64 == 0 && C <= 320;
+      const bool fused_ln = C % 32 == 0 && C <= 320;
       const bool proj_half = fused_ln && !proj_f32;
       if (proj_half) PROF("gemm_proj", gemm_rows64(st, st->a2_mat, tb.proj, B, C, nullptr, reinterpret_cast<__nv_bfloat16*>(n->t2), C, s, &st->t2h_out));
       else PROF("gemm_proj", gemm_rows64(st, st->a2_mat, tb.proj, B, C, n->t2, nullptr, C, s, &st->t2f_out));
@@ -894,16 +910,16 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
   if (st->val_tail_tc) {
     // fc1 (+ activation) -> 16-bit, fc2 (+ activation) and the gate's linear layer + sigmoid on tensor cores (resnet.py:747-752);
     // value = tanh(fc3(fc2_out * gate)) in one small reduction kernel
-    PROF("gemm_val_fc1", launch_gemm(st, st->vh_fc_mat, st->val_fc1, B, 0, 1, 8192, 0, C, nullptr, st->vf1_h, 2 * C, 0, w.val_fc1_b, vact, 1.0f, s, nullptr,
-                                     nullptr, nullptr, -1, 2));
+    PROF("gemm_val_fc1", launch_gemm(st, st->vh_fc_mat, st->val_fc1, B, 0, 1, 8192, 0, st->val_fc1.n_launch, nullptr, st->vf1_h, 2 * C, 0, w.val_fc1_b, vact,
+                                     1.0f, s, nullptr, nullptr, nullptr, -1, 2 * C / st->val_fc1.n_launch));
     PROF("gemm_val_fc2", launch_gemm(st, st->vf1_mat, st->val_fc2, B, 0, 1, 2 * C, 0, st->val_fc2.n_launch, n->vf2, st->vf2_h, C, 0, w.val_fc2_b, vact, 1.0f, s,
                                      nullptr, nullptr, nullptr, -1, C / st->val_fc2.n_launch));
     PROF("gemm_val_gate", launch_gemm(st, st->vf2_mat, st->val_gate, B, 0, 1, C, 0, st->val_gate.n_launch, n->vg, nullptr, C, 0, w.val_gate_b, ACT_SIGMOID, 1.0f,
                                       s, nullptr, nullptr, nullptr, -1, C / st->val_gate.n_launch));
     PROF("value_tail", nn_value_tail(n->vg, n->vf2, w.val_fc3_w, w.val_fc3_b, values, B, C, s));
   } else {
-    PROF("gemm_val_fc1", launch_gemm(st, st->vh_fc_mat, st->val_fc1, B, 0, 1, 8192, 0, C, n->vf1, nullptr, 2 * C, 0, w.val_fc1_b, vact, 1.0f, s, nullptr, nullptr,
-                                     nullptr, -1, 2));
+    PROF("gemm_val_fc1", launch_gemm(st, st->vh_fc_mat, st->val_fc1, B, 0, 1, 8192, 0, st->val_fc1.n_launch, n->vf1, nullptr, 2 * C, 0, w.val_fc1_b, vact, 1.0f,
+                                     s, nullptr, nullptr, nullptr, -1, 2 * C / st->val_fc1.n_launch));
     PROF("gemm_f32", nn_gemm_f32(A_DIRECT, n->vf1, w.val_fc2_w, w.val_fc2_b, nullptr, n->vf2, B, C, 2 * C, 2 * C, C, 0, vact, 1.0f, s));
     PROF("gemm_f32", nn_gemm_f32(A_DIRECT, n->vf2, w.val_gate_w, w.val_gate_b, n->vf2, n->vg, B, C, C, C, C, 0, ACT_SIGMOID, 1.0f, s));
     PROF("gemm_f32", nn_gemm_f32(A_DIRECT, n->vg, w.val_fc3_w, w.val_fc3_b, nullptr, values, B, 1, C, C, 1, 0, ACT_TANH, 1.0f, s));
@@ -918,8 +934,9 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
 //   taps = 9: out[b*64+sq][n] = conv3x3(act NHWC bf16 [boards][8][8][cin], w [n][9*cin]) ; taps = 1: plain GEMM act[boards*64][cin] x w[n][cin]^T
 extern "C" int m0_tc_conv(const uint16_t* d_act_bf16, const uint16_t* d_w_bf16, int boards, int cin, int n, int taps, float* d_out_f32,
                           void* stream) {
-  if (!d_act_bf16 || !d_w_bf16 || !d_out_f32 || boards <= 0 || (boards & 1) || cin % 64 != 0 || n % 16 != 0 || n > 320 || (taps != 1 && taps != 9)) {
-    m0_set_error("m0_tc_conv: invalid argument (boards even, cin %% 64 == 0, n %% 16 == 0, n <= 320, taps in {1, 9})");
+  if (!d_act_bf16 || !d_w_bf16 || !d_out_f32 || boards <= 0 || (boards & 1) || cin <= 0 || cin % 32 != 0 || n % 16 != 0 || n > 320 ||
+      (taps != 1 && taps != 9)) {
+    m0_set_error("m0_tc_conv: invalid argument (boards even, cin %% 32 == 0, n %% 16 == 0, n <= 320, taps in {1, 9})");
     return M0_ERR_ARG;
   }
   // the operands of this entry point are bf16 by contract, whatever 16-bit format the last forward of the process selected
@@ -939,32 +956,48 @@ extern "C" int m0_tc_conv(const uint16_t* d_act_bf16, const uint16_t* d_w_bf16, 
   }
   cudaDeviceGetAttribute(&st.sm_count, cudaDevAttrMultiProcessorCount, dev);
   cudaDeviceGetAttribute(&st.max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-  TcWeight w;
-  w.w = (__nv_bfloat16*)d_w_bf16;
-  w.n = n;
-  w.k = taps * cin;
-  w.n_part = n_part_for(n);
-  w.cluster = pick_cluster(w.n_part);
-  TRY(make_map_2d(&w.map, d_w_bf16, (uint64_t)n, (uint64_t)taps * cin, (uint32_t)(w.n_part / w.cluster)));
-  CUtensorMap a;
-  w.n_launch = n;
-  if (taps == 9 && pair_ok(n)) {
-    w.pair = true;
-    TRY(make_map_2d(&w.map_pair, d_w_bf16, (uint64_t)n, (uint64_t)taps * cin, (uint32_t)(n / 4)));
-    TRY(make_map_nhwc(&a, d_act_bf16, (uint64_t)boards, (uint64_t)cin, 10));
-    CUtensorMap om;
-    TRY(make_map_out(&om, d_out_f32, (uint64_t)boards * 64, (uint64_t)n, true));
-    return launch_conv_pair(&st, a, w, boards, cin, d_out_f32, nullptr, n, ACT_NONE, (cudaStream_t)stream, nullptr, nullptr, nullptr, nullptr, 1, 1, &om);
+  const cudaStream_t s = (cudaStream_t)stream;
+  // 3x3 weights with cin % 64 == 32 are copied with every tap padded to whole k-blocks (the layout make_weight gives the network's
+  // weights); the copy is stream-ordered and freed after the launch
+  const int kw = taps * kblocks_for(cin) * 64;
+  void* w_pad = nullptr;
+  if (taps == 9 && kw != taps * cin) {
+    M0_CUDA_TRY(cudaMallocAsync(&w_pad, (size_t)n * kw * 2, s));
+    pad_cols_kernel<uint16_t><<<(n * kw + 255) / 256, 256, 0, s>>>(d_w_bf16, (uint16_t*)w_pad, n * taps, cin, kw / taps);
+    const int rc = m0_check_launch("pad_taps");
+    if (rc != M0_OK) { cudaFreeAsync(w_pad, s); return rc; }
   }
-  if (taps == 1 && pair_ok(n) && cin <= 320) {   // plain GEMM over whole boards on the CTA-pair kernel (qkv / proj / piece-square projections)
-    w.pair = true;
-    TRY(make_map_2d(&w.map_pair, d_w_bf16, (uint64_t)n, (uint64_t)cin, (uint32_t)(n / 4)));
-    TRY(make_map_2d(&a, d_act_bf16, (uint64_t)boards * 64, (uint64_t)cin, 128));
-    return launch_conv_pair(&st, a, w, boards, cin, d_out_f32, nullptr, n, ACT_NONE, (cudaStream_t)stream, nullptr, nullptr, nullptr, nullptr, 0, 1);
-  }
-  if (taps == 9) TRY(make_map_nhwc(&a, d_act_bf16, (uint64_t)boards, (uint64_t)cin));
-  else TRY(make_map_2d(&a, d_act_bf16, (uint64_t)boards * 64, (uint64_t)cin, 128));
-  return launch_gemm(&st, a, w, boards * 64, taps == 9 ? 1 : 0, taps, cin, 0, n, d_out_f32, nullptr, n, 0, nullptr, ACT_NONE, 1.0f, (cudaStream_t)stream);
+  auto run = [&](const void* wp, int k) -> int {
+    TcWeight w;
+    w.w = (__nv_bfloat16*)wp;
+    w.n = n;
+    w.k = k;
+    w.n_part = n_part_for(n);
+    w.cluster = pick_cluster(w.n_part);
+    TRY(make_map_2d(&w.map, wp, (uint64_t)n, (uint64_t)k, (uint32_t)(w.n_part / w.cluster)));
+    CUtensorMap a;
+    w.n_launch = n;
+    if (taps == 9 && pair_ok(n)) {
+      w.pair = true;
+      TRY(make_map_2d(&w.map_pair, wp, (uint64_t)n, (uint64_t)k, (uint32_t)(n / 4)));
+      TRY(make_map_nhwc(&a, d_act_bf16, (uint64_t)boards, (uint64_t)cin, 10));
+      CUtensorMap om;
+      TRY(make_map_out(&om, d_out_f32, (uint64_t)boards * 64, (uint64_t)n, true));
+      return launch_conv_pair(&st, a, w, boards, cin, d_out_f32, nullptr, n, ACT_NONE, s, nullptr, nullptr, nullptr, nullptr, 1, 1, &om);
+    }
+    if (taps == 1 && pair_ok(n) && cin <= 320) {   // plain GEMM over whole boards on the CTA-pair kernel (qkv / proj / piece-square projections)
+      w.pair = true;
+      TRY(make_map_2d(&w.map_pair, wp, (uint64_t)n, (uint64_t)cin, (uint32_t)(n / 4)));
+      TRY(make_map_2d(&a, d_act_bf16, (uint64_t)boards * 64, (uint64_t)cin, 128));
+      return launch_conv_pair(&st, a, w, boards, cin, d_out_f32, nullptr, n, ACT_NONE, s, nullptr, nullptr, nullptr, nullptr, 0, 1);
+    }
+    if (taps == 9) TRY(make_map_nhwc(&a, d_act_bf16, (uint64_t)boards, (uint64_t)cin));
+    else TRY(make_map_2d(&a, d_act_bf16, (uint64_t)boards * 64, (uint64_t)cin, 128));
+    return launch_gemm(&st, a, w, boards * 64, taps == 9 ? 1 : 0, taps, cin, 0, n, d_out_f32, nullptr, n, 0, nullptr, ACT_NONE, 1.0f, s);
+  };
+  const int rc = w_pad ? run(w_pad, kw) : run(d_w_bf16, taps * cin);
+  if (w_pad) cudaFreeAsync(w_pad, s);
+  return rc;
 }
 
 // ---- per-launch-site timing of the tensor-core forward (bench.py roofline; diagnostics) -------------------------------------------
