@@ -307,9 +307,23 @@ se_gate_kernel(const float* __restrict__ pool, const float* __restrict__ w1t, co
 
 int nn_se_gate(const float* pool, const float* w1t, const float* b1, const float* w2t, const float* b2, float* gate, int B, int C, int hid, int act,
                cudaStream_t s) {
-  if (hid <= 0 || hid > 320) { m0_set_error("se_gate: unsupported hidden width %d", hid); return M0_ERR_ARG; }
+  if (hid <= 0 || hid > 320 || C > 320) { m0_set_error("se_gate: unsupported shape C = %d, hidden width %d", C, hid); return M0_ERR_ARG; }
   const int parts = 320 / hid;
-  se_gate_kernel<<<(B + 15) / 16, 320, (size_t)16 * (C + hid + (size_t)parts * hid) * sizeof(float), s>>>(pool, w1t, b1, w2t, b2, gate, B, C, hid, act);
+  const size_t smem = (size_t)16 * (C + hid + (size_t)parts * hid) * sizeof(float);
+  if (smem > 48 * 1024) {
+    // past the 48 KB default (C = 320 with hid > 256 needs up to 60 KB): grant the largest need of any supported shape, once per device,
+    // so that no net lowers the limit under another
+    static unsigned long long granted = 0;   // bit d: device d's kernel has the grant
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev >= 64 || !((granted >> dev) & 1ull)) {
+      const int most = 16 * (320 + 320 + 320) * (int)sizeof(float);
+      cudaError_t e = cudaFuncSetAttribute(se_gate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, most);
+      if (e != cudaSuccess) { m0_set_error("se_gate: cannot reserve %d bytes of shared memory (%s)", most, cudaGetErrorString(e)); return M0_ERR_CUDA; }
+      if (dev < 64) granted |= 1ull << dev;
+    }
+  }
+  se_gate_kernel<<<(B + 15) / 16, 320, smem, s>>>(pool, w1t, b1, w2t, b2, gate, B, C, hid, act);
   return m0_check_launch("se_gate");
 }
 

@@ -176,7 +176,9 @@ struct TcState {
   int sm_count = 148;
   int max_smem = 0;
   // dynamic shared memory already granted to the kernels ON THIS STATE'S DEVICE (cudaFuncSetAttribute is per device: a process-wide
-  // record would leave the kernels of a second device at the 48 KB default)
+  // record would leave the kernels of a second device at the 48 KB default).  The limit itself belongs to the kernel, shared by every
+  // net of the process, so every state grants the device's maximum: a grant of only what this net's launches need would lower the
+  // limit under a wider net's launches (invalid argument at its next launch).
   size_t smem_pair[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
   size_t smem_gemm = 0;
   TcWeight pst, inter;
@@ -361,9 +363,9 @@ int launch_conv_pair(TcState* st, const CUtensorMap& a_map, const TcWeight& w, i
                 : fz == 1 ? (nch <= 1 ? tc::conv_pair_kernel<1, 1> : nch <= 3 ? tc::conv_pair_kernel<3, 1> : tc::conv_pair_kernel<4, 1>)
                           : (nch <= 1 ? tc::conv_pair_kernel<1, 0> : nch <= 3 ? tc::conv_pair_kernel<3, 0> : tc::conv_pair_kernel<4, 0>);
   const int kidx = (nch <= 1 ? 0 : nch <= 3 ? 1 : 2) + 3 * fz;
-  if (smem > st->smem_pair[kidx]) {
-    M0_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    st->smem_pair[kidx] = smem;
+  if (st->smem_pair[kidx] < (size_t)st->max_smem) {
+    M0_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, st->max_smem));
+    st->smem_pair[kidx] = (size_t)st->max_smem;
   }
   const int tiles = (boards + 3) / 4;
   int clusters = st->sm_count / 2;
@@ -480,9 +482,9 @@ int launch_gemm(TcState* st, const CUtensorMap& a_map, const TcWeight& w, int M,
   if (stages < 2) { m0_set_error("tensor-core GEMM: tile does not fit in shared memory (N=%d)", N); return M0_ERR_ARG; }
   p.stages = stages;
   const size_t smem = (size_t)stages * stage_bytes + tc::EPI_STAGE_BYTES + 1024 + 256;
-  if (smem > st->smem_gemm) {
-    M0_CUDA_TRY(cudaFuncSetAttribute(tc::gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    st->smem_gemm = smem;
+  if (st->smem_gemm < (size_t)st->max_smem) {
+    M0_CUDA_TRY(cudaFuncSetAttribute(tc::gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, st->max_smem));
+    st->smem_gemm = (size_t)st->max_smem;
   }
   const int tiles = (M + tc::BM - 1) / tc::BM;
   const int cs = w.cluster;
@@ -668,7 +670,21 @@ int tc_net_prepare(::m0_net* n, cudaStream_t s) {
       if ((rc = m0_check_cuda(cudaMemcpy2DAsync(w2p, (size_t)rp * 4, n->w.pol_fc2_w, (size_t)r * 4, (size_t)r * 4, c.policy_size,
                                                 cudaMemcpyDeviceToDevice, s), "pad pol_fc2")) != M0_OK) break;
       if ((rc = make_weight(st, &st->pol_conv, n->w.pol_conv_w, 64, C, 64, s)) != M0_OK) break;
-      if ((rc = make_weight(st, &st->pol_fc1, n->w.pol_fc1_w, r, 4096, r, s)) != M0_OK) break;
+      // a rank above 256 would run as two MMAs of r / 2 columns: 136 and 152 (rank 272, 304) are no valid MMA width for 128 rows, and
+      // the second accumulator would start off a 32-column boundary.  Its weight rows are zero-padded to rp = 320 instead, which runs
+      // as two 160-column halves; only the r real columns are stored.
+      const int fc1_n = r > 256 ? rp : r;
+      if (fc1_n != r) {
+        float* w1p = nullptr;
+        if ((rc = m0_check_cuda(cudaMallocAsync((void**)&w1p, (size_t)fc1_n * 4096 * 4, s), "cudaMalloc pol_fc1")) != M0_OK) break;
+        rc = m0_check_cuda(cudaMemsetAsync(w1p, 0, (size_t)fc1_n * 4096 * 4, s), "memset pol_fc1");
+        if (rc == M0_OK) rc = m0_check_cuda(cudaMemcpyAsync(w1p, n->w.pol_fc1_w, (size_t)r * 4096 * 4, cudaMemcpyDeviceToDevice, s), "pad pol_fc1");
+        if (rc == M0_OK) rc = make_weight(st, &st->pol_fc1, w1p, fc1_n, 4096, fc1_n, s);
+        cudaFreeAsync(w1p, s);
+        if (rc != M0_OK) break;
+      } else if ((rc = make_weight(st, &st->pol_fc1, n->w.pol_fc1_w, r, 4096, r, s)) != M0_OK) {
+        break;
+      }
       if ((rc = make_weight(st, &st->pol_fc2, w2p, ps_pad, rp, 320, s)) != M0_OK) break;
       if ((rc = make_weight(st, &st->val_conv1, n->w.val_conv1_w, 128, C, 128, s)) != M0_OK) break;
       if ((rc = make_weight(st, &st->val_conv2, n->w.val_conv2_w, 128, 128, 128, s)) != M0_OK) break;
@@ -898,7 +914,8 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
   // policy: conv1x1 C->64, GN, act, fc1 + ReLU, fc2 * logit scale
   PROF("gemm_pol_conv", launch_gemm(st, st->a1_mat, st->pol_conv, M, 0, 1, C, 0, 64, n->t1, nullptr, 64, 0, none, ACT_NONE, 1.0f, s));
   PROF("gn_act_res", nn_gn_act_res(n->t1, w.pol_gn_w, w.pol_gn_b, nullptr, 0, nullptr, st->ph_h, B, 64, act, s));
-  PROF("gemm_pol_fc1", launch_gemm(st, st->ph_mat, st->pol_fc1, B, 0, 1, 4096, 0, r, nullptr, st->pf_h, rp, 0, w.pol_fc1_b, ACT_RELU, 1.0f, s));
+  PROF("gemm_pol_fc1", launch_gemm(st, st->ph_mat, st->pol_fc1, B, 0, 1, 4096, 0, st->pol_fc1.n, nullptr, st->pf_h, rp, 0, w.pol_fc1_b, ACT_RELU, 1.0f, s,
+                                   nullptr, nullptr, nullptr, r));
   // one launch over all 320-column slices of the (zero-padded) policy_fc2 weight; the padding columns are not stored
   PROF("gemm_pol_fc2", launch_gemm(st, st->pf_mat, st->pol_fc2, B, 0, 1, rp, 0, 320, logits, nullptr, c.policy_size, 0, w.pol_fc2_b, ACT_NONE,
                                    w.policy_logit_scale, s, nullptr, nullptr, nullptr, c.policy_size, (c.policy_size + 319) / 320));

@@ -2,7 +2,8 @@
 
 Plain PyTorch CPU ops on a reference-format ``state_dict`` (``azchess/model/resnet.py``), each step
 citing the reference lines it follows.  ``infer_amp_tower`` is forced off: this is the fp32 oracle
-(SURVEY Q11).  Pinned against the UNMODIFIED reference module (loaded with a stub ``chess``) in
+(SURVEY Q11).  ``forward`` runs in the state dict's dtype, so an fp64 state dict gives the fp64 reference of
+tests/tc_matrix_cases.py.  Pinned against the UNMODIFIED reference module (loaded with a stub ``chess``) in
 tests/test_oracle_nn.py where the reference tree is present, and through tests/golden/nn_golden.npz.
 ``make_state_dict`` produces deterministic weights from the parameter names so that goldens need
 to store outputs only.  Only tests/, smoke() and bench.py's CPU legs import this module.
@@ -90,7 +91,7 @@ def forward(sd: Dict[str, torch.Tensor], cfg, x: torch.Tensor, return_ssl: bool 
     """cfg: object with NetConfig attributes (matrix0_b200.model.NetConfig or the reference's)."""
     from matrix0_b200.model import SSL_ORDER, tower_layout
     act = cfg.activation
-    x = x.float()
+    x = x.to(sd["stem.0.weight"].dtype)   # an fp64 state dict gives an fp64 forward
     # stem + chess-specific features (always fp32), resnet.py:662-668, :229-244
     x = _act(_gn(F.conv2d(x, sd["stem.0.weight"], padding=1), sd["stem.1.weight"], sd["stem.1.bias"]), act)
     if cfg.chess_features:
