@@ -245,7 +245,9 @@ int m0_net_create(int device, const m0_net_config* cfg, const m0_net_weights* we
 int m0_net_destroy(m0_net* net);
 /* PolicyValueNet.forward (resnet.py:755-760): d_planes float32[B][planes][8][8] -> d_logits float32[B][4672], d_values
  * float32[B].  precision 0 = fp32 SIMT kernels (parity <= 1e-4), 1 = bf16 and 2 = fp16 operands on the tcgen05 tensor-core pipeline
- * (fp32 accumulation; fp16 is the reference's autocast dtype and the default of the Python layer). */
+ * (fp32 accumulation; fp16 is the reference's autocast dtype and the default of the Python layer), 3 = fp8: the fp16 pipeline with
+ * e4m3 operands for the residual tower's conv1 / conv2 (per-output-channel power-of-two weight scales, unscaled activations); it
+ * needs the fused CTA-pair tower (M0_ERR_ARG otherwise, e.g. se_hidden > 256). */
 int m0_net_forward(m0_net* net, const float* d_planes, int B, float* d_logits, float* d_values, int precision, void* stream);
 /* The dominant kernel on its own (tests, roofline micro-benchmark): tcgen05/TMA implicit GEMM over bf16 operands.
  * taps = 9: 3x3 "same" convolution of NHWC activations d_act_bf16[boards][8][8][cin] with d_w_bf16[n][9*cin]
@@ -254,8 +256,13 @@ int m0_net_forward(m0_net* net, const float* d_planes, int B, float* d_logits, f
  * of each tap is half empty: the activations are zero-filled past cin, and 3x3 weights are copied with each tap padded to whole
  * k-blocks (stream-ordered allocation, freed after the launch). */
 int m0_tc_conv(const uint16_t* d_act_bf16, const uint16_t* d_w_bf16, int boards, int cin, int n, int taps, float* d_out_f32, void* stream);
+/* The e4m3 counterpart of m0_tc_conv (3x3 only, the kernel of precision 3): d_out_f32[boards*64][n] = d_w_scale[n] *
+ * conv3x3(d_act_e4m3[boards][8][8][cin], d_w_e4m3[n][9*cin]), accumulated in fp32.  boards even, cin % 32 == 0, cin <= 512,
+ * n % 32 == 0, 64 <= n <= 320.  The weights are copied with each tap padded to whole 128-channel k-blocks when cin % 128 != 0. */
+int m0_tc_conv_fp8(const uint8_t* d_act_e4m3, const uint8_t* d_w_e4m3, const float* d_w_scale, int boards, int cin, int n, float* d_out_f32,
+                   void* stream);
 /* Per-launch-site CUDA-event timing of the tensor-core forward (measurement aid, no reference counterpart): after
- * m0_profile_enable(1) every kernel launch of m0_net_forward (precision 1, 2) is bracketed by events on its stream;
+ * m0_profile_enable(1) every kernel launch of m0_net_forward (precision 1, 2, 3) is bracketed by events on its stream;
  * m0_profile_get returns the accumulated milliseconds and launch count of one site ("conv1+gn", "conv2+pool",
  * "se_apply_gn", "attention_tc", ... ; NULL = all sites).  m0_profile_enable(0) switches it off and clears the table. */
 int m0_profile_enable(int enable);

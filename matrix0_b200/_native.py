@@ -20,6 +20,9 @@ class NativeLibraryError(RuntimeError):
     pass
 
 
+M0_ERR_ARG = -2   # include/matrix0_b200.h: invalid argument
+
+
 _lib: Optional[ctypes.CDLL] = None
 
 # name -> (restype, argtypes); kept in one table so tests can check every header symbol is exported
@@ -73,6 +76,7 @@ SIGNATURES = {
     "m0_net_destroy": (c_int, [c_void_p]),
     "m0_net_forward": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p]),
     "m0_tc_conv": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "m0_tc_conv_fp8": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "m0_profile_enable": (c_int, [c_int]),
     "m0_profile_get": (c_int, [c_char_p, ctypes.POINTER(c_double), ctypes.POINTER(ctypes.c_longlong)]),
     "m0_net_forward_ssl": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),

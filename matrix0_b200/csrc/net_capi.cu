@@ -1,6 +1,6 @@
 // C-ABI of the evaluator: PolicyValueNet.forward (azchess/model/resnet.py:755-760) as a sequence of
 // CUDA kernel launches on the caller's stream.  precision 0 = fp32 SIMT path (parity within 1e-4),
-// precision 1 = bf16 tensor-core path (nn_tc_kernels.cu).
+// precision 1 / 2 = bf16 / fp16 tensor-core path, 3 = fp8 (fp16 with e4m3 tower convolutions) (nn_tc_kernels.cu).
 #include "net_host.cuh"
 #include <new>
 #include <string.h>
@@ -148,15 +148,15 @@ int m0_net_destroy(m0_net* n) {
 }
 
 // PolicyValueNet.forward(x) (resnet.py:755-760): d_planes float32[B][planes][8][8] -> d_logits float32[B][4672],
-// d_values float32[B].  precision: 0 = fp32, 1 = bf16 tensor cores.
+// d_values float32[B].  precision: 0 = fp32, 1 = bf16, 2 = fp16, 3 = fp8 tensor cores.
 int m0_net_forward(m0_net* n, const float* d_planes, int B, float* d_logits, float* d_values, int precision, void* stream) {
   if (!n || !d_planes || !d_logits || !d_values || B < 0) { m0_set_error("m0_net_forward: invalid argument"); return M0_ERR_ARG; }
   if (B == 0) return M0_OK;
   cudaStream_t s = (cudaStream_t)stream;
-  if (precision == 1 || precision == 2) {  // 1 = bf16, 2 = fp16 operands (fp32 accumulate)
-    nn_set_half_format(precision == 2);
-    TRY(tc_net_prepare(n, s));
-    return tc_net_forward(n, d_planes, B, d_logits, d_values, s);
+  if (precision >= 1 && precision <= 3) {  // 1 = bf16, 2 = fp16 operands, 3 = fp16 with e4m3 tower convolutions (fp32 accumulate)
+    nn_set_half_format(precision >= 2);
+    TRY(tc_net_prepare(n, precision - 1, s));
+    return tc_net_forward(n, precision - 1, d_planes, B, d_logits, d_values, s);
   }
   TRY(ws_reserve(n, B));
   TRY(forward_features_f32(n, d_planes, B, s));

@@ -17,7 +17,8 @@ struct m0_net {
 namespace m0 {
 int net_ws_reserve(::m0_net* n, int B);
 int net_forward_heads_f32(::m0_net* n, int B, float* logits, float* values, cudaStream_t s);
-int tc_net_prepare(::m0_net* net, cudaStream_t s);
-int tc_net_forward(::m0_net* net, const float* d_planes, int B, float* d_logits, float* d_values, cudaStream_t s);
+// slot: 0 = bf16, 1 = fp16, 2 = fp8 (e4m3 tower convolutions, fp16 elsewhere)
+int tc_net_prepare(::m0_net* net, int slot, cudaStream_t s);
+int tc_net_forward(::m0_net* net, int slot, const float* d_planes, int B, float* d_logits, float* d_values, cudaStream_t s);
 void tc_net_release(::m0_net* net);
 }  // namespace m0

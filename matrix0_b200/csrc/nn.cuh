@@ -25,7 +25,7 @@ int nn_layernorm_residual_f32(const float* proj, const float* x, const float* ga
                               cudaStream_t s);
 int nn_nhwc_to_nchw_f32(const float* in, float* out, int B, int C, cudaStream_t s);
 int nn_ln_res_gn(const void* proj, int proj_half, float* x, const float* ln_g, const float* ln_b, const float* gn_g, const float* gn_b,
-                 __nv_bfloat16* a_out, int B, int C, int act, cudaStream_t s);
+                 __nv_bfloat16* a_out, int B, int C, int act, cudaStream_t s, bool a_e4m3 = false);
 
 }  // namespace m0
 

@@ -7,6 +7,7 @@
 // W[n][k], k = (ky*3 + kx)*Cin + ci for 3x3 convolutions).
 #include "nn.cuh"
 #include <cuda_fp16.h>
+#include <cuda_fp8.h>
 
 namespace m0 {
 
@@ -292,6 +293,7 @@ __global__ void layernorm_residual_f32_kernel(const float* __restrict__ proj, co
 // take no part in the LayerNorm statistics or the stores.
 // HALF_IN: proj is the 16-bit output of the projection GEMM (the reference's proj convolution runs under autocast, resnet.py:676-677);
 // gn_g == nullptr with a_out != nullptr: a_out = half(x_new) without the GroupNorm (the operand of the head GEMMs after the last block)
+// fp16 = 2 (precision fp8): 16-bit values are fp16 and the GroupNorm'ed a_out is e4m3 (the operand of the next e4m3 conv1)
 template <int C, bool HALF_IN>
 __global__ void __launch_bounds__(256, 2)
 ln_res_gn_kernel(const float* __restrict__ proj, float* __restrict__ x, const float* __restrict__ ln_g, const float* __restrict__ ln_b,
@@ -427,6 +429,11 @@ ln_res_gn_kernel(const float* __restrict__ proj, float* __restrict__ x, const fl
         float y0 = fmaf(v[t][2 * j], g0, b0), y1 = fmaf(v[t][2 * j + 1], g1, b1);
         if (act == ACT_SILU) { y0 = __fdividef(y0, 1.0f + __expf(-y0)); y1 = __fdividef(y1, 1.0f + __expf(-y1)); }
         else if (act == ACT_RELU) { y0 = fmaxf(y0, 0.f); y1 = fmaxf(y1, 0.f); }
+        if (fp16 == 2) {
+          *reinterpret_cast<uint16_t*>(reinterpret_cast<uint8_t*>(a_out) + base + (size_t)t * C + 64 * j) =
+              __nv_cvt_float2_to_fp8x2(make_float2(y0, y1), __NV_SATFINITE, __NV_E4M3);
+          continue;
+        }
         uint32_t pk;
         if (fp16) { __half2 h = __floats2half2_rn(y0, y1); pk = *reinterpret_cast<uint32_t*>(&h); }
         else { __nv_bfloat162 h = __floats2bfloat162_rn(y0, y1); pk = *reinterpret_cast<uint32_t*>(&h); }
@@ -493,8 +500,8 @@ int nn_layernorm_residual_f32(const float* proj, const float* x, const float* ga
 }
 // x <- LN(proj + x) in place; a_out (optional) = half(act(GroupNorm(x))) with the next block's bn1 parameters
 int nn_ln_res_gn(const void* proj, int proj_half, float* x, const float* ln_g, const float* ln_b, const float* gn_g, const float* gn_b,
-                 __nv_bfloat16* a_out, int B, int C, int act, cudaStream_t s) {
-  const int fp16 = g_half_fp16;
+                 __nv_bfloat16* a_out, int B, int C, int act, cudaStream_t s, bool a_e4m3) {
+  const int fp16 = a_e4m3 ? 2 : g_half_fp16;
   const float* p = reinterpret_cast<const float*>(proj);
 #define M0_LN_CASE(C)                                                                                                     \
   if (proj_half) ln_res_gn_kernel<C, true><<<B, 256, 0, s>>>(p, x, ln_g, ln_b, gn_g, gn_b, a_out, act, fp16);             \

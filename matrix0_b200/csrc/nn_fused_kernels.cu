@@ -2,6 +2,7 @@
 // written once per residual block.
 #include "nn.cuh"
 #include <cuda_fp16.h>
+#include <cuda_fp8.h>
 
 namespace m0 {
 
@@ -22,7 +23,8 @@ __device__ __forceinline__ __nv_bfloat16 fk_half(float x, int fp16) {
 
 // x_new = x + conv_out * gate   (SE excitation + residual add, resnet.py:68-80)
 // a_out = half(act(GroupNorm(x_new)))   (bn1 + activation of the NEXT pre-activation block, resnet.py:46-47), or half(x_new) when
-// gamma is null, or nothing when a_out is null.  conv_out is the 16-bit output of conv2 (operand format).
+// gamma is null, or nothing when a_out is null.  conv_out is the 16-bit output of conv2 (operand format).  fp16 = 2 (precision fp8):
+// 16-bit values are fp16 and the GroupNorm'ed a_out is e4m3 (the operand of the next e4m3 conv1).
 // One block per board, C threads.  Thread (rg, q) owns 8 consecutive channels of 8 rows: every access is 16 bytes wide (8 halves or
 // one of two float4), x and conv_out are read once, x_new / a_out written once.  GroupNorm statistics: 2 adjacent threads (= 16
 // channels) x 8 row groups per group.
@@ -46,6 +48,12 @@ __device__ __forceinline__ uint32_t fk_pack2(float a, float b, int fp16) {
   }
   __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
   return *reinterpret_cast<uint32_t*>(&t);
+}
+
+__device__ __forceinline__ uint32_t fk_e4m3x4(float a, float b, float c, float d) {
+  const uint32_t lo = __nv_cvt_float2_to_fp8x2(make_float2(a, b), __NV_SATFINITE, __NV_E4M3);
+  const uint32_t hi = __nv_cvt_float2_to_fp8x2(make_float2(c, d), __NV_SATFINITE, __NV_E4M3);
+  return lo | (hi << 16);
 }
 
 __global__ void __launch_bounds__(320, 2)
@@ -140,6 +148,10 @@ se_apply_gn_kernel(const __nv_bfloat16* __restrict__ conv_out, const float* __re
     float y[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) y[j] = fk_act(fmaf(v[r][j], gsc[j], bsh[j]), act);
+    if (fp16 == 2) {
+      *reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(a_out) + base + (size_t)r * C) = make_uint2(fk_e4m3x4(y[0], y[1], y[2], y[3]), fk_e4m3x4(y[4], y[5], y[6], y[7]));
+      continue;
+    }
     *reinterpret_cast<uint4*>(ao + (size_t)r * C) =
         make_uint4(fk_pack2(y[0], y[1], fp16), fk_pack2(y[2], y[3], fp16), fk_pack2(y[4], y[5], fp16), fk_pack2(y[6], y[7], fp16));
   }
@@ -328,10 +340,10 @@ int nn_se_gate(const float* pool, const float* w1t, const float* b1, const float
 }
 
 int nn_se_apply_gn(const __nv_bfloat16* conv_out, const float* gate, float* x, const float* gamma, const float* beta, __nv_bfloat16* a_out, int B,
-                   int C, int act, cudaStream_t s) {
+                   int C, int act, cudaStream_t s, bool a_e4m3) {
   if (C > 320 || C % 32 != 0) { m0_set_error("se_apply_gn: unsupported channel count %d", C); return M0_ERR_ARG; }
   if (C % 16 != 0) { m0_set_error("se_apply_gn: channels must be a multiple of 16"); return M0_ERR_ARG; }
-  se_apply_gn_kernel<<<B, C, 0, s>>>(conv_out, gate, x, gamma, beta, a_out, C, act, nn_half_format());
+  se_apply_gn_kernel<<<B, C, 0, s>>>(conv_out, gate, x, gamma, beta, a_out, C, act, a_e4m3 ? 2 : nn_half_format());
   return m0_check_launch("se_apply_gn");
 }
 int nn_gn_act_res(const float* x, const float* gamma, const float* beta, const float* residual, long long residual_bstride, float* out,

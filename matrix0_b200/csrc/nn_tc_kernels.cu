@@ -1,4 +1,5 @@
-// Tensor-core path of PolicyValueNet.forward (precision fp16 = default, or bf16): the 3x3 convolutions of the trunk run on the CTA-pair
+// Tensor-core path of PolicyValueNet.forward (precision fp16 = default, bf16, or fp8: fp16 with e4m3 operands for the residual tower's
+// conv1 / conv2, see tc_net_prepare): the 3x3 convolutions of the trunk run on the CTA-pair
 // tcgen05 kernel of tc_conv_pair.cuh, the 1x1 convolutions / linear layers on the single-CTA tcgen05 GEMM of tc_gemm.cuh (16-bit operands,
 // fp32 accumulation in tensor memory); normalisation statistics, the SE gate, softmax and the last value layers stay in fp32.
 // This file owns the per-network device state (16-bit weights, TMA tensor maps, activation buffers) and issues the launches.
@@ -20,7 +21,7 @@ using namespace m0;
 
 namespace m0 {
 int nn_se_apply_gn(const __nv_bfloat16* conv_out, const float* gate, float* x, const float* gamma, const float* beta, __nv_bfloat16* a_out, int B,
-                   int C, int act, cudaStream_t s);
+                   int C, int act, cudaStream_t s, bool a_e4m3 = false);
 int nn_planes_to_nhwc_half(const float* planes, __nv_bfloat16* out, int B, int P, cudaStream_t s);
 int nn_se_hidden(const float* part, int splits, long long split_stride, const float* b1, __nv_bfloat16* hidden, int B, int hid, int ld, int act,
                  cudaStream_t s);
@@ -85,6 +86,40 @@ __global__ void pad_cols_kernel(const T* __restrict__ in, T* __restrict__ out, i
   const int r = i / cols_pad, c = i - r * cols_pad;
   out[i] = c < cols ? in[r * cols + c] : T(0);
 }
+// e4m3 weights of a 3x3 convolution, one block per output channel n: w [n][9][cin] fp32 -> q [n][9][cin_pad] e4m3 (taps zero-padded
+// to whole 128-channel k-blocks), q = e4m3_rn_satfinite(w * s_n) with the power-of-two scale s_n = 2^floor(log2(448 / max|w_n|)) (1 for
+// an all-zero row) that lifts the row out of e4m3's subnormal range; dq[n] = 1 / s_n (exact).  deq (optional) [n][9][cin] = q / s_n,
+// the weights the tensor cores actually multiply by (the SE fold of conv2 is built from them).
+__global__ void quantize_e4m3_kernel(const float* __restrict__ w, uint8_t* __restrict__ q, float* __restrict__ dq, float* __restrict__ deq, int cin,
+                                     int cin_pad) {
+  __shared__ float s_max[32];
+  const int n = blockIdx.x;
+  const float* row = w + (size_t)n * 9 * cin;
+  float m = 0.f;
+  for (int i = threadIdx.x; i < 9 * cin; i += blockDim.x) m = fmaxf(m, fabsf(row[i]));
+  for (int off = 16; off > 0; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xFFFFFFFFu, m, off));
+  if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = m;
+  __syncthreads();
+  m = 0.f;
+  for (int i = 0; i < (int)(blockDim.x >> 5); ++i) m = fmaxf(m, s_max[i]);
+  // floor(log2(448 / m)) exactly: m = f * 2^k with f in [1, 2), 448 = 1.75 * 2^8
+  int e = 0;
+  if (m > 0.f) {
+    int k2;
+    const float f = 2.0f * frexpf(m, &k2);
+    e = (f <= 1.75f ? 8 : 7) - (k2 - 1);
+    e = max(-126, min(126, e));
+  }
+  const float sc = ldexpf(1.0f, e), inv = ldexpf(1.0f, -e);
+  if (threadIdx.x == 0) dq[n] = inv;
+  for (int i = threadIdx.x; i < 9 * cin_pad; i += blockDim.x) {
+    const int t = i / cin_pad, c = i - t * cin_pad;
+    const float v = c < cin ? row[t * cin + c] : 0.f;
+    const __nv_fp8_storage_t b = __nv_cvt_float_to_fp8(v * sc, __NV_SATFINITE, __NV_E4M3);
+    q[(size_t)n * 9 * cin_pad + i] = b;
+    if (deq && c < cin) deq[(size_t)n * 9 * cin + t * cin + c] = __half2float(__half(__nv_cvt_fp8_to_halfraw(b, __NV_E4M3))) * inv;
+  }
+}
 }  // namespace m0
 
 namespace {
@@ -103,43 +138,44 @@ EncodeTiledFn get_encode() {
   return fn;
 }
 
-// 2-D bf16 row-major matrix [rows][cols], box {64 cols, box_rows}, 128-byte swizzle, zero fill outside
-int make_map_2d(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows) {
+// 2-D bf16 row-major matrix [rows][cols], box {64 cols, box_rows}, 128-byte swizzle, zero fill outside (e4m3: bytes, box {128 cols, box_rows})
+int make_map_2d(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows, bool e4m3 = false) {
   EncodeTiledFn enc = get_encode();
   if (!enc) { m0_set_error("cuTensorMapEncodeTiled is not available from the driver"); return M0_ERR_CUDA; }
   cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {cols * 2};
-  cuuint32_t box[2] = {64, box_rows};
+  cuuint64_t strides[1] = {cols * (e4m3 ? 1 : 2)};
+  cuuint32_t box[2] = {e4m3 ? 128u : 64u, box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+  CUresult r = enc(m, e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) { m0_set_error("cuTensorMapEncodeTiled(2d %llu x %llu) failed: %d", (unsigned long long)rows, (unsigned long long)cols, (int)r); return M0_ERR_CUDA; }
   return M0_OK;
 }
 
-// 4-D view of NHWC activations [boards][8][8][C] bf16: dims {C, 8, 8, boards}, box {64, 8, 8, 2}
-int make_map_nhwc(CUtensorMap* m, const void* ptr, uint64_t boards, uint64_t C, uint32_t box_x = 8) {
+// 4-D view of NHWC activations [boards][8][8][C] bf16: dims {C, 8, 8, boards}, box {64, 8, 8, 2} (e4m3: bytes, box {128, 8, 8, 2})
+int make_map_nhwc(CUtensorMap* m, const void* ptr, uint64_t boards, uint64_t C, uint32_t box_x = 8, bool e4m3 = false) {
   EncodeTiledFn enc = get_encode();
   if (!enc) { m0_set_error("cuTensorMapEncodeTiled is not available from the driver"); return M0_ERR_CUDA; }
+  const uint64_t es = e4m3 ? 1 : 2;
   cuuint64_t dims[4] = {C, 8, 8, boards};
-  cuuint64_t strides[3] = {C * 2, C * 2 * 8, C * 2 * 64};
-  cuuint32_t box[4] = {64, box_x, 8, 2};   // box_x = 10: the CTA-pair kernel's x-padded box (tc_conv_pair.cuh)
+  cuuint64_t strides[3] = {C * es, C * es * 8, C * es * 64};
+  cuuint32_t box[4] = {e4m3 ? 128u : 64u, box_x, 8, 2};   // box_x = 10: the CTA-pair kernel's x-padded box (tc_conv_pair.cuh)
   cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+  CUresult r = enc(m, e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) { m0_set_error("cuTensorMapEncodeTiled(nhwc boards=%llu C=%llu) failed: %d", (unsigned long long)boards, (unsigned long long)C, (int)r); return M0_ERR_CUDA; }
   return M0_OK;
 }
 
-// row-major output tensor [rows][cols] (16-bit or fp32) written by the pair kernel's bulk stores: box {16 columns, 32 rows}, no swizzle
-int make_map_out(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, bool fp32, bool swizzle64 = false) {
+// row-major output tensor [rows][cols] (16-bit, fp32 or e4m3 bytes) written by the pair kernel's bulk stores: box {16 columns, 32 rows}, no swizzle
+int make_map_out(CUtensorMap* m, const void* ptr, uint64_t rows, uint64_t cols, bool fp32, bool swizzle64 = false, bool e4m3 = false) {
   EncodeTiledFn enc = get_encode();
   if (!enc) { m0_set_error("cuTensorMapEncodeTiled is not available from the driver"); return M0_ERR_CUDA; }
   cuuint64_t dims[2] = {cols, rows};
-  cuuint64_t strides[1] = {cols * (fp32 ? 4 : 2)};
+  cuuint64_t strides[1] = {cols * (fp32 ? 4 : e4m3 ? 1 : 2)};
   cuuint32_t box[2] = {16, 32};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(m, fp32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
+  CUresult r = enc(m, fp32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : e4m3 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) { m0_set_error("cuTensorMapEncodeTiled(out %llu x %llu) failed: %d", (unsigned long long)rows, (unsigned long long)cols, (int)r); return M0_ERR_CUDA; }
@@ -153,6 +189,8 @@ struct TcWeight {
   bool pair = false;
   int n = 0, k = 0, n_part = 0, cluster = 1;
   int n_launch = 0;            // output channels per launch / slice
+  bool fp8 = false;            // e4m3 3x3 weights [n][9][cin padded to 128] (map_pair only), dequantised by dq[n]
+  const float* dq = nullptr;
 };
 
 // CTAs per cluster for a launch: the W tile is multicast within the cluster (M0_TC_CLUSTER overrides)
@@ -175,11 +213,12 @@ struct TcBlock {
 struct TcState {
   int sm_count = 148;
   int max_smem = 0;
+  bool fp8 = false;   // precision fp8: the tower's conv1 / conv2 take e4m3 operands (a1 / a2 hold e4m3 when a convolution reads them)
   // dynamic shared memory already granted to the kernels ON THIS STATE'S DEVICE (cudaFuncSetAttribute is per device: a process-wide
   // record would leave the kernels of a second device at the 48 KB default).  The limit itself belongs to the kernel, shared by every
   // net of the process, so every state grants the device's maximum: a grant of only what this net's launches need would lower the
   // limit under a wider net's launches (invalid argument at its next launch).
-  size_t smem_pair[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  size_t smem_pair[15] = {};   // 16-bit kernels 0..8, e4m3 kernels 9..14
   size_t smem_gemm = 0;
   TcWeight pst, inter;
   std::vector<TcBlock> blocks;
@@ -216,6 +255,8 @@ struct TcState {
   const void* x_ptr = nullptr;
   CUtensorMap qkv_out, t2f_out;                   // qkv (half, 3C columns) and n->t2 as fp32 (attention projection)
   CUtensorMap a1_out, a2_out, t1_out, t2h_out;    // output maps of the pair kernel's bulk stores (a1, a2 half; n->t1 fp32; n->t2 as half)
+  CUtensorMap a1_out8;                            // fp8: a1 as e4m3 (conv2's epilogue writing the next block's conv1 operand)
+  CUtensorMap a1_convp8, a2_convp8;               // fp8: x-padded e4m3 boxes of a1 / a2 for the tower's conv1 / conv2
   const void *t1_ptr = nullptr, *t2_ptr = nullptr;
   int out_rows = 0;
   std::vector<void*> allocs;
@@ -331,9 +372,11 @@ int launch_conv_pair(TcState* st, const CUtensorMap& a_map, const TcWeight& w, i
   memset(&p, 0, sizeof(p));
   p.boards = boards;
   p.N = w.n_launch;
-  p.kb_per_tap = kblocks_for(cin);
+  p.kb_per_tap = w.fp8 ? (cin + 127) / 128 : kblocks_for(cin);
   p.conv = conv;
   p.n_slices = n_slices;
+  p.w_dq = w.dq;
+  if (w.fp8 && (!conv || n_slices != 1)) { m0_set_error("pair kernel: e4m3 operands need the 3x3 mode"); return M0_ERR_ARG; }
   if (n_slices > 1 && (gn_gamma || pool_part || fuse)) { m0_set_error("pair kernel: fused epilogues need a single slice"); return M0_ERR_ARG; }
   p.fp16 = nn_half_format();
   p.out_f32 = out_f32;
@@ -358,11 +401,14 @@ int launch_conv_pair(TcState* st, const CUtensorMap& a_map, const TcWeight& w, i
   const size_t smem = (size_t)stages * stage_bytes + a_res + epi_bytes + 1024 + 512;
   // epilogue register tile: 16-column chunks per warp = ceil((N / 2 / 16) / CP_CSETS)
   const int nch = (w.n_launch / 32 + tc::CP_CSETS - 1) / tc::CP_CSETS;
-  if (nch > 4) { m0_set_error("pair kernel: N = %d is too wide", w.n_launch); return M0_ERR_ARG; }
-  auto kernel = fz == 2 ? (nch <= 1 ? tc::conv_pair_kernel<1, 2> : nch <= 3 ? tc::conv_pair_kernel<3, 2> : tc::conv_pair_kernel<4, 2>)
+  if (nch > 4 || (w.fp8 && nch > 3)) { m0_set_error("pair kernel: N = %d is too wide", w.n_launch); return M0_ERR_ARG; }
+  auto kernel = w.fp8 ? (fz == 2 ? (nch <= 1 ? tc::conv_pair_kernel<1, 2, true> : tc::conv_pair_kernel<3, 2, true>)
+                         : fz == 1 ? (nch <= 1 ? tc::conv_pair_kernel<1, 1, true> : tc::conv_pair_kernel<3, 1, true>)
+                                   : (nch <= 1 ? tc::conv_pair_kernel<1, 0, true> : tc::conv_pair_kernel<3, 0, true>))
+              : fz == 2 ? (nch <= 1 ? tc::conv_pair_kernel<1, 2> : nch <= 3 ? tc::conv_pair_kernel<3, 2> : tc::conv_pair_kernel<4, 2>)
                 : fz == 1 ? (nch <= 1 ? tc::conv_pair_kernel<1, 1> : nch <= 3 ? tc::conv_pair_kernel<3, 1> : tc::conv_pair_kernel<4, 1>)
                           : (nch <= 1 ? tc::conv_pair_kernel<1, 0> : nch <= 3 ? tc::conv_pair_kernel<3, 0> : tc::conv_pair_kernel<4, 0>);
-  const int kidx = (nch <= 1 ? 0 : nch <= 3 ? 1 : 2) + 3 * fz;
+  const int kidx = w.fp8 ? 9 + (nch <= 1 ? 0 : 1) + 2 * fz : (nch <= 1 ? 0 : nch <= 3 ? 1 : 2) + 3 * fz;
   if (st->smem_pair[kidx] < (size_t)st->max_smem) {
     M0_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, st->max_smem));
     st->smem_pair[kidx] = (size_t)st->max_smem;
@@ -418,6 +464,28 @@ int make_weight(TcState* st, TcWeight* out, const float* w_f32, int n, int k, in
   out->pair = pair_ok(n_launch) && n % n_launch == 0;
   if (out->pair) TRY(make_map_2d(&out->map_pair, out->w, (uint64_t)n, (uint64_t)k, (uint32_t)(n_launch / 4)));
   return make_map_2d(&out->map, out->w, (uint64_t)n, (uint64_t)k, (uint32_t)(out->n_part / out->cluster));
+}
+
+// e4m3 weights of a 3x3 convolution w_f32 [n][9][cin] for the CTA-pair kernel (quantize_e4m3_kernel); deq (optional, [n][9][cin] fp32)
+// receives the dequantised values
+int make_weight_fp8(TcState* st, TcWeight* out, const float* w_f32, int n, int cin, cudaStream_t s, float* deq = nullptr) {
+  const int cin_pad = (cin + 127) / 128 * 128, k = 9 * cin_pad;
+  void *q = nullptr, *dq = nullptr;
+  M0_CUDA_TRY(cudaMalloc(&q, (size_t)n * k));
+  st->allocs.push_back(q);
+  M0_CUDA_TRY(cudaMalloc(&dq, (size_t)n * 4));
+  st->allocs.push_back(dq);
+  quantize_e4m3_kernel<<<n, 256, 0, s>>>(w_f32, (uint8_t*)q, (float*)dq, deq, cin, cin_pad);
+  TRY(m0_check_launch("quantize_e4m3"));
+  out->w = (__nv_bfloat16*)q;
+  out->n = out->n_launch = n;
+  out->k = k;
+  out->n_part = n_part_for(n);
+  out->cluster = 1;
+  out->pair = true;
+  out->fp8 = true;
+  out->dq = (const float*)dq;
+  return make_map_2d(&out->map_pair, q, (uint64_t)n, (uint64_t)k, (uint32_t)(n / 4), true);
 }
 
 int pow2_cols(int n) {
@@ -605,6 +673,10 @@ int tc_reserve(m0_net* n, TcState* st, int B) {
   TRY(make_map_nhwc(&st->a2_conv, st->a2, need, C));
   TRY(make_map_nhwc(&st->a1_convp, st->a1, need, C, 10));
   TRY(make_map_nhwc(&st->a2_convp, st->a2, need, C, 10));
+  if (st->fp8) {
+    TRY(make_map_nhwc(&st->a1_convp8, st->a1, need, C, 10, true));
+    TRY(make_map_nhwc(&st->a2_convp8, st->a2, need, C, 10, true));
+  }
   st->t1_ptr = st->t2_ptr = nullptr;   // the output maps are rebuilt on the next forward
   TRY(make_map_2d(&st->a1_mat, st->a1, (uint64_t)need * 64, C, 128));
   TRY(make_map_2d(&st->a2_mat, st->a2, (uint64_t)need * 64, C, 128));
@@ -617,22 +689,33 @@ int tc_reserve(m0_net* n, TcState* st, int B) {
 namespace m0 {
 
 struct TcStates {
-  TcState* st[2] = {nullptr, nullptr};
+  TcState* st[3] = {nullptr, nullptr, nullptr};   // by slot: bf16, fp16, fp8
 };
 
-int tc_net_prepare(::m0_net* n, cudaStream_t s) {
+// slot 0 = bf16, 1 = fp16, 2 = fp8 (fp16 with e4m3 tower convolutions; the 16-bit format of the process must be fp16)
+int tc_net_prepare(::m0_net* n, int slot, cudaStream_t s) {
   if (!n->tc) n->tc = new (std::nothrow) TcStates();
   TcStates* all = (TcStates*)n->tc;
   if (!all) { m0_set_error("out of host memory"); return M0_ERR_ARG; }
-  const int fmt = nn_half_format();
-  if (all->st[fmt]) return M0_OK;
+  if (all->st[slot]) return M0_OK;
   const m0_net_config& c = n->cfg;
   if (c.channels % 32 != 0 || c.channels < 64 || c.channels > 320) {
     m0_set_error("16-bit tensor-core path needs channels %% 32 == 0 and 64 <= channels <= 320 (got %d)", c.channels);
     return M0_ERR_ARG;
   }
+  const bool fp8 = slot == 2;
+  const bool se_fused = env_int("M0_TC_FUSE_SE", 1) != 0 && pair_ok(c.channels) && (!c.se || c.se_hidden <= 256);
+  if (fp8 && !se_fused) {
+    // the e4m3 tower convolutions exist only as variants of the fused CTA-pair pipeline
+    m0_set_error("fp8 precision needs the fused CTA-pair pipeline of the tower: %s",
+                 !pair_ok(c.channels) ? "the CTA-pair convolution is off (M0_TC_PAIR=0)"
+                 : env_int("M0_TC_FUSE_SE", 1) == 0 ? "the fused SE / residual epilogue is off (M0_TC_FUSE_SE=0)"
+                                                   : "se_hidden > 256 runs the unfused SE path");
+    return M0_ERR_ARG;
+  }
   TcState* st = new (std::nothrow) TcState();
   if (!st) { m0_set_error("out of host memory"); return M0_ERR_ARG; }
+  st->fp8 = fp8;
   cudaDeviceGetAttribute(&st->sm_count, cudaDevAttrMultiProcessorCount, n->device);
   cudaDeviceGetAttribute(&st->max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, n->device);
   const int C = c.channels;
@@ -705,23 +788,33 @@ int tc_net_prepare(::m0_net* n, cudaStream_t s) {
     }
     // fused SE + residual epilogue of conv2 (M0_TC_FUSE_SE=0 keeps the separate SE / residual kernels)
     st->hid_pad = (c.se_hidden + 63) / 64 * 64;
-    st->se_fused = env_int("M0_TC_FUSE_SE", 1) != 0 && pair_ok(C) && (!c.se || c.se_hidden <= 256);
+    st->se_fused = se_fused;
     st->blocks.resize(c.blocks);
     for (int i = 0; i < c.blocks && rc == M0_OK; ++i) {
       const m0_block_weights& b = n->w.blocks[i];
-      if ((rc = make_weight(st, &st->blocks[i].conv1, b.conv1_w, C, 9 * C, C, s, 9)) != M0_OK) break;
-      if ((rc = make_weight(st, &st->blocks[i].conv2, b.conv2_w, C, 9 * C, C, s, 9)) != M0_OK) break;
+      // fp8: the SE fold of conv2 is built from the dequantised e4m3 weights (the ones conv2 multiplies by)
+      float* conv2_deq = nullptr;
+      if (fp8) {
+        if ((rc = make_weight_fp8(st, &st->blocks[i].conv1, b.conv1_w, C, C, s)) != M0_OK) break;
+        if (c.se && (rc = m0_check_cuda(cudaMallocAsync((void**)&conv2_deq, (size_t)C * 9 * C * 4, s), "cudaMalloc conv2_deq")) != M0_OK) break;
+        rc = make_weight_fp8(st, &st->blocks[i].conv2, b.conv2_w, C, C, s, conv2_deq);
+        if (rc != M0_OK) { if (conv2_deq) cudaFreeAsync(conv2_deq, s); break; }
+      } else {
+        if ((rc = make_weight(st, &st->blocks[i].conv1, b.conv1_w, C, 9 * C, C, s, 9)) != M0_OK) break;
+        if ((rc = make_weight(st, &st->blocks[i].conv2, b.conv2_w, C, 9 * C, C, s, 9)) != M0_OK) break;
+      }
       if (st->se_fused && c.se) {
         // the first SE GEMM runs hid16 = hid rounded up to 16 output columns (the MMA width granule); the extra rows of the folded
         // weight are zero and their columns are not stored
         const int hid = c.se_hidden, hid16 = (hid + 15) / 16 * 16, K = 12 * C, hp = st->hid_pad;
         float *fold = nullptr, *w2p = nullptr;
-        if ((rc = m0_check_cuda(cudaMalloc((void**)&fold, (size_t)hid16 * K * 4), "cudaMalloc se_fold")) != M0_OK) break;
+        if ((rc = m0_check_cuda(cudaMalloc((void**)&fold, (size_t)hid16 * K * 4), "cudaMalloc se_fold")) != M0_OK) { if (conv2_deq) cudaFreeAsync(conv2_deq, s); break; }
         st->allocs.push_back(fold);
         if ((rc = m0_check_cuda(cudaMemsetAsync(fold, 0, (size_t)hid16 * K * 4, s), "memset se_fold")) != M0_OK) break;
         if ((rc = m0_check_cuda(cudaMalloc((void**)&w2p, (size_t)C * hp * 4), "cudaMalloc se_w2")) != M0_OK) break;
         st->allocs.push_back(w2p);
-        se_fold_kernel<<<(hid * K + 255) / 256, 256, 0, s>>>(b.conv2_w, b.se_w1, fold, C, hid);
+        se_fold_kernel<<<(hid * K + 255) / 256, 256, 0, s>>>(conv2_deq ? conv2_deq : b.conv2_w, b.se_w1, fold, C, hid);
+        if (conv2_deq) cudaFreeAsync(conv2_deq, s);
         pad_cols_kernel<float><<<(C * hp + 255) / 256, 256, 0, s>>>(b.se_w2, w2p, C, hid, hp);
         if ((rc = m0_check_launch("se_fold")) != M0_OK) break;
         if ((rc = make_weight(st, &st->blocks[i].se_fold, fold, hid16, K, hid16, s)) != M0_OK) break;
@@ -738,14 +831,14 @@ int tc_net_prepare(::m0_net* n, cudaStream_t s) {
     delete st;
     return rc;
   }
-  all->st[fmt] = st;
+  all->st[slot] = st;
   return M0_OK;
 }
 
 void tc_net_release(::m0_net* n) {
   TcStates* all = (TcStates*)n->tc;
   if (!all) return;
-  for (int f = 0; f < 2; ++f) {
+  for (int f = 0; f < 3; ++f) {
     TcState* st = all->st[f];
     if (!st) continue;
     for (void* p : st->allocs) cudaFree(p);
@@ -770,8 +863,8 @@ void tc_net_release(::m0_net* n) {
   n->tc = nullptr;
 }
 
-int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float* values, cudaStream_t s) {
-  TcState* st = ((TcStates*)n->tc)->st[nn_half_format()];
+int tc_net_forward(::m0_net* n, int slot, const float* planes, int B, float* logits, float* values, cudaStream_t s) {
+  TcState* st = ((TcStates*)n->tc)->st[slot];
   TRY(net_ws_reserve(n, B));
   TRY(tc_reserve(n, st, B));
   const m0_net_config& c = n->cfg;
@@ -782,6 +875,7 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
     // output maps of the bulk stores: their row extent is exactly this batch (rows of padding boards are clipped by TMA)
     TRY(make_map_out(&st->a1_out, st->a1, (uint64_t)M, C, false));
     TRY(make_map_out(&st->a2_out, st->a2, (uint64_t)M, C, false));
+    if (st->fp8) TRY(make_map_out(&st->a1_out8, st->a1, (uint64_t)M, C, false, false, true));
     TRY(make_map_out(&st->t1_out, n->t1, (uint64_t)M, C, true));
     TRY(make_map_out(&st->t2h_out, n->t2, (uint64_t)M, C, false));
     TRY(make_map_out(&st->t2f_out, n->t2, (uint64_t)M, C, true));
@@ -809,7 +903,7 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
     PROF("groupnorm_f32", nn_groupnorm_f32(n->t1, w.stem_gn_w, w.stem_gn_b, nullptr, 0, n->x, B, C, act, s));
   }
   // a1 = act(GN1(x)) of the first block; later blocks get it from the fused SE / residual kernel of their predecessor
-  if (c.blocks > 0) PROF("se_apply_gn", nn_se_apply_gn(nullptr, nullptr, n->x, w.blocks[0].gn1_w, w.blocks[0].gn1_b, st->a1, B, C, act, s));
+  if (c.blocks > 0) PROF("se_apply_gn", nn_se_apply_gn(nullptr, nullptr, n->x, w.blocks[0].gn1_w, w.blocks[0].gn1_b, st->a1, B, C, act, s, st->fp8));
   int att_seen = 0;
   bool heads_input_ready = false;   // a1 already holds half(x) of the final residual stream
   const int stride = c.infer_attention_stride > 1 ? c.infer_attention_stride : 1;
@@ -829,7 +923,7 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
       // conv1: a2 = act(GN2(conv1(a1))) and, for SE, the half-board sums of a2 that determine conv2's pooled output
       ConvFusion f1;
       f1.prims = c.se ? st->prims : nullptr;
-      PROF("conv1+gn", conv3x3(st, st->a1_conv, st->a1_convp, tb.conv1, B, C, nullptr, st->a2, act, s, b.gn2_w, b.gn2_b, nullptr, &f1));
+      PROF("conv1+gn", conv3x3(st, st->a1_conv, st->fp8 ? st->a1_convp8 : st->a1_convp, tb.conv1, B, C, nullptr, st->a2, act, s, b.gn2_w, b.gn2_b, nullptr, &f1));
       if (c.se) {
         // SE excitation before conv2 runs: hidden = act(fold * sums + b1), gate = sigmoid(W2 hidden + b2)  (resnet.py:61-64)
         // first layer split over K (60 k-blocks on only B/128 tiles otherwise), partial sums reduced with the bias + activation
@@ -856,12 +950,14 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
       se_done:;
       }
       // conv2 with the whole block tail in its epilogue: x += gate * conv2 ; a1 = act(GN1_{i+1}(x)) (or half(x) before attention)
+      // (fp8: the next block's conv1 operand is e4m3, half(x) for the qkv GEMM stays 16-bit)
       ConvFusion f2;
       f2.resid_x = n->x;
       f2.gate = c.se ? st->se_gate : nullptr;
       f2.x_map = &st->x_io;
-      PROF("conv2+se+res+gn", conv3x3(st, st->a2_conv, st->a2_convp, tb.conv2, B, C, nullptr, next_a, act, s, fuse_next ? w.blocks[i + 1].gn1_w : nullptr,
-                                      fuse_next ? w.blocks[i + 1].gn1_b : nullptr, nullptr, &f2, next_a ? &st->a1_out : nullptr));
+      const CUtensorMap* a1_map = !next_a ? nullptr : (st->fp8 && fuse_next) ? &st->a1_out8 : &st->a1_out;
+      PROF("conv2+se+res+gn", conv3x3(st, st->a2_conv, st->fp8 ? st->a2_convp8 : st->a2_convp, tb.conv2, B, C, nullptr, next_a, act, s, fuse_next ? w.blocks[i + 1].gn1_w : nullptr,
+                                      fuse_next ? w.blocks[i + 1].gn1_b : nullptr, nullptr, &f2, a1_map));
     } else {
       // conv1 with GN2 + activation fused into the epilogue: a2 = act(GN2(conv1(a1)))
       PROF("conv1+gn", conv3x3(st, st->a1_conv, st->a1_convp, tb.conv1, B, C, nullptr, st->a2, act, s, b.gn2_w, b.gn2_b, nullptr, nullptr, &st->a2_out));
@@ -900,10 +996,10 @@ int tc_net_forward(::m0_net* n, const float* planes, int B, float* logits, float
       if (fused_ln) {
         heads_input_ready = last && st->heads_tc;
         PROF("ln_res_gn", nn_ln_res_gn(n->t2, proj_half ? 1 : 0, n->x, b.att_ln_w, b.att_ln_b, last ? nullptr : w.blocks[i + 1].gn1_w,
-                                       last ? nullptr : w.blocks[i + 1].gn1_b, (last && !st->heads_tc) ? nullptr : st->a1, B, C, act, s));
+                                       last ? nullptr : w.blocks[i + 1].gn1_b, (last && !st->heads_tc) ? nullptr : st->a1, B, C, act, s, st->fp8 && !last));
       } else {
         PROF("layernorm_residual_f32", nn_layernorm_residual_f32(n->t2, n->x, b.att_ln_w, b.att_ln_b, n->x, M, C, s));
-        if (!last) PROF("se_apply_gn", nn_se_apply_gn(nullptr, nullptr, n->x, w.blocks[i + 1].gn1_w, w.blocks[i + 1].gn1_b, st->a1, B, C, act, s));
+        if (!last) PROF("se_apply_gn", nn_se_apply_gn(nullptr, nullptr, n->x, w.blocks[i + 1].gn1_w, w.blocks[i + 1].gn1_b, st->a1, B, C, act, s, st->fp8));
       }
     }
   }
@@ -1013,6 +1109,56 @@ extern "C" int m0_tc_conv(const uint16_t* d_act_bf16, const uint16_t* d_w_bf16, 
     return launch_gemm(&st, a, w, boards * 64, taps == 9 ? 1 : 0, taps, cin, 0, n, d_out_f32, nullptr, n, 0, nullptr, ACT_NONE, 1.0f, s);
   };
   const int rc = w_pad ? run(w_pad, kw) : run(d_w_bf16, taps * cin);
+  if (w_pad) cudaFreeAsync(w_pad, s);
+  return rc;
+}
+
+// Stand-alone e4m3 3x3 convolution on the CTA-pair kernel (kernel-alone tests of precision fp8):
+//   out[b*64+sq][n] = w_scale[n] * conv3x3(act e4m3 [boards][8][8][cin], w e4m3 [n][9*cin])
+extern "C" int m0_tc_conv_fp8(const uint8_t* d_act_e4m3, const uint8_t* d_w_e4m3, const float* d_w_scale, int boards, int cin, int n, float* d_out_f32,
+                              void* stream) {
+  if (!d_act_e4m3 || !d_w_e4m3 || !d_w_scale || !d_out_f32 || boards <= 0 || (boards & 1) || cin <= 0 || cin % 32 != 0 || cin > 512 ||
+      n % 32 != 0 || n < 64 || n > 320 || !pair_ok(n)) {
+    m0_set_error("m0_tc_conv_fp8: invalid argument (boards even, cin %% 32 == 0, cin <= 512, n %% 32 == 0, 64 <= n <= 320, CTA-pair kernel on)");
+    return M0_ERR_ARG;
+  }
+  static TcState st;
+  static int st_dev = -1;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev != st_dev) {   // shared-memory grants are per device
+    for (size_t& v : st.smem_pair) v = 0;
+    st_dev = dev;
+  }
+  cudaDeviceGetAttribute(&st.sm_count, cudaDevAttrMultiProcessorCount, dev);
+  cudaDeviceGetAttribute(&st.max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+  const cudaStream_t s = (cudaStream_t)stream;
+  // every tap padded to whole 128-channel k-blocks (the layout make_weight_fp8 gives the network's weights), stream-ordered copy
+  const int cin_pad = (cin + 127) / 128 * 128, kw = 9 * cin_pad;
+  const void* wp = d_w_e4m3;
+  void* w_pad = nullptr;
+  if (cin_pad != cin) {
+    M0_CUDA_TRY(cudaMallocAsync(&w_pad, (size_t)n * kw, s));
+    pad_cols_kernel<uint8_t><<<(n * kw + 255) / 256, 256, 0, s>>>(d_w_e4m3, (uint8_t*)w_pad, n * 9, cin, cin_pad);
+    const int rc = m0_check_launch("pad_taps");
+    if (rc != M0_OK) { cudaFreeAsync(w_pad, s); return rc; }
+    wp = w_pad;
+  }
+  auto run = [&]() -> int {
+    TcWeight w;
+    w.w = (__nv_bfloat16*)wp;
+    w.n = w.n_launch = n;
+    w.k = kw;
+    w.pair = true;
+    w.fp8 = true;
+    w.dq = d_w_scale;
+    TRY(make_map_2d(&w.map_pair, wp, (uint64_t)n, (uint64_t)kw, (uint32_t)(n / 4), true));
+    CUtensorMap a, om;
+    TRY(make_map_nhwc(&a, d_act_e4m3, (uint64_t)boards, (uint64_t)cin, 10, true));
+    TRY(make_map_out(&om, d_out_f32, (uint64_t)boards * 64, (uint64_t)n, true));
+    return launch_conv_pair(&st, a, w, boards, cin, d_out_f32, nullptr, n, ACT_NONE, s, nullptr, nullptr, nullptr, nullptr, 1, 1, &om);
+  };
+  const int rc = run();
   if (w_pad) cudaFreeAsync(w_pad, s);
   return rc;
 }

@@ -28,8 +28,15 @@
 //                  double buffered per warp), then the next block's GroupNorm + activation -> out_half; conv1 additionally writes
 //                  the half-board sums from which the SE gate of conv2 is computed ahead of conv2 (ConvPairParams::prims)
 // A plain GEMM mode (conv = 0, K <= 320) keeps the A tile of a group of boards resident across its (slice, half) work items.
+//
+// F8 (3x3 mode only): the operands are e4m3 and a k-block is 128 channels -- still one 128-byte row, so the A box, CP_A_SLOT, the
+// swizzle and the dx-shifted descriptors are the 16-bit ones byte for byte.  Each k-block issues 4 x kind::f8f6f4 MMAs of K = 32
+// (32 bytes each, like the 4 x K = 16 of the 16-bit kernel).  The epilogue first multiplies the accumulator by ConvPairParams::w_dq
+// (the inverse of the power-of-two weight scale, exact), and writes its GroupNorm'ed output as e4m3 (rounded in registers first, so
+// that the SE half-board sums describe exactly what conv2 reads).
 #pragma once
 #include "tc_gemm.cuh"
+#include <cuda_fp8.h>
 
 namespace m0 {
 namespace tc {
@@ -65,6 +72,7 @@ struct ConvPairParams {
   float* resid_x;
   const float* gate;
   __nv_bfloat16* prims;
+  const float* w_dq;   // F8: per output channel factor applied to the accumulator before anything else (1 / weight scale)
 };
 
 static constexpr int CP_EPI_WARP0 = 4;    // warpgroup 0: TMA producer, MMA issuer, two idle warps
@@ -119,6 +127,27 @@ __device__ __forceinline__ void umma_pair(uint32_t tmem_d, uint64_t desc_a, uint
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// the same with e4m3 operands (the instruction descriptor's A / B format 0 = E4M3 under kind::f8f6f4, K = 32 per instruction)
+__device__ __forceinline__ void umma_pair_f8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t"
+      "}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// four floats -> four e4m3 bytes (round to nearest even, saturating to +-448), the first in the lowest byte
+__device__ __forceinline__ uint32_t pack_e4m3x4(float a, float b, float c, float d) {
+  const uint32_t lo = __nv_cvt_float2_to_fp8x2(make_float2(a, b), __NV_SATFINITE, __NV_E4M3);
+  const uint32_t hi = __nv_cvt_float2_to_fp8x2(make_float2(c, d), __NV_SATFINITE, __NV_E4M3);
+  return lo | (hi << 16);
+}
+// x rounded to the nearest e4m3 value (saturating), as a float
+__device__ __forceinline__ float round_e4m3(float x) {
+  return __half2float(__half(__nv_cvt_fp8_to_halfraw(__nv_cvt_float_to_fp8(x, __NV_SATFINITE, __NV_E4M3), __NV_E4M3)));
+}
 __device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
                "h"(cta_mask)
@@ -151,7 +180,7 @@ __device__ __forceinline__ uint64_t make_smem_desc_sbo(uint32_t smem_addr, uint3
 // FUSE compiles the extra epilogues in (kept out of the plain kernels: code size costs instruction fetch):
 //   0 = plain / GroupNorm, 1 = + half-board sums (conv1 of a fused block), 2 = SE gate + residual + next GroupNorm (conv2; 8 KB of
 //   tiles per epilogue warp, which leaves room for 3 pipeline stages instead of 4)
-template <int NCH, int FUSE>
+template <int NCH, int FUSE, bool F8 = false>
 __global__ void __launch_bounds__(CP_THREADS, 1)
 conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w, const __grid_constant__ CUtensorMap tma_out,
                  const __grid_constant__ CUtensorMap tma_x, const ConvPairParams p) {
@@ -187,6 +216,7 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   const int num_clusters = gridDim.x >> 1;
   const int cluster_id = blockIdx.x >> 1;
   const int steps = p.conv ? p.kb_per_tap * 3 : p.kb_per_tap;
+  constexpr int KE = F8 ? 128 : BK;   // operand elements per k-block (one 128-byte row either way)
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tma_a);
@@ -246,10 +276,10 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
                 if (rank == 0) mbar_expect_tx(&full_bar[stage], (uint32_t)(2 * stage_bytes));
                 const uint32_t bar = lead_full + (uint32_t)stage * 8u;
                 uint8_t* a_dst = smem + (size_t)stage * stage_bytes;
-                tma_load_4d_pair(a_dst, &tma_a, bar, kc * BK, -1, dyi - 1, board0);
+                tma_load_4d_pair(a_dst, &tma_a, bar, kc * KE, -1, dyi - 1, board0);
 #pragma unroll
                 for (int dxi = 0; dxi < 3; ++dxi)
-                  tma_load_2d_pair(a_dst + CP_A_SLOT + dxi * wq_bytes, &tma_w, bar, ((dyi * 3 + dxi) * p.kb_per_tap + kc) * BK, w_row);
+                  tma_load_2d_pair(a_dst + CP_A_SLOT + dxi * wq_bytes, &tma_w, bar, ((dyi * 3 + dxi) * p.kb_per_tap + kc) * KE, w_row);
                 if (++stage == p.stages) { stage = 0; phase ^= 1; }
               }
             }
@@ -267,7 +297,7 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   } else if (warp == 1) {
     // ===== MMA issuer (leader CTA) =====
     if (rank == 0) {
-      const uint32_t idesc = make_idesc_bf16(256, nh, p.fp16);
+      const uint32_t idesc = make_idesc_bf16(256, nh, F8 ? 1 : p.fp16);   // F8: format 0 = E4M3 (1 would be E5M2)
       const uint32_t smem_base = smem_u32(smem);
       int stage = 0;
       uint32_t phase = 0, unit = 0;
@@ -293,8 +323,13 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
                 for (int dxi = 0; dxi < 3; ++dxi) {
                   const uint64_t adesc = make_smem_desc_sbo(a_addr + dxi * 128, 1280);
                   const uint64_t bdesc = make_smem_desc_sbo(a_addr + CP_A_SLOT + dxi * wq_bytes, 1024);
+                  if constexpr (F8) {   // 4 x K = 32 e4m3: 32 bytes of K per instruction, as 4 x K = 16 at 16 bits
 #pragma unroll
-                  for (int k = 0; k < BK / 16; ++k) umma_pair(d, adesc + 2 * k, bdesc + 2 * k, idesc, (step > 0 || dxi > 0 || k > 0) ? 1u : 0u);
+                    for (int k = 0; k < 4; ++k) umma_pair_f8(d, adesc + 2 * k, bdesc + 2 * k, idesc, (step > 0 || dxi > 0 || k > 0) ? 1u : 0u);
+                  } else {
+#pragma unroll
+                    for (int k = 0; k < BK / 16; ++k) umma_pair(d, adesc + 2 * k, bdesc + 2 * k, idesc, (step > 0 || dxi > 0 || k > 0) ? 1u : 0u);
+                  }
                 }
               } else {
                 const uint64_t adesc = make_smem_desc_sbo(a_tile + (uint32_t)step * A_TILE_BYTES, 1024);
@@ -334,6 +369,7 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     const bool fused_gn = p.gn_gamma != nullptr;
     const bool resid = FUSE == 2 && p.resid_x != nullptr;
     const bool want_prims = FUSE == 1 && p.prims != nullptr;
+    const bool out8 = F8 && fused_gn;   // the GroupNorm'ed output is the e4m3 operand of the next convolution
     const int epi_tid = ((warp - CP_EPI_WARP0) << 5) | lane;
     const uint32_t lead_empty = mapa_u32(smem_u32(tmem_empty_bar), 0);
     const int nchunks = nh >> 4;
@@ -382,6 +418,22 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(lead_empty + buf * 8u);
+        if constexpr (F8) {
+          // undo the weight scale first: GroupNorm statistics, SE sums and the residual add all see the true convolution
+#pragma unroll
+          for (int k = 0; k < NCH; ++k) {
+            const int ci = cset + CP_CSETS * k;
+            if (ci >= nchunks) break;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+              const float4 d4 = __ldg(reinterpret_cast<const float4*>(p.w_dq + cbase + ci * 16 + 4 * q));
+              r[k][4 * q + 0] = __float_as_uint(__uint_as_float(r[k][4 * q + 0]) * d4.x);
+              r[k][4 * q + 1] = __float_as_uint(__uint_as_float(r[k][4 * q + 1]) * d4.y);
+              r[k][4 * q + 2] = __float_as_uint(__uint_as_float(r[k][4 * q + 2]) * d4.z);
+              r[k][4 * q + 3] = __float_as_uint(__uint_as_float(r[k][4 * q + 3]) * d4.w);
+            }
+          }
+        }
         if (resid) {
           // x_new = x + gate * conv  (SE excitation + residual add, resnet.py:68-80): the x tile arrives by TMA (64-byte swizzle: 16-byte
           // chunk c of row i sits at c ^ ((i >> 1) & 3)), x_new leaves the same way; nothing here touches global memory directly
@@ -474,6 +526,10 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 #pragma unroll
               for (int j = 0; j < 16; ++j) y[j] = fmaxf(y[j], 0.0f);
             }
+            if constexpr (F8) {
+#pragma unroll
+              for (int j = 0; j < 16; ++j) y[j] = round_e4m3(y[j]);
+            }
 #pragma unroll
             for (int j = 0; j < 16; ++j) r[k][j] = __float_as_uint(y[j]);
           }
@@ -496,7 +552,18 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
               a1 += __shfl_xor_sync(0xFFFFFFFFu, a1, 1);
               if (!(lane & 1)) p.pool_part[(size_t)(row0 >> 5) * p.N + col + (b4 ? 8 : 0) + (b3 ? 4 : 0) + (b2 ? 2 : 0) + (b1 ? 1 : 0)] = a1;
             }
-            if (p.out_half) {
+            if (p.out_half && out8) {
+              uint8_t* tile = xout + (nstore & 1) * (FUSE == 2 ? 2048 : 1024);   // 32 rows x 16 e4m3 bytes
+              if (lane == 0) tma_store_wait_read<1>();
+              __syncwarp();
+              const float* f = reinterpret_cast<const float*>(r[k]);
+              *reinterpret_cast<uint4*>(tile + lane * 16) = make_uint4(pack_e4m3x4(f[0], f[1], f[2], f[3]), pack_e4m3x4(f[4], f[5], f[6], f[7]),
+                                                                      pack_e4m3x4(f[8], f[9], f[10], f[11]), pack_e4m3x4(f[12], f[13], f[14], f[15]));
+              fence_proxy_async();
+              __syncwarp();
+              if (lane == 0) { tma_store_2d(&tma_out, tile, col, row0); tma_store_commit(); }
+              ++nstore;
+            } else if (p.out_half) {
               uint8_t* tile = xout + (nstore & 1) * (FUSE == 2 ? 2048 : 1024);   // two tiles alternate
               if (lane == 0) tma_store_wait_read<1>();                                 // the store that last read this tile is done
               __syncwarp();
@@ -585,7 +652,21 @@ conv_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
               }
             }
           }
-          if (p.out_half) {
+          if (p.out_half && out8) {
+            const int hq = lane & 1;
+#pragma unroll
+            for (int i = 0; i < 2; ++i) {
+              const int rr = (lane >> 1) + 16 * i;
+              const int m = row0 + rr;
+              if (m < M) {
+                const int sw2 = (rr >> 1) & 3;
+                float4 lo = *reinterpret_cast<const float4*>(stg + rr * 16 + (((2 * hq) ^ sw2) << 2));
+                float4 hi = *reinterpret_cast<const float4*>(stg + rr * 16 + (((2 * hq + 1) ^ sw2) << 2));
+                *reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(p.out_half) + (size_t)m * p.ldc + col + 8 * hq) =
+                    make_uint2(pack_e4m3x4(lo.x, lo.y, lo.z, lo.w), pack_e4m3x4(hi.x, hi.y, hi.z, hi.w));
+              }
+            }
+          } else if (p.out_half) {
             const int hq = lane & 1;
 #pragma unroll
             for (int i = 0; i < 2; ++i) {

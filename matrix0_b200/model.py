@@ -4,7 +4,8 @@
 ``load_state_dict(sd, strict=False)`` with the reference's key names, ``eval()``, ``to()``,
 ``count_parameters()``, ``cfg.policy_size``) but holds its parameters as plain CUDA tensors in the
 layouts the kernels consume and runs the forward through the C ABI (``m0_net_forward``): fp32 SIMT
-kernels (``precision="fp32"``) or the bf16 tcgen05 pipeline (``precision="bf16"``).  There is no
+kernels (``precision="fp32"``) or the tcgen05 pipeline with 16-bit operands (``"fp16"``, ``"bf16"``) or with e4m3
+operands for the residual tower's 3x3 convolutions (``"fp8"``, opt-in; DESIGN.md section 4).  There is no
 ``torch.nn`` forward and no CPU path.  Training-only members of the reference module (losses, SSRL /
 WDL / aux heads, ``to_coreml``) are out of scope (SURVEY.md section 2.1 #3).
 """
@@ -23,6 +24,7 @@ from ._native import c_float, c_int, c_void_p
 MAX_BLOCKS = 64
 MAX_SSL = 8
 ACT = {"none": 0, "relu": 1, "silu": 2, "leaky_relu": 3}
+PRECISIONS = {"fp32": 0, "bf16": 1, "fp16": 2, "fp8": 3}   # m0_net_forward's precision argument
 SSL_CHANNELS = {"piece": 13, "threat": 1, "pin": 1, "fork": 1, "control": 3, "pawn_structure": 8, "king_safety": 3}
 SSL_ORDER = ["piece", "threat", "pin", "fork", "control", "pawn_structure", "king_safety"]  # ModuleDict insertion order, resnet.py:366-433
 
@@ -471,15 +473,18 @@ class PolicyValueNet:
         B = planes.shape[0]
         logits = torch.empty((B, self.cfg.policy_size), dtype=torch.float32, device=planes.device)
         values = torch.empty((B,), dtype=torch.float32, device=planes.device)
-        prec = {"fp32": 0, "bf16": 1, "fp16": 2}[precision or self.precision]
+        prec = PRECISIONS[precision or self.precision]
         if B == 0:
             return logits, values
         if B > getattr(self, "_max_batch", 0):     # the library grows its workspaces: captured graphs of smaller batches are stale
             self._max_batch = B
             self._ws_epoch = getattr(self, "_ws_epoch", 0) + 1
         with torch.cuda.device(planes.device):
-            _native.check(_native.lib().m0_net_forward(self._handle, planes.data_ptr(), B, logits.data_ptr(), values.data_ptr(), prec,
-                                                       _native.current_stream()), "m0_net_forward")
+            rc = _native.lib().m0_net_forward(self._handle, planes.data_ptr(), B, logits.data_ptr(), values.data_ptr(), prec,
+                                              _native.current_stream())
+        if rc == _native.M0_ERR_ARG and prec == PRECISIONS["fp8"]:   # a configuration the fp8 pipeline does not cover
+            raise ValueError(f"precision='fp8': {_native.load_library().m0_last_error().decode()}")
+        _native.check(rc, "m0_net_forward")
         return logits, values
 
     def capture_forward(self, planes, precision: Optional[str] = None):
