@@ -166,6 +166,25 @@ int m0_search_expand_backup_multi(m0_engine* e, int g0, int g1, const float* d_l
  * when the evaluator changes.  Counter 12 counts the roots expanded from the store. */
 int m0_search_reuse_enable(m0_engine* e, int slots, float* d_miss_planes, int32_t* d_miss_count);
 int m0_search_reuse_clear(m0_engine* e, void* stream);
+/* ---- Gumbel AlphaZero search (DESIGN.md §9): one leaf per game and simulation step, sequential halving over the
+ * max_considered_actions moves of largest g + logit at the root, policy target softmax(logits + sigma(completed Q)).
+ * Per move: m0_trees_clear -> m0_search_begin -> evaluator -> m0_gumbel_expand_backup (the root)
+ *           -> num_simulations x [m0_gumbel_select -> evaluator -> m0_gumbel_expand_backup] -> m0_gumbel_result.
+ * m0_gumbel_configure allocates the per-node logits and values (not with the root-evaluation store: M0_ERR_STATE);
+ * num_simulations 1..4096, max_considered_actions 1..256, c_visit >= 0, c_scale > 0. */
+int m0_gumbel_configure(m0_engine* e, int num_simulations, int max_considered_actions, double c_visit, double c_scale);
+/* d_draws float64[G][256]: the Gumbel(0, 1) draw of each legal move (generation order) of the roots expanded next; NULL = device
+ * generator keyed by (seed, game, expansion call, move slot).  The buffer must stay alive. */
+int m0_gumbel_set_draws(m0_engine* e, const double* d_draws);
+/* one leaf per game into row g of d_planes float32[G][19][8][8]; terminal leaves are backed up at once, and they, finished and idle
+ * games write no row (m0_search_pending reports 0 for them) */
+int m0_gumbel_select(m0_engine* e, float* d_planes, void* stream);
+/* expansion from row g of d_logits float32[G][stride >= 4672] / d_values float32[G] and backup, for every pending game */
+int m0_gumbel_expand_backup(m0_engine* e, const float* d_logits, int logits_stride, const float* d_values, void* stream);
+/* d_move uint16[G] (0xFFFF: nothing searched), d_value float64[G] = W(root) / N(root); optional (NULL): d_pi float32[G][4672], and
+ * per root child d_visits int32[G][256], d_q float64[G][256] (-W / N, 0 unvisited), d_pi_children float64[G][256], d_count int32[G] */
+int m0_gumbel_result(m0_engine* e, uint16_t* d_move, float* d_pi, double* d_value, int32_t* d_visits, double* d_q, double* d_pi_children,
+                     int32_t* d_count, void* stream);
 int m0_engine_counters(m0_engine* e, unsigned long long* h_out16); /* host buffer; synchronises */
 int m0_engine_status(m0_engine* e, int32_t* d_status_out, int32_t* d_node_count_out, void* stream);
 
@@ -190,6 +209,8 @@ typedef struct m0_finished_game {
 int m0_selfplay_configure(m0_engine* e, const m0_selfplay_config* cfg, void* stream);
 int m0_selfplay_start(m0_engine* e, void* stream);                      /* new game in every slot, internal.py:326-379 */
 int m0_selfplay_advance(m0_engine* e, uint16_t* d_out_move, void* stream); /* one ply: sample, resign, push, finish/restart */
+/* the same ply after m0_gumbel_result: plays the search's move; its value and the entropy of its policy target feed the resign rule */
+int m0_selfplay_advance_gumbel(m0_engine* e, uint16_t* d_out_move, void* stream);
 /* `games` argument of selfplay_worker (internal.py:94, :326): at most `games` more games are started (initial start + restarts), idle
  * slots afterwards, so every started game is played to its end; < 0 = unlimited (default) */
 int m0_selfplay_set_start_budget(m0_engine* e, long long games, void* stream);

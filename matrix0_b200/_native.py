@@ -60,6 +60,12 @@ SIGNATURES = {
     "m0_search_expand_backup_multi": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p]),
     "m0_search_reuse_enable": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "m0_search_reuse_clear": (c_int, [c_void_p, c_void_p]),
+    "m0_gumbel_configure": (c_int, [c_void_p, c_int, c_int, c_double, c_double]),
+    "m0_gumbel_set_draws": (c_int, [c_void_p, c_void_p]),
+    "m0_gumbel_select": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "m0_gumbel_expand_backup": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "m0_gumbel_result": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "m0_selfplay_advance_gumbel": (c_int, [c_void_p, c_void_p, c_void_p]),
     "m0_engine_counters": (c_int, [c_void_p, c_void_p]),
     "m0_engine_status": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "m0_search_select_var": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p]),

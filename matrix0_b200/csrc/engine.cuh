@@ -119,6 +119,20 @@ struct EngineView {
   int* rc_miss_count;     // [1] caller's counter: rows written to rc_miss_planes by the last search_begin
 };
 
+// Gumbel AlphaZero search (gumbel_kernels.cu; DESIGN.md §9).  Allocated by m0_gumbel_configure only, so the other search modes keep
+// their memory.  Node statistics are node_n / node_w of EngineView, from the view of the side to move at the node.
+struct GumbelView {
+  int n, m;               // simulations per move, max_considered_actions
+  double c_visit, c_scale;
+  float* logit;           // [G][max_nodes] the parent's network logit of the move that leads to the node (fp32, read as float64)
+  float* r;               // [G][max_nodes] the node's network value, clipped to [-1, 1]
+  double* draw;           // [G][256] Gumbel draws of the current root's moves, in child order
+  const double* user_draw;// [G][256] caller-supplied draws, or NULL for the counter-based device generator
+  int* choice;            // [G] root child played by the last result, -1 = none
+  double* value;          // [G] search value W(root) / N(root) of the last result
+  double* entropy;        // [G] entropy of the last result's policy target (the resign rule's input)
+};
+
 static constexpr u32 MOVE_NONE = 0xFFFFu;
 
 // ---- transposition table -----------------------------------------------------------------------

@@ -21,6 +21,12 @@ __global__ void multi_scan_kernel(EngineView E);
 __global__ void multi_encode_kernel(EngineView E, int g0, int g1, int row0, int mode, float* planes, int row_cap);
 __global__ void search_expand_backup_multi_kernel(EngineView E, int g0, int g1, const float* logits, int logits_stride, const float* values,
                                                   int row0, int per_sample, int row_cap);
+// kernels (gumbel_kernels.cu)
+__global__ void gumbel_select_kernel(EngineView E, GumbelView GB, float* planes);
+__global__ void gumbel_expand_backup_kernel(EngineView E, GumbelView GB, const float* logits, int logits_stride, const float* values,
+                                            unsigned long long rng_step);
+__global__ void gumbel_result_kernel(EngineView E, GumbelView GB, u16* out_move, float* out_pi, double* out_value, int* out_visits,
+                                     double* out_q, double* out_pi_children, int* out_count);
 }  // namespace m0
 
 using namespace m0;
@@ -102,6 +108,8 @@ int m0_engine_create(int device, int max_games, int max_nodes, int tt_capacity, 
   e->rng_step = 0;
   memset(&e->v, 0, sizeof(e->v));
   memset(&e->sp, 0, sizeof(e->sp));
+  memset(&e->gb, 0, sizeof(e->gb));
+  e->gb_step = 0;
   e->d_sp_params = nullptr;
   e->sp_step = 0;
   e->finished_read = 0;
@@ -353,6 +361,7 @@ int m0_search_expand_backup_multi(m0_engine* e, int g0, int g1, const float* d_l
 // the outputs of the network that produced them: m0_search_reuse_clear must be called when the evaluator changes.
 int m0_search_reuse_enable(m0_engine* e, int slots, float* d_miss_planes, int32_t* d_miss_count) {
   if (!e || slots <= 0 || slots > REUSE_MAX_SLOTS || !d_miss_planes || !d_miss_count) { m0_set_error("m0_search_reuse_enable: invalid argument"); return M0_ERR_ARG; }
+  if (e->gb.logit) { m0_set_error("m0_search_reuse_enable: the engine is configured for the Gumbel search"); return M0_ERR_STATE; }
   if (e->v.rc_slots && e->v.rc_slots != slots) { m0_set_error("m0_search_reuse_enable: already enabled with %d slots", e->v.rc_slots); return M0_ERR_STATE; }
   EngineView& v = e->v;
   if (!v.rc_slots) {
@@ -375,6 +384,74 @@ int m0_search_reuse_enable(m0_engine* e, int slots, float* d_miss_planes, int32_
 int m0_search_reuse_clear(m0_engine* e, void* stream) {
   if (!e || !e->v.rc_slots) { m0_set_error("m0_search_reuse_clear: invalid argument (store not enabled)"); return M0_ERR_ARG; }
   return m0_check_cuda(cudaMemsetAsync(e->v.rc_fill, 0, sizeof(int) * e->v.G, (cudaStream_t)stream), "m0_search_reuse_clear");
+}
+
+// ---- Gumbel AlphaZero search (gumbel_kernels.cu, DESIGN.md §9) ----------------------------------------------------------------------
+// Allocates the per-node logits and values and the per-game draws on the first call; later calls change the parameters.
+// num_simulations 1..4096, max_considered_actions 1..256, c_visit >= 0, c_scale > 0 (both finite).
+int m0_gumbel_configure(m0_engine* e, int num_simulations, int max_considered_actions, double c_visit, double c_scale) {
+  if (!e || num_simulations < 1 || num_simulations > 4096 || max_considered_actions < 1 || max_considered_actions > MAX_MOVES ||
+      !(c_visit >= 0.0) || !(c_scale > 0.0) || !isfinite(c_visit) || !isfinite(c_scale)) {
+    m0_set_error("m0_gumbel_configure: invalid argument");
+    return M0_ERR_ARG;
+  }
+  if (e->v.rc_slots) { m0_set_error("m0_gumbel_configure: the root-evaluation store is enabled (the Gumbel search evaluates its roots)"); return M0_ERR_STATE; }
+  GumbelView& gb = e->gb;
+  if (!gb.logit) {
+    m0::DeviceGuard device_guard(e->device);
+    M0_CUDA_TRY(device_guard.err);
+    const size_t G = e->v.G, N = G * (size_t)e->v.max_nodes;
+    TRY(dev_alloc(e, &gb.logit, N, false));
+    TRY(dev_alloc(e, &gb.r, N, false));
+    TRY(dev_alloc(e, &gb.draw, G * MAX_MOVES));
+    TRY(dev_alloc(e, &gb.choice, G));
+    TRY(dev_alloc(e, &gb.value, G));
+    TRY(dev_alloc(e, &gb.entropy, G));
+  }
+  gb.n = num_simulations;
+  gb.m = max_considered_actions;
+  gb.c_visit = c_visit;
+  gb.c_scale = c_scale;
+  return M0_OK;
+}
+
+// d_draws float64[G][256]: the Gumbel(0, 1) draw of every legal move (python-chess generation order) for the roots the following
+// expansions create; NULL returns to the counter-based device generator.  The buffer must stay alive.
+int m0_gumbel_set_draws(m0_engine* e, const double* d_draws) {
+  if (!e || !e->gb.logit) { m0_set_error("m0_gumbel_set_draws: call m0_gumbel_configure first"); return M0_ERR_STATE; }
+  e->gb.user_draw = d_draws;
+  return M0_OK;
+}
+
+// One simulation step: one leaf per game, its planes in row g of d_planes float32[G][19][8][8].  Games whose leaf is terminal (backed
+// up here), that have run their simulations or that hold no search write no row; m0_search_pending reports 0 for them.
+int m0_gumbel_select(m0_engine* e, float* d_planes, void* stream) {
+  if (!e || !d_planes) { m0_set_error("m0_gumbel_select: invalid argument"); return M0_ERR_ARG; }
+  if (!e->gb.logit) { m0_set_error("m0_gumbel_select: call m0_gumbel_configure first"); return M0_ERR_STATE; }
+  gumbel_select_kernel<<<tree_blocks(e), TREE_WARPS * 32, 0, (cudaStream_t)stream>>>(e->v, e->gb, d_planes);
+  return m0_check_launch("m0_gumbel_select");
+}
+
+// Expansion + backup of every pending game from row g of d_logits float32[G][stride] / d_values float32[G].  After m0_trees_clear and
+// m0_search_begin this is the root expansion (children, r, Gumbel draws, N = 1, W = r); after m0_gumbel_select, the leaves'.
+int m0_gumbel_expand_backup(m0_engine* e, const float* d_logits, int logits_stride, const float* d_values, void* stream) {
+  if (!e || !d_logits || !d_values || logits_stride < POLICY_SIZE) { m0_set_error("m0_gumbel_expand_backup: invalid argument"); return M0_ERR_ARG; }
+  if (!e->gb.logit) { m0_set_error("m0_gumbel_expand_backup: call m0_gumbel_configure first"); return M0_ERR_STATE; }
+  e->gb_step += 1;
+  gumbel_expand_backup_kernel<<<tree_blocks(e), TREE_WARPS * 32, 0, (cudaStream_t)stream>>>(e->v, e->gb, d_logits, logits_stride, d_values, e->gb_step);
+  return m0_check_launch("m0_gumbel_expand_backup");
+}
+
+// After the simulations: d_move uint16[G] (0xFFFF: no search), d_value float64[G] = W(root) / N(root); optional: d_pi float32[G][4672]
+// (the policy target), per root child d_visits int32[G][256], d_q float64[G][256] (-W / N, 0 when unvisited), d_pi_children
+// float64[G][256], d_count int32[G].  Also keeps the move, value and target entropy for m0_selfplay_advance_gumbel.
+int m0_gumbel_result(m0_engine* e, uint16_t* d_move, float* d_pi, double* d_value, int32_t* d_visits, double* d_q, double* d_pi_children,
+                     int32_t* d_count, void* stream) {
+  if (!e || !d_move || !d_value) { m0_set_error("m0_gumbel_result: invalid argument"); return M0_ERR_ARG; }
+  if (!e->gb.logit) { m0_set_error("m0_gumbel_result: call m0_gumbel_configure first"); return M0_ERR_STATE; }
+  gumbel_result_kernel<<<tree_blocks(e), TREE_WARPS * 32, 0, (cudaStream_t)stream>>>(e->v, e->gb, d_move, d_pi, d_value, d_visits, d_q,
+                                                                                       d_pi_children, d_count);
+  return m0_check_launch("m0_gumbel_result");
 }
 
 // Engine counters (uint64[16], see engine.cuh CTR_*) and sticky per-game status bits (int32[G])

@@ -35,6 +35,8 @@ struct m0_engine {
   m0::SelfPlayParams* d_sp_params;
   unsigned long long sp_step;
   unsigned finished_read;
+  m0::GumbelView gb;           // Gumbel search state (gumbel_kernels.cu); gb.logit == NULL until m0_gumbel_configure
+  unsigned long long gb_step;  // expansion calls so far: keys the device Gumbel draws
 };
 
 static constexpr int TREE_WARPS = 4;

@@ -4,7 +4,8 @@
 
 namespace m0 {
 __global__ void selfplay_start_kernel(EngineView E, SelfPlayState S, int all, unsigned long long step);
-__global__ void selfplay_advance_kernel(EngineView E, SelfPlayState S, unsigned long long step, u16* out_move);
+template <bool GUMBEL>
+__global__ void selfplay_advance_kernel(EngineView E, SelfPlayState S, unsigned long long step, u16* out_move, GumbelView GB);
 __global__ void clear_trees_kernel(EngineView E);
 }  // namespace m0
 
@@ -144,8 +145,17 @@ int m0_selfplay_active_games(m0_engine* e, int* h_out, void* stream) {
 int m0_selfplay_advance(m0_engine* e, uint16_t* d_out_move, void* stream) {
   if (!e || !e->sp.ply) { m0_set_error("m0_selfplay_advance: self-play not configured"); return M0_ERR_STATE; }
   e->sp_step += 1;
-  selfplay_advance_kernel<<<(e->v.G + 3) / 4, 128, 0, (cudaStream_t)stream>>>(e->v, e->sp, e->sp_step, d_out_move);
+  selfplay_advance_kernel<false><<<(e->v.G + 3) / 4, 128, 0, (cudaStream_t)stream>>>(e->v, e->sp, e->sp_step, d_out_move, GumbelView{});
   return m0_check_launch("m0_selfplay_advance");
+}
+
+// The same ply after a Gumbel search (m0_gumbel_result): the move is the search's choice, the search value and the entropy of the
+// policy target feed the resign rule and avg_policy_entropy; temperature and visit sampling do not apply.
+int m0_selfplay_advance_gumbel(m0_engine* e, uint16_t* d_out_move, void* stream) {
+  if (!e || !e->sp.ply || !e->gb.logit) { m0_set_error("m0_selfplay_advance_gumbel: self-play or the Gumbel search not configured"); return M0_ERR_STATE; }
+  e->sp_step += 1;
+  selfplay_advance_kernel<true><<<(e->v.G + 3) / 4, 128, 0, (cudaStream_t)stream>>>(e->v, e->sp, e->sp_step, d_out_move, e->gb);
+  return m0_check_launch("m0_selfplay_advance_gumbel");
 }
 
 // Drop all trees (nodes + transposition tables), keep positions and histories: what constructing a fresh

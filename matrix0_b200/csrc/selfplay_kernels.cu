@@ -234,9 +234,12 @@ __device__ void settle_game(const EngineView& E, const SelfPlayState& S, int g, 
   }
 }
 
-// one ply for every game: sample the move from the finished search, resign rule, push, settle
+// one ply for every game: sample the move from the finished search, resign rule, push, settle.
+// GUMBEL: the move, the search value and the policy entropy come from gumbel_result_kernel (GB) instead of the visit counts; the
+// temperature schedule and the visit sampling do not apply (the Gumbel draw is the sampling).
+template <bool GUMBEL>
 __global__ void __launch_bounds__(SP_WARPS * 32)
-selfplay_advance_kernel(EngineView E, SelfPlayState S, unsigned long long step, u16* __restrict__ out_move) {
+selfplay_advance_kernel(EngineView E, SelfPlayState S, unsigned long long step, u16* __restrict__ out_move, GumbelView GB) {
   __shared__ u16 s_moves[SP_WARPS][MAX_MOVES];
   __shared__ float s_w[SP_WARPS][MAX_MOVES];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -253,83 +256,94 @@ selfplay_advance_kernel(EngineView E, SelfPlayState S, unsigned long long step, 
   }
   const int fc = E.node_first[nb + root];
   const int nc = fc < 0 ? 0 : E.node_nchild[nb + root];
-  // temperature schedule by full-move number (internal.py:386-394)
-  double temperature = P.temperature_end;
-  if (P.temperature_moves > 0) {
-    int mn = pos_fullmove(pos);
-    double t = (double)(mn < P.temperature_moves ? mn : P.temperature_moves) / (double)P.temperature_moves;
-    temperature = P.temperature_start + (P.temperature_end - P.temperature_start) * t;
-  }
-  if (P.argmax_after_plies >= 0) temperature = S.ply[g] < P.argmax_after_plies ? P.temperature_start : 0.0;   // arena.py:75-91
-  // visit counts -> move (internal.py:690-735)
-  long long total = 0;
-  int best_n = -1, best_j = 0;
-  for (int j = lane; j < nc; j += 32) {
-    int n = E.node_n[nb + fc + j];
-    total += n;
-    if (n > best_n) { best_n = n; best_j = j; }
-  }
-  for (int off = 16; off > 0; off >>= 1) {
-    total += __shfl_xor_sync(FULLM, total, off);
-    int on = __shfl_xor_sync(FULLM, best_n, off), oj = __shfl_xor_sync(FULLM, best_j, off);
-    if (on > best_n || (on == best_n && oj < best_j)) { best_n = on; best_j = oj; }
-  }
-  int pick = best_j;
-  double entropy = 0.0;
-  // the one np.random draw sample_move_from_counts makes (np.random.choice): supplied by the caller or from the device generator
-  const double u01 = S.uniforms ? S.uniforms[g] : sp_uniform(rng);
-  if (P.low_visit_threshold > 0 && best_n < P.low_visit_threshold && temperature < 0.8) temperature = 0.8;   // internal.py:419-425
-  if (total > 0) {
-    // policy entropy of pi = n / total, pi clipped to [1e-12, 1] over all 4672 entries (internal.py:433-441)
-    double e = 0.0;
+  int pick = 0;
+  double entropy = 0.0, v = 0.0;
+  if constexpr (GUMBEL) {
+    pick = GB.choice[g];
+    entropy = GB.entropy[g];
+    v = GB.value[g];
+    if (pick < 0 || pick >= nc) {   // no result for this search
+      settle_game(E, S, g, s_moves[wib], lane, rng);
+      return;
+    }
+  } else {
+    // temperature schedule by full-move number (internal.py:386-394)
+    double temperature = P.temperature_end;
+    if (P.temperature_moves > 0) {
+      int mn = pos_fullmove(pos);
+      double t = (double)(mn < P.temperature_moves ? mn : P.temperature_moves) / (double)P.temperature_moves;
+      temperature = P.temperature_start + (P.temperature_end - P.temperature_start) * t;
+    }
+    if (P.argmax_after_plies >= 0) temperature = S.ply[g] < P.argmax_after_plies ? P.temperature_start : 0.0;   // arena.py:75-91
+    // visit counts -> move (internal.py:690-735)
+    long long total = 0;
+    int best_n = -1, best_j = 0;
     for (int j = lane; j < nc; j += 32) {
-      double p = (double)(float)((double)E.node_n[nb + fc + j] / (double)total);
-      if (p < 1e-12) p = 1e-12;
-      e -= p * log(p);
+      int n = E.node_n[nb + fc + j];
+      total += n;
+      if (n > best_n) { best_n = n; best_j = j; }
     }
-    for (int off = 16; off > 0; off >>= 1) e += __shfl_xor_sync(FULLM, e, off);
-    entropy = e - (double)(POLICY_SIZE - nc) * (1e-12 * log(1e-12));
-    if (temperature >= 1e-3) {
-      // visits.astype(float32) ** (1 / T), float32 pairwise sum, float32 divide; np.random.choice(k, p): p as float64, cdf = cumsum(p),
-      // cdf /= cdf[-1], index = searchsorted(cdf, u, 'right') (internal.py:713-734)
-      const float inv_t = (float)(1.0 / temperature);
-      for (int j = lane; j < nc; j += 32) s_w[wib][j] = powf((float)E.node_n[nb + fc + j], inv_t);
-      __syncwarp();
-      if (lane == 0) {
-        const float sum = np_pairwise_sum_f32(s_w[wib], nc);
-        if (sum > 0.0f && isfinite(sum)) {
-          double last = 0.0;
-          for (int j = 0; j < nc; ++j) last = d_add(last, (double)f_div(s_w[wib][j], sum));
-          double acc = 0.0;
-          int sel = nc - 1;
-          for (int j = 0; j < nc; ++j) {
-            acc = d_add(acc, (double)f_div(s_w[wib][j], sum));
-            if (d_div(acc, last) > u01) { sel = j; break; }
-          }
-          pick = sel;
-        } else if (!(sum <= 0.0f)) {
-          // the float32 sum overflowed: visit_dist /= inf leaves NaNs and the reference falls back to np.random.choice(legal_moves)
-          pick = (int)(u01 * nc);
-          if (pick >= nc) pick = nc - 1;
-        } else {
-          pick = (int)(u01 * nc);   // visit_sum <= 0: uniform over the legal moves (:717-722)
-          if (pick >= nc) pick = nc - 1;
-        }
+    for (int off = 16; off > 0; off >>= 1) {
+      total += __shfl_xor_sync(FULLM, total, off);
+      int on = __shfl_xor_sync(FULLM, best_n, off), oj = __shfl_xor_sync(FULLM, best_j, off);
+      if (on > best_n || (on == best_n && oj < best_j)) { best_n = on; best_j = oj; }
+    }
+    pick = best_j;
+    // the one np.random draw sample_move_from_counts makes (np.random.choice): supplied by the caller or from the device generator
+    const double u01 = S.uniforms ? S.uniforms[g] : sp_uniform(rng);
+    if (P.low_visit_threshold > 0 && best_n < P.low_visit_threshold && temperature < 0.8) temperature = 0.8;   // internal.py:419-425
+    if (total > 0) {
+      // policy entropy of pi = n / total, pi clipped to [1e-12, 1] over all 4672 entries (internal.py:433-441)
+      double e = 0.0;
+      for (int j = lane; j < nc; j += 32) {
+        double p = (double)(float)((double)E.node_n[nb + fc + j] / (double)total);
+        if (p < 1e-12) p = 1e-12;
+        e -= p * log(p);
       }
+      for (int off = 16; off > 0; off >>= 1) e += __shfl_xor_sync(FULLM, e, off);
+      entropy = e - (double)(POLICY_SIZE - nc) * (1e-12 * log(1e-12));
+      if (temperature >= 1e-3) {
+        // visits.astype(float32) ** (1 / T), float32 pairwise sum, float32 divide; np.random.choice(k, p): p as float64, cdf = cumsum(p),
+        // cdf /= cdf[-1], index = searchsorted(cdf, u, 'right') (internal.py:713-734)
+        const float inv_t = (float)(1.0 / temperature);
+        for (int j = lane; j < nc; j += 32) s_w[wib][j] = powf((float)E.node_n[nb + fc + j], inv_t);
+        __syncwarp();
+        if (lane == 0) {
+          const float sum = np_pairwise_sum_f32(s_w[wib], nc);
+          if (sum > 0.0f && isfinite(sum)) {
+            double last = 0.0;
+            for (int j = 0; j < nc; ++j) last = d_add(last, (double)f_div(s_w[wib][j], sum));
+            double acc = 0.0;
+            int sel = nc - 1;
+            for (int j = 0; j < nc; ++j) {
+              acc = d_add(acc, (double)f_div(s_w[wib][j], sum));
+              if (d_div(acc, last) > u01) { sel = j; break; }
+            }
+            pick = sel;
+          } else if (!(sum <= 0.0f)) {
+            // the float32 sum overflowed: visit_dist /= inf leaves NaNs and the reference falls back to np.random.choice(legal_moves)
+            pick = (int)(u01 * nc);
+            if (pick >= nc) pick = nc - 1;
+          } else {
+            pick = (int)(u01 * nc);   // visit_sum <= 0: uniform over the legal moves (:717-722)
+            if (pick >= nc) pick = nc - 1;
+          }
+        }
+        pick = __shfl_sync(FULLM, pick, 0);
+      }
+    } else if (nc > 0) {
+      if (lane == 0) pick = (int)(u01 * nc);  // uniform over legal moves (internal.py:701-707)
       pick = __shfl_sync(FULLM, pick, 0);
+      if (pick >= nc) pick = nc - 1;
     }
-  } else if (nc > 0) {
-    if (lane == 0) pick = (int)(u01 * nc);  // uniform over legal moves (internal.py:701-707)
-    pick = __shfl_sync(FULLM, pick, 0);
-    if (pick >= nc) pick = nc - 1;
-  }
-  if (nc == 0) {  // cannot happen for a searched root; be safe
-    settle_game(E, S, g, s_moves[wib], lane, rng);
-    return;
+    if (nc == 0) {  // cannot happen for a searched root; be safe
+      settle_game(E, S, g, s_moves[wib], lane, rng);
+      return;
+    }
+    const int rn = E.node_n[nb + root];
+    v = rn > 0 ? E.node_q[nb + root] : 0.0;  // value returned by MCTS.run (mcts.py:504)
   }
   const Move mv = (Move)(E.node_mv[nb + fc + pick] & 0xFFFFu);
-  const int rn = E.node_n[nb + root];
-  const double v = rn > 0 ? E.node_q[nb + root] : 0.0;  // value returned by MCTS.run (mcts.py:504)
   int ply = S.ply[g] + 1;                               // len(states) after the append (internal.py:447)
   bool resigned = false;
   if (lane == 0) {
@@ -400,6 +414,9 @@ selfplay_advance_kernel(EngineView E, SelfPlayState S, unsigned long long step, 
   __syncwarp();
   settle_game(E, S, g, s_moves[wib], lane, rng);
 }
+
+template __global__ void selfplay_advance_kernel<false>(EngineView, SelfPlayState, unsigned long long, u16*, GumbelView);
+template __global__ void selfplay_advance_kernel<true>(EngineView, SelfPlayState, unsigned long long, u16*, GumbelView);
 
 // drop every game's tree (nodes + transposition table) but keep positions and history: the
 // per-move equivalent of constructing a fresh MCTS (see DESIGN.md, reference quirk Q12)

@@ -233,6 +233,38 @@ class SearchEngine:
                                                               int(row0), 1 if per_sample else 0, int(row_cap), self._stream()),
                       "m0_search_expand_backup_multi")
 
+    # ---- Gumbel AlphaZero search (csrc/gumbel_kernels.cu, DESIGN.md §9) ------------------------------------------------------
+    def gumbel_configure(self, num_simulations: int, max_considered_actions: int, c_visit: float, c_scale: float) -> None:
+        import torch
+        _native.check(self._lib.m0_gumbel_configure(self._h, int(num_simulations), int(max_considered_actions), float(c_visit), float(c_scale)),
+                      "m0_gumbel_configure")
+        if not hasattr(self, "gb_move"):
+            self.gb_move = torch.zeros((self.G,), dtype=torch.int16, device=self.device)
+            self.gb_value = torch.zeros((self.G,), dtype=torch.float64, device=self.device)
+            self.gb_pi_children = torch.zeros((self.G, MAX_MOVES), dtype=torch.float64, device=self.device)
+
+    def gumbel_set_draws(self, draws=None) -> None:
+        """draws: float64 [G, 256] device tensor of Gumbel(0, 1) draws per legal move of the next roots, or None (device generator)."""
+        assert draws is None or (draws.dtype.is_floating_point and draws.element_size() == 8 and draws.is_contiguous()
+                                 and tuple(draws.shape) == (self.G, MAX_MOVES))
+        self._gumbel_draws = draws
+        _native.check(self._lib.m0_gumbel_set_draws(self._h, _native.ptr(draws)), "m0_gumbel_set_draws")
+
+    def gumbel_select(self) -> None:
+        _native.check(self._lib.m0_gumbel_select(self._h, self.planes.data_ptr(), self._stream()), "m0_gumbel_select")
+
+    def gumbel_expand_backup(self, logits, values) -> None:
+        assert logits.dtype.is_floating_point and logits.element_size() == 4 and logits.is_contiguous()
+        assert values.element_size() == 4 and values.is_contiguous()
+        _native.check(self._lib.m0_gumbel_expand_backup(self._h, logits.data_ptr(), logits.shape[1], values.data_ptr(), self._stream()),
+                      "m0_gumbel_expand_backup")
+
+    def gumbel_result(self, with_pi: bool = True) -> None:
+        """gb_move / gb_value, res_pi (with_pi), and per root child res_visits / res_q / gb_pi_children / res_count."""
+        _native.check(self._lib.m0_gumbel_result(self._h, self.gb_move.data_ptr(), self.res_pi.data_ptr() if with_pi else None,
+                                                 self.gb_value.data_ptr(), self.res_visits.data_ptr(), self.res_q.data_ptr(),
+                                                 self.gb_pi_children.data_ptr(), self.res_count.data_ptr(), self._stream()), "m0_gumbel_result")
+
     def counters(self) -> dict:
         buf = (ctypes.c_uint64 * 16)()
         _native.check(self._lib.m0_engine_counters(self._h, buf), "m0_engine_counters")

@@ -2,7 +2,8 @@
 ``DataManager.add_selfplay_data`` (azchess/selfplay/internal.py:447-466, 612-651):
 
     s          float32[T, 19, 8, 8]   encode_board of the position before every searched move       (internal.py:447)
-    pi         float32[T, 4672]       MCTS visit distribution returned by MCTS.run                   (internal.py:408, mcts.py:828-849)
+    pi         float32[T, 4672]       MCTS visit distribution returned by MCTS.run                   (internal.py:408, mcts.py:828-849);
+                                      the improved policy softmax(logits + sigma) in Gumbel mode (DESIGN.md §9)
     z          float32[T]             game result (White's view) x (+1 White / -1 Black to move)     (internal.py:612-616)
     legal_mask uint8[T, 4672]         MoveEncoder.get_legal_actions                                  (internal.py:454)
     meta_moves int32[1], meta_result float32[1], meta_resigned int8[1], meta_draw int8[1],
@@ -62,6 +63,8 @@ class GameRecorder:
         self._idx = torch.zeros((K, self.G, 256), dtype=torch.int16, device=dev)
         self._vis = torch.zeros((K, self.G, 256), dtype=torch.int32, device=dev)
         self._cnt = torch.zeros((K, self.G), dtype=torch.int32, device=dev)
+        # Gumbel search: the recorded pi is the improved policy of the root children (float32, child order), not n / total
+        self._gpi = torch.zeros((K, self.G, 256), dtype=torch.float32, device=dev) if getattr(sp, "gumbel", None) else None
         self._mvcnt = torch.zeros((self.G,), dtype=torch.int32, device=dev)
         self._now = 0                                       # engine plies recorded so far
         self._start = np.zeros((self.G,), dtype=np.int64)   # engine ply at which the current game of a slot started
@@ -82,7 +85,11 @@ class GameRecorder:
             self._ring_read = None
         st = _native.current_stream()
         k = self._now % self.keep_plies
-        eng.result(with_pi=False)
+        if self._gpi is not None:
+            self.sp.gumbel_result()
+            self._gpi[k].copy_(eng.gb_pi_children)
+        else:
+            eng.result(with_pi=False)
         _native.check(lib.m0_games_get_positions(eng._h, self._pos[k].data_ptr(), st), "m0_games_get_positions")
         # policy index of every root child (child order = legal-move order = m0_legal_moves order)
         _native.check(lib.m0_legal_moves(self._pos[k].data_ptr(), self.G, None, self._idx[k].data_ptr(), self._mvcnt.data_ptr(), st), "m0_legal_moves")
@@ -210,6 +217,8 @@ class GameRecorder:
             tot = n.sum(1)
             # pi[child.move_idx] = child.n / total: float64 divide, float32 store (mcts.py:840-847); the padding entries add 0.0 at index 0
             vals = torch.where(live & (tot[:, None] > 0), n / tot.clamp(min=1.0)[:, None], 0.0).to(torch.float32)
+            if self._gpi is not None:
+                vals = torch.where(live, self._gpi[d_ply, d_slot], 0.0)
             pi = torch.zeros((N, 4672), dtype=torch.float32, device=dev)
             pi.scatter_add_(1, torch.where(live, idx, 0), vals)
             planes = torch.empty((N, 19, 8, 8), dtype=torch.float32, device=dev)

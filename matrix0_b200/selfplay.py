@@ -83,6 +83,32 @@ def resolve_mcts_config(cfg_dict: Dict[str, Any]) -> MCTSConfig:
     return MCTSConfig.from_dict(m)
 
 
+GUMBEL_DEFAULTS = {"num_simulations": 32, "max_considered_actions": 16, "maxvisit_init": 50.0, "value_scale": 0.1}
+
+
+def resolve_gumbel_config(cfg_dict: Dict[str, Any]) -> Dict[str, Any]:
+    """The optional ``gumbel:`` section: num_simulations (1..4096), max_considered_actions (1..256), maxvisit_init (c_visit >= 0) and
+    value_scale (c_scale > 0); out-of-range values raise ValueError."""
+    sec = cfg_dict.get("gumbel", {}) or {}
+    unknown = set(sec) - set(GUMBEL_DEFAULTS)
+    if unknown:
+        raise ValueError(f"unknown gumbel option(s): {sorted(unknown)}")
+    out = dict(GUMBEL_DEFAULTS)
+    out.update(sec)
+    for key, lo, hi in (("num_simulations", 1, 4096), ("max_considered_actions", 1, 256)):
+        v = out[key]
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or not lo <= int(v) <= hi:
+            raise ValueError(f"gumbel.{key} must be an integer in [{lo}, {hi}], got {v!r}")
+        out[key] = int(v)
+    for key, positive in (("maxvisit_init", False), ("value_scale", True)):
+        v = out[key]
+        if isinstance(v, bool) or not isinstance(v, (int, float, np.integer, np.floating)) or not math.isfinite(float(v)) \
+                or (float(v) <= 0.0 if positive else float(v) < 0.0):
+            raise ValueError(f"gumbel.{key} must be a finite number {'> 0' if positive else '>= 0'}, got {v!r}")
+        out[key] = float(v)
+    return out
+
+
 @_native.on_own_device
 class SelfPlayEngine:
     # The root of a move is the child played at the previous move, and that child was evaluated during the previous search (a child
@@ -101,12 +127,18 @@ class SelfPlayEngine:
                           evaluator batches of ``forward_rows`` rows, samples are expanded / backed up in collection order;
         ``"virtual_loss"`` throughput mode: ``as_shipped`` plus the reference's in-flight marking (``_select``'s ``inflight_counts``,
                           mcts.py:889-890 / :922-923 -- code the reference ships but never activates, SURVEY Q2b) inside every mini-batch,
-                          so the simulations of a batch spread over distinct leaves and (almost) every simulation evaluates its own row."""
+                          so the simulations of a batch spread over distinct leaves and (almost) every simulation evaluates its own row;
+        ``"gumbel"``      Gumbel AlphaZero (DESIGN.md §9): ``gumbel.num_simulations`` simulation steps of one network row per game,
+                          sequential halving at the root, the recorded policy is the improved policy softmax(logits + sigma(completed Q)).
+                          Dirichlet noise, selection jitter, entropy noise, playout-cap randomisation and the temperature schedule do
+                          not apply in this mode: the Gumbel draw at the root is its exploration."""
         import torch
-        if search_mode not in ("collapsed", "as_shipped", "virtual_loss"):
-            raise ValueError(f"search_mode must be 'collapsed', 'as_shipped' or 'virtual_loss', got {search_mode!r}")
+        if search_mode not in ("collapsed", "as_shipped", "virtual_loss", "gumbel"):
+            raise ValueError(f"search_mode must be 'collapsed', 'as_shipped', 'virtual_loss' or 'gumbel', got {search_mode!r}")
         self.virtual_loss = search_mode == "virtual_loss"
         self.search_mode = search_mode = "as_shipped" if self.virtual_loss else search_mode
+        self.gumbel = resolve_gumbel_config(cfg_dict) if search_mode == "gumbel" else None
+        self.reuse_root_evals = self.reuse_root_evals and self.gumbel is None    # a Gumbel move evaluates its root (its draws are new)
         self.model = model
         self.cfg_dict = cfg_dict
         self.mcfg = resolve_mcts_config(cfg_dict)
@@ -120,13 +152,19 @@ class SelfPlayEngine:
         if max_nodes is None:
             # a fresh tree per move: every evaluated leaf adds its children (<= ~40 on average, 218 at most)
             sims_hi = int(self.mcfg.num_simulations * (1.0 + max(0.0, float(self.mcfg.playout_random_frac)))) + 1
-            leaves = (sims_hi if search_mode == "as_shipped" else (sims_hi + bs - 1) // bs) + 2
+            if self.gumbel:
+                sims_hi = self.gumbel["num_simulations"] + 1
+            leaves = (sims_hi if search_mode in ("as_shipped", "gumbel") else (sims_hi + bs - 1) // bs) + 2
             max_nodes = max(4096, 1 << int(math.ceil(math.log2(leaves * 48 + 256))))
         opening = int(self.sp.get("opening_random_plies", cfg_dict.get("openings", {}).get("random_plies", 0)))
         with torch.cuda.device(self.device):
-            self.engine = SearchEngine(self.G, max_nodes=max_nodes, max_depth=128,
+            depth = 128 if not self.gumbel else max(128, self.gumbel["num_simulations"] + 2)   # a Gumbel path grows by at most one per step
+            self.engine = SearchEngine(self.G, max_nodes=max_nodes, max_depth=depth,
                                        hist_cap=int(self.sp.get("max_game_len", 200)) + opening + 64, device=self.device_index)
             self.engine.configure(self.mcfg, deterministic, seed, virtual_loss=self.virtual_loss)
+            if self.gumbel:
+                gb = self.gumbel
+                self.engine.gumbel_configure(gb["num_simulations"], gb["max_considered_actions"], gb["maxvisit_init"], gb["value_scale"])
             if search_mode == "as_shipped":
                 self.engine.enable_multi(bs, virtual_loss=self.virtual_loss)
                 if forward_rows is None:
@@ -189,9 +227,15 @@ class SelfPlayEngine:
         self.tree_events = None     # set to a list to collect CUDA events around the tree kernels of every search step
         self.moves = 0
         self.steps = 0
+        self._result_ready = False  # Gumbel mode: gumbel_result() ran for the current move
 
     # ---- step plan --------------------------------------------------------------------------------
+    def sims_per_move(self) -> float:
+        return float(self.gumbel["num_simulations"] if self.gumbel else self.mcfg.num_simulations)
+
     def batches_per_move(self) -> int:
+        if self.gumbel:
+            return self.gumbel["num_simulations"]     # one simulation (one network row per game) per step
         sims = int(self.mcfg.num_simulations)
         frac = 0.0 if self.deterministic else float(self.mcfg.playout_random_frac)
         hi = int(max(max(1, sims * (1.0 - frac)), sims * (1.0 + frac))) if frac > 0 else sims
@@ -251,6 +295,13 @@ class SelfPlayEngine:
         import torch
         eng = self.engine
         _native.check(self._lib.m0_trees_clear(eng._h, _native.current_stream()), "m0_trees_clear")
+        if self.gumbel:
+            eng.begin()
+            logits, values = self._forward(eng.planes)
+            eng.gumbel_expand_backup(logits, values)           # the root: children, r, Gumbel draws, N = 1, W = r
+            self._result_ready = False
+            self.steps += 1
+            return
         if not self.reuse_root_evals:
             eng.begin()
             logits, values = self._forward(eng.planes)
@@ -292,14 +343,20 @@ class SelfPlayEngine:
             import torch
             e = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
             e[0].record()
-        _native.check(self._lib.m0_search_select_var(eng._h, int(self.mcfg.inference_batch_size), self.sims_left.data_ptr(),
-                                                     eng.planes.data_ptr(), _native.current_stream()), "m0_search_select_var")
+        if self.gumbel:
+            eng.gumbel_select()
+        else:
+            _native.check(self._lib.m0_search_select_var(eng._h, int(self.mcfg.inference_batch_size), self.sims_left.data_ptr(),
+                                                         eng.planes.data_ptr(), _native.current_stream()), "m0_search_select_var")
         if ev is not None:
             e[1].record()
         logits, values = self._forward(eng.planes)
         if ev is not None:
             e[2].record()
-        eng.expand_backup(logits, values)
+        if self.gumbel:
+            eng.gumbel_expand_backup(logits, values)
+        else:
+            eng.expand_backup(logits, values)
         if ev is not None:
             e[3].record()
             ev.append(e)
@@ -347,8 +404,21 @@ class SelfPlayEngine:
             g0 = g1
         self.steps += 1
 
+    def gumbel_result(self, with_pi: bool = False) -> None:
+        """Gumbel mode, after the simulations of a move: the move to play, the search value and the policy target (engine.gb_*,
+        engine.res_*); end_move() calls it when nobody did."""
+        self.engine.gumbel_result(with_pi=with_pi)
+        self._result_ready = True
+
     def end_move(self) -> None:
-        _native.check(self._lib.m0_selfplay_advance(self.engine._h, self.moves_played.data_ptr(), _native.current_stream()), "m0_selfplay_advance")
+        if self.gumbel:
+            if not self._result_ready:
+                self.gumbel_result()
+            self._result_ready = False
+            _native.check(self._lib.m0_selfplay_advance_gumbel(self.engine._h, self.moves_played.data_ptr(), _native.current_stream()),
+                          "m0_selfplay_advance_gumbel")
+        else:
+            _native.check(self._lib.m0_selfplay_advance(self.engine._h, self.moves_played.data_ptr(), _native.current_stream()), "m0_selfplay_advance")
         self.moves += 1
 
     def play_move(self) -> None:
@@ -404,7 +474,8 @@ def _selfplay_worker_on_device(proc_id: int, cfg_dict: Dict[str, Any], ckpt_path
         model.load_state_dict(sd, strict=False)
     G = int(concurrent_games or min(int(games), 4096))
     # "as_shipped": the reference's search with its configured selection jitter and entropy noise (distinct leaves per mini-batch);
-    # "collapsed": one evaluated leaf per game and mini-batch (the throughput mode, exact when the jitter is neutralised)
+    # "collapsed": one evaluated leaf per game and mini-batch (the throughput mode, exact when the jitter is neutralised);
+    # "gumbel": Gumbel AlphaZero with the improved policy as the recorded target (the config's `gumbel:` section)
     sp = SelfPlayEngine(model, cfg_dict, games=G, device=dev, deterministic=False, seed=seed, precision=precision, search_mode=search_mode)
     sp.warm_up_forward()
     mcfg = cfg_dict.get("model", {}) or {}
@@ -493,7 +564,7 @@ def _selfplay_worker_on_device(proc_id: int, cfg_dict: Dict[str, Any], ckpt_path
             if sp.active_games() == 0:
                 break                            # every started game is over (games that ended inside their opening plies leave no shard)
             if q is not None and time.perf_counter() - last_hb >= 2.0:
-                q.put({"type": "heartbeat", "proc": proc_id, "game": submitted, "moves": sp.moves, "avg_sims": float(sp.mcfg.num_simulations),
+                q.put({"type": "heartbeat", "proc": proc_id, "game": submitted, "moves": sp.moves, "avg_sims": sp.sims_per_move(),
                        "resigned": False, "avg_policy_entropy": 0.0})
                 last_hb = time.perf_counter()
         handle_all(rec.flush())
