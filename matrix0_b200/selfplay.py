@@ -83,6 +83,16 @@ def resolve_mcts_config(cfg_dict: Dict[str, Any]) -> MCTSConfig:
     return MCTSConfig.from_dict(m)
 
 
+MAX_LEGAL_MOVES = 218     # the most legal moves a chess position can have
+GUMBEL_NODE_BYTES = 50    # per node slot: prior, w, q (float64), n, first child, creator, move (int32), child count (int16), logit, r (fp32)
+
+
+def gumbel_max_nodes(num_simulations: int) -> int:
+    """Node slots a Gumbel move can fill in one game: the root, then at most num_simulations + 1 expansions (the root's and one per
+    simulation) of at most 218 children each.  The tree has no transpositions, so a position with 218 moves at every node fills it."""
+    return 1 + (int(num_simulations) + 1) * MAX_LEGAL_MOVES
+
+
 GUMBEL_DEFAULTS = {"num_simulations": 32, "max_considered_actions": 16, "maxvisit_init": 50.0, "value_scale": 0.1}
 
 
@@ -149,17 +159,28 @@ class SelfPlayEngine:
         self.device_index = torch.cuda.current_device() if device is None else int(device)
         self.device = torch.device("cuda", self.device_index)
         bs = max(1, int(self.mcfg.inference_batch_size))
-        if max_nodes is None:
+        tt_capacity = 0                 # the engine's default: 2 * max_nodes
+        if self.gumbel:
+            # the table only holds the root (m0_search_begin); the tree itself has no transpositions
+            tt_capacity = 64
+            if max_nodes is None:
+                max_nodes = gumbel_max_nodes(self.gumbel["num_simulations"])
+                # the pool must fit in what the device has free now (the network and its workspaces are already allocated); a pool
+                # that fits but leaves too little for the rest fails in the engine's allocation instead
+                free, _ = torch.cuda.mem_get_info(self.device)
+                if self.G * max_nodes * GUMBEL_NODE_BYTES > free:
+                    raise ValueError(f"the Gumbel node pool of {self.G} games x {max_nodes} nodes (1 + (num_simulations + 1) x 218) needs "
+                                     f"{self.G * max_nodes * GUMBEL_NODE_BYTES / 2**30:.1f} GiB, more than the {free / 2**30:.1f} GiB free on the "
+                                     f"device: pass max_nodes= (a pool that can overflow on positions with many moves), fewer games or fewer simulations")
+        elif max_nodes is None:
             # a fresh tree per move: every evaluated leaf adds its children (<= ~40 on average, 218 at most)
             sims_hi = int(self.mcfg.num_simulations * (1.0 + max(0.0, float(self.mcfg.playout_random_frac)))) + 1
-            if self.gumbel:
-                sims_hi = self.gumbel["num_simulations"] + 1
-            leaves = (sims_hi if search_mode in ("as_shipped", "gumbel") else (sims_hi + bs - 1) // bs) + 2
+            leaves = (sims_hi if search_mode == "as_shipped" else (sims_hi + bs - 1) // bs) + 2
             max_nodes = max(4096, 1 << int(math.ceil(math.log2(leaves * 48 + 256))))
         opening = int(self.sp.get("opening_random_plies", cfg_dict.get("openings", {}).get("random_plies", 0)))
         with torch.cuda.device(self.device):
             depth = 128 if not self.gumbel else max(128, self.gumbel["num_simulations"] + 2)   # a Gumbel path grows by at most one per step
-            self.engine = SearchEngine(self.G, max_nodes=max_nodes, max_depth=depth,
+            self.engine = SearchEngine(self.G, max_nodes=max_nodes, tt_capacity=tt_capacity, max_depth=depth,
                                        hist_cap=int(self.sp.get("max_game_len", 200)) + opening + 64, device=self.device_index)
             self.engine.configure(self.mcfg, deterministic, seed, virtual_loss=self.virtual_loss)
             if self.gumbel:

@@ -7,7 +7,9 @@ visit schedule, interior selection by ``argmax softmax(l + sigma) - N / (1 + Nc)
 at the root.  Every node holds N and W from the view of its side to move; a child's value for its parent is ``-W / N``.
 
 ``search`` also returns the smallest decision margin (best minus second-best score over every argmax the search took): a test
-that compares the device search against this one may drop games whose margin is at rounding level.
+that compares the device search against this one may drop games whose margin is at rounding level.  It counts the nodes it creates
+as the device allocates them (the root, then every child of every expansion) and the simulations that ended on a terminal leaf, by
+kind, so a test built around a terminal rule can check that the tree reaches it.
 """
 from __future__ import annotations
 
@@ -78,6 +80,20 @@ def terminal_value(b, draw_penalty: float) -> Optional[float]:
     return -1.0 if b.is_checkmate() else float(draw_penalty)
 
 
+TERMINAL_KINDS = ("checkmate", "stalemate", "insufficient_material", "seventyfive_moves", "fivefold_repetition")
+
+
+def terminal_kind(b) -> str:
+    """Which rule ends a position that is_game_over() calls over (checkmate first: its value is -1, every other kind is a draw)."""
+    if b.is_checkmate():
+        return "checkmate"
+    if b.is_stalemate():
+        return "stalemate"
+    if b.is_insufficient_material():
+        return "insufficient_material"
+    return "seventyfive_moves" if b.is_seventyfive_moves() else "fivefold_repetition"
+
+
 def _argmax(scores: np.ndarray) -> Tuple[int, float]:
     """First maximum and the margin to the second-best finite score (inf when there is no second)."""
     j = int(np.argmax(scores))
@@ -91,6 +107,10 @@ def search(board, evaluate: Callable, gumbel: np.ndarray, n: int, m: int, c_visi
     """One Gumbel search from `board` (history included).  evaluate(planes float32[19, 8, 8]) -> (logits float32[4672], value);
     gumbel: float64 draws, one per legal move in generation order."""
     margin = [math.inf]
+    nodes = [1]                                   # the root
+    max_depth = [0]                               # longest selection path, in moves from the root
+    terminals = dict.fromkeys(TERMINAL_KINDS, 0)
+    terminal_depth = {}                           # kind -> shallowest depth (moves from the root) it was reached at
 
     def expand(node: _Node, b) -> None:
         lg, v = evaluate(encode_board(b))
@@ -100,6 +120,7 @@ def search(board, evaluate: Callable, gumbel: np.ndarray, n: int, m: int, c_visi
         node.logits = np.array([float(lg[move_to_index_unchecked(wtm, mv.from_square, mv.to_square, mv.promotion)]) for mv in node.moves],
                                dtype=np.float64)
         node.children = [_Node() for _ in node.moves]
+        nodes[0] += len(node.moves)
         node.r = max(-1.0, min(1.0, float(np.float32(v))))
 
     def stats(node: _Node):
@@ -138,10 +159,15 @@ def search(board, evaluate: Callable, gumbel: np.ndarray, n: int, m: int, c_visi
             b.push(node.moves[j])
             node = node.children[j]
             path.append(node)
+        max_depth[0] = max(max_depth[0], len(path) - 1)
         v = terminal_value(b, draw_penalty)
         if v is None:
             expand(node, b)
             v = node.r
+        else:
+            kind = terminal_kind(b)
+            terminals[kind] += 1
+            terminal_depth[kind] = min(terminal_depth.get(kind, len(path)), len(path) - 1)
         v = max(-1.0, min(1.0, v))
         for nd in reversed(path):
             nd.n += 1
@@ -158,4 +184,4 @@ def search(board, evaluate: Callable, gumbel: np.ndarray, n: int, m: int, c_visi
         pi[move_to_index_unchecked(wtm, mv.from_square, mv.to_square, mv.promotion)] = np.float32(p)
     return {"moves": root.moves, "actions": actions, "visits": N, "q": np.where(N > 0, -W / np.maximum(N, 1), 0.0),
             "pi_legal": pi_legal, "pi": pi, "chosen": chosen, "move": root.moves[chosen], "value": root.w / root.n,
-            "margin": margin[0]}
+            "margin": margin[0], "nodes": nodes[0], "terminals": terminals, "terminal_depth": terminal_depth, "depth": max_depth[0]}

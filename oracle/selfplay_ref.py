@@ -93,7 +93,9 @@ class GameLoopRef:
         self.search_values: List[float] = []
         self.recent_values: List[float] = []
         self.recent_entropies: List[float] = []
+        self.entropies: List[float] = []        # one per ply: their mean is the game's average policy entropy
         self.consec_bad = 0
+        self.resign_checks: List[tuple] = []    # per ply the resign rule ran: (enough bad plies in a row, stable_bad, low_unc)
         self.resigned = False
         self.z: Optional[float] = None
         self.window_k = int(sp_cfg.get("resign_window", 4))
@@ -135,8 +137,17 @@ class GameLoopRef:
         if thr > 0 and max(visits) < thr:
             temp = max(temp, 0.8)
         idx = sample_move_from_counts(moves, visits, temp, u)
+        return self._advance(moves, idx, pi, v)
+
+    def play_gumbel(self, moves: List, idx: int, pi: np.ndarray, v: float):
+        """The same ply after a Gumbel search (DESIGN.md §9): the search chose moves[idx], v is its value W(root) / N(root) and pi its
+        policy target pi' (float32 over the 4672 policy indices); no temperature and no sampling.  Returns idx, or None when resigned."""
+        return self._advance(moves, int(idx), pi, v)
+
+    def _advance(self, moves: List, idx: int, pi: np.ndarray, v: float):
         _pi = np.clip(pi.astype(np.float64, copy=False), 1e-12, 1.0)
         ent = float(-np.sum(_pi * np.log(_pi)))
+        self.entropies.append(ent)
         self.recent_entropies.append(ent)
         if len(self.recent_entropies) > self.window_k:
             self.recent_entropies.pop(0)
@@ -151,7 +162,9 @@ class GameLoopRef:
             need = max(2, self.window_k // 2)
             stable_bad = len(self.recent_values) >= need and (sum(self.recent_values) / len(self.recent_values)) < (resign_thr + float(self.sp.get("resign_value_margin", 0.05)))
             low_unc = len(self.recent_entropies) >= need and (sum(self.recent_entropies) / len(self.recent_entropies)) < float(self.sp.get("resign_min_entropy", 0.3))
-            if self.consec_bad >= int(self.sp.get("resign_consecutive_bad", 5)) and (stable_bad or low_unc):
+            streak = self.consec_bad >= int(self.sp.get("resign_consecutive_bad", 5))
+            self.resign_checks.append((streak, stable_bad, low_unc))
+            if streak and (stable_bad or low_unc):
                 self.resigned = True
                 self.z = -1.0 if self.board.turn == chess.WHITE else 1.0
                 return None

@@ -104,3 +104,67 @@ def test_gumbel_config_is_validated():
                 {"maxvisit_init": -1.0}, {"value_scale": 0.0}, {"value_scale": float("nan")}, {"num_simulations": 1.5}, {"bogus": 1}):
         with pytest.raises(ValueError):
             resolve_gumbel_config({"gumbel": bad})
+
+
+def test_schedule_grid_reaches_every_branch():
+    """The (n, m) grid of tests/test_gumbel_edges_gpu.py against the device's halving_schedule_at, restated branch by branch: equal
+    to the oracle's schedule at every grid entry, and together the entries take every branch (the grid's boards have at least m
+    legal moves, so m' = m)."""
+    from gumbel_cases import SCHEDULE_BRANCHES, SCHEDULE_GRID, schedule_branches
+    taken = {}
+    for n, m in SCHEDULE_GRID:
+        T, branches = schedule_branches(m, n)
+        assert T == GR.schedule(m, n), (n, m)
+        for b in branches:
+            taken.setdefault(b, []).append((n, m))
+    assert set(taken) == SCHEDULE_BRANCHES, sorted(SCHEDULE_BRANCHES - set(taken))
+
+
+def test_schedule_branches_of_known_settings():
+    from gumbel_cases import schedule_branches
+    assert schedule_branches(1, 4) == ([0, 1, 2, 3], {"single_candidate"})
+    assert schedule_branches(2, 8)[1] == {"one_halving_level", "repeats_above_one", "clamped_to_two"}
+    assert schedule_branches(16, 32)[1] == {"repeats_clamped", "repeats_above_one"}
+    assert schedule_branches(7, 50)[1] == {"repeats_above_one", "odd_halving", "clamped_to_two"}
+    assert schedule_branches(16, 2)[1] == {"n_below_m", "repeats_clamped"}
+
+
+def _small_net_evaluator(golden_dir):
+    """The golden small network through the oracle's float32 forward on the CPU, one position per call (cached)."""
+    import torch
+    from oracle import nn_ref
+    from test_oracle_nn import load_case
+    _, cfg, sd = load_case(golden_dir, "small")
+    sd = {k: v.float() for k, v in sd.items()}
+    cache = {}
+
+    def evaluate(planes):
+        key = planes.tobytes()
+        if key not in cache:
+            with torch.no_grad():
+                p, v = nn_ref.forward(sd, cfg, torch.from_numpy(planes[None]))
+            cache[key] = (p[0].numpy().astype(np.float32), float(v.reshape(-1)[0]))
+        return cache[key]
+    return evaluate
+
+
+@pytest.mark.parametrize("n", [64, 200])
+def test_gumbel_node_pool_bound_holds_on_edge_boards(golden_dir, n):
+    """SelfPlayEngine sizes a Gumbel game's node pool as gumbel_max_nodes(n) = 1 + (n + 1) * 218.  The oracle counts the nodes it
+    creates as the device allocates them: on every constructed board the count stays within the bound, each board's tree reaches
+    the terminal rule it was built for, and the five-queen board outgrows the 4096 slots the visit-count sizing gave at n = 64."""
+    from gumbel_cases import EDGE_BOARDS, EDGE_DRAW_SEED, EDGE_M
+    from matrix0_b200.selfplay import gumbel_max_nodes
+    evaluate = _small_net_evaluator(golden_dir)
+    draws = np.random.default_rng(EDGE_DRAW_SEED).gumbel(size=256)
+    bound = gumbel_max_nodes(n)
+    assert bound == 1 + (n + 1) * 218
+    for name, make, kind, min_depth in EDGE_BOARDS:
+        b = make()
+        out = GR.search(b.copy(), evaluate, draws, n=n, m=EDGE_M, draw_penalty=-0.05)
+        assert out["nodes"] <= bound, name
+        if kind is not None and n == 200:
+            assert out["terminals"][kind] > 0, (name, out["terminals"])
+            assert out["terminal_depth"][kind] >= min_depth, (name, out["terminal_depth"])
+        if name == "five_queens" and n == 64:
+            assert out["nodes"] > 4096, out["nodes"]

@@ -54,3 +54,28 @@ def test_sample_move_from_counts_matches_reference():
         assert list(counts.keys())[got] == want, (seed, T)
         n += 1
     assert n == 400
+
+
+def test_game_loop_gumbel_variant_plays_the_chosen_move_and_resigns():
+    """GameLoopRef.play_gumbel: the searched move is pushed as chosen (no temperature, no sampling), the entropy of pi' and the search
+    value feed the same resign rule as play(), and play() with an argmax pick of the same move leaves the same state."""
+    import math
+    from oracle.selfplay_ref import GameLoopRef
+    sp = {"resign_threshold": -0.5, "min_resign_plies": 2, "resign_window": 4, "resign_consecutive_bad": 2, "resign_min_entropy": 9.0,
+          "resign_value_margin": 0.05, "temperature_start": 1e-4, "temperature_end": 1e-4}
+    pi = np.zeros(4672, dtype=np.float32)
+    pi[[7, 9]] = 0.5
+    gum, vis = GameLoopRef(sp, {}), GameLoopRef(sp, {})
+    for ply, (idx, v) in enumerate([(3, -0.9), (0, -0.9)]):
+        moves = list(gum.board.legal_moves)
+        assert gum.play_gumbel(moves, idx, pi, v) == idx
+        counts = [0] * len(moves)
+        counts[idx] = 5
+        assert vis.play(moves, counts, pi, v, 0.5) == idx
+        assert gum.board.fen() == vis.board.fen() and gum.entropies == vis.entropies and gum.consec_bad == vis.consec_bad
+    assert gum.board.move_stack[0] == list(chess.Board().legal_moves)[3]
+    assert gum.entropies[0] == pytest.approx(math.log(2.0) - 4670 * 1e-12 * math.log(1e-12), rel=1e-12)
+    # third ply: two values below the threshold in a row at ply >= min_resign_plies, and a mean entropy below 9: White resigns
+    assert gum.play_gumbel(list(gum.board.legal_moves), 0, pi, -0.9) is None
+    assert gum.resigned and gum.z == -1.0 and gum.n_states == 3 and len(gum.board.move_stack) == 2
+    assert gum.resign_checks == [(False, False, True), (True, True, True)]     # plies 2 and 3: (bad streak, stable_bad, low_unc)
